@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the headline benchmark of the hot path (BASELINE.json metric: k-NN queries/sec).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c2|t128|c1] [--no-extras]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c2|t128|c1] [--no-extras] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic queries: batched exact k-NN (k = 10) on the
 configuration BASELINE.json quotes the metric on, config 2: BallTree 1M x 16 f32 uniform points, 1M queries per GPU.
@@ -24,6 +24,10 @@ its own 1M queries.
 
 `--impl reference` times the reference's own CPU implementation of the path (the oracle's C restatement of the Rust
 crate -- no Rust toolchain exists in this image) on the host cores.
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's batch) as DIR/*.npy, so that two builds can be
+compared output for output on the same seeded inputs: a fixed, seeded sample of query rows (`query_rows`), their
+neighbour indices (`indices`, float64: exact below 2^53) and distances (`distances`, the tree's dtype), 32 MiB at most.
 """
 from __future__ import annotations
 
@@ -118,6 +122,22 @@ class ClockSampler:
         if not sm:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": [], "samples": 0}
         return {"sm_mhz": float(np.median(sm)), "sm_max_mhz": mx, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, idx, dist):
+    """Writes the rows of a seeded sample of the (nq, k) result tensors `idx`, `dist` (see --dump-outputs)."""
+    import torch
+    nq, k = idx.shape
+    m = min(nq, DUMP_BYTES // (8 + k * (8 + dist.element_size())))
+    rows = np.sort(np.random.default_rng(0).choice(nq, size=m, replace=False))
+    sel = torch.from_numpy(rows).to(idx.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "query_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "indices.npy"), idx.index_select(0, sel).cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "distances.npy"), dist.index_select(0, sel).cpu().numpy())
 
 
 def make_inputs(wl, rank):
@@ -513,8 +533,14 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra configurations (t128, c3, c4, multi-GPU arms)")
     ap.add_argument("--extras", default="", help="comma-separated subset of t128,c3,c4,multi (default: all)")
     ap.add_argument("--queries", type=int, default=0, help="override queries per GPU (profiling runs only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs as DIR/*.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 0)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the B200 arm (the reference arm's query sample depends on its timing)")
+    sys.dont_write_bytecode = True  # the tree may be read-only; leave it as it was found
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -600,6 +626,8 @@ def main():
     clocks = sampler.stop(t_wall0, t_wall1)
     ms_steps = [a.elapsed_time(b) for a, b in evs]
     total_ms = float(sum(ms_steps))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, idx_dev, dist_dev)
     # one synchronous call to read the engine's work counters for exactly one step
     tree.query_knn_dev(q_dev.data_ptr(), nq, d, k, idx_dev.data_ptr(), dist_dev.data_ptr(),
                        stream=stream.cuda_stream, sync=True)
