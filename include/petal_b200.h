@@ -168,9 +168,10 @@ int32_t pn_tree_destroy(pn_tree *tree); /* Rust Drop */
  * (src/distance.rs:19), so several threads may query one tree at once.  Calls on ONE handle serialise on its mutex
  * (they share one stream and one set of workspaces).  A session is a second handle onto the same device-resident tree
  * -- nothing of the tree is copied -- with its own stream, events, workspaces and counters: calls on different
- * sessions overlap on the device.  One session per calling thread is the intended use.  Sessions and the tree they
- * came from may be destroyed in any order (the arrays live until the last of them is gone); a session answers every
- * query entry point of its tree's kind. */
+ * sessions overlap on the device.  One session per calling thread is the intended use.  The tree, including a
+ * partition built later by a query on any of them, is shared by the handle and all its sessions (and their sessions)
+ * and lives until the last of them is destroyed, in any order.  Its device memory is reported by the handle that built
+ * it (pn_tree_info::device_bytes; 0 on a session).  A session answers every query entry point of its tree's kind. */
 int32_t pn_tree_session(pn_tree *tree, pn_tree **out);
 
 /* --- BallTree::query (src/ball_tree.rs:102-121), batched: `nq` queries, row stride

@@ -41,16 +41,37 @@ static int fail(int code, const std::string& msg) {
         if (r_ != PN_OK) return r_; \
     } while (0)
 
+struct DeviceGuard {
+    int prev = -1;
+    bool ok = true;
+    explicit DeviceGuard(int dev) {
+        if (cudaGetDevice(&prev) != cudaSuccess) { ok = false; (void)cudaGetLastError(); return; }
+        if (prev != dev && cudaSetDevice(dev) != cudaSuccess) { ok = false; (void)cudaGetLastError(); }
+    }
+    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+};
+
+// A device allocation that grows on demand and is freed on the device it was made on, whichever device is current.
 struct DevBuf {
     void* p = nullptr;
     size_t cap = 0;
-    bool borrowed = false;   // an alias of another handle's array (pn_tree_session): never freed or grown here
-    void alias(const DevBuf& o) { release(); p = o.p; cap = o.cap; borrowed = true; }
+    int device = -1;
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : p(o.p), cap(o.cap), device(o.device) { o.p = nullptr; o.cap = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept {
+        if (this != &o) {
+            release();
+            p = o.p; cap = o.cap; device = o.device;
+            o.p = nullptr; o.cap = 0;
+        }
+        return *this;
+    }
+    ~DevBuf() { release(); }
     int ensure(size_t bytes) {
         if (bytes <= cap) return PN_OK;
-        if (borrowed) return fail(PN_BAD_ARG, "internal: a borrowed array cannot grow");
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
+        release();
         size_t want = bytes + bytes / 8 + 256;
         cudaError_t e = cudaMalloc(&p, want);
         if (e != cudaSuccess) {
@@ -60,20 +81,17 @@ struct DevBuf {
         }
         if (e != cudaSuccess) { p = nullptr; return fail(PN_OOM, std::string("cudaMalloc: ") + cudaGetErrorString(e)); }
         cap = want;
+        if (cudaGetDevice(&device) != cudaSuccess) (void)cudaGetLastError();
         return PN_OK;
     }
-    void release() { if (p && !borrowed) cudaFree(p); p = nullptr; cap = 0; borrowed = false; }
-    template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
-};
-
-struct DeviceGuard {
-    int prev = -1;
-    bool ok = true;
-    explicit DeviceGuard(int dev) {
-        if (cudaGetDevice(&prev) != cudaSuccess) { ok = false; (void)cudaGetLastError(); return; }
-        if (prev != dev && cudaSetDevice(dev) != cudaSuccess) { ok = false; (void)cudaGetLastError(); }
+    void release() {
+        if (p) {
+            DeviceGuard g(device);
+            cudaFree(p);
+        }
+        p = nullptr; cap = 0;
     }
-    ~DeviceGuard() { if (prev >= 0) cudaSetDevice(prev); }
+    template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
 };
 
 }  // namespace petal
@@ -103,8 +121,6 @@ struct PeerShared {
     void fail() { std::lock_guard<std::mutex> lk(mu); failed = true; cv.notify_all(); }
 };
 
-static std::mutex g_life;   // lifetime bookkeeping of trees and their sessions (pn_tree_destroy, pn_tree_session)
-
 // The opaque handle.
 struct pn_tree {
     virtual ~pn_tree() {}
@@ -112,11 +128,7 @@ struct pn_tree {
     pn_counters counters{};
     std::mutex mu;
     bool host_only = false;
-    // sessions (pn_tree_session): handles that borrow this handle's device arrays.  The owner is freed when it has been
-    // destroyed AND its last session is gone.
-    pn_tree* owner = nullptr;
-    std::atomic<int> n_sessions{0};
-    bool zombie = false;
+    virtual uint64_t device_bytes() const = 0;   // pn_tree_info::device_bytes
     virtual int session(pn_tree** out) = 0;
     virtual int knn_host(const void* q, size_t nq, size_t stride, size_t k, uint64_t* idx, void* dist) = 0;
     virtual int knn_dev(const void* q, size_t nq, size_t stride, size_t k, uint64_t* idx, void* dist,
@@ -134,98 +146,57 @@ struct pn_tree {
 
 namespace petal {
 
+#define NC(x)                                                                                                      \
+    do {                                                                                                           \
+        ncclResult_t r_ = (x);                                                                                     \
+        if (r_ != ncclSuccess) return fail(PN_NCCL, std::string(#x) + ": " + cm->api->GetErrorString(r_));         \
+    } while (0)
+
 template <typename A>
-struct Engine final : pn_tree {
+struct DeviceTree {
     using V = typename VT<A>::V;
     FlatTree<A> ft;  // host copy of the flattened tree (point rows dropped after upload)
     int device = 0;
-    int n_sms = 148;
-    cudaStream_t stream = nullptr, last_stream = nullptr;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    DevBuf d_pts, d_ids, d_blo, d_bhi, d_centers, d_radii, d_vpids, d_plane_w, d_plane_t;
-    DevBuf w_qraw, w_q, w_home, w_hist, w_cursor, w_order, w_part_d, w_part_i, w_floor_d, w_floor_i,
-        w_counters, w_out_i, w_out_d, w_counts, w_offsets, w_hits;
-    DevTree<A> dt{};
-    // host-buffer calls are software-pipelined over chunks of queries: H2D of chunk i+1 and D2H of chunk i-1 run on their own
-    // streams under the kernels of chunk i (two sets of raw-query / result buffers)
-    cudaStream_t s_in = nullptr, s_out = nullptr;
-    cudaEvent_t e_in[2] = {nullptr, nullptr}, e_cmp[2] = {nullptr, nullptr}, e_out[2] = {nullptr, nullptr};
-    DevBuf w_qraw2[2], w_oi2[2], w_od2[2];
-    DevBuf sh_li[2], sh_ld[2], sh_pack[2], sh_gat[2], sh_gat_d[2];   // sharded k-NN: local lists, packed keys, gathered lists
-    std::vector<cudaEvent_t> sh_ev;                                    // timing events of the sharded pipeline (reused)
-    DevBuf r_qraw[2], r_q[2], r_counts[2], r_offsets[2], r_hits[2], r_slab[2], r_qlist[2], r_nlist[2], r_sums[2];  // radius pipeline workspaces
-    unsigned long long* pin_tot = nullptr;                            // pinned: chunk totals of the radius count pass
-    void* pin_stage[2] = {nullptr, nullptr};  // pinned D2H staging for the variable-length radius output
-    cudaEvent_t pin_ev[2] = {nullptr, nullptr};
-    static constexpr size_t PIN_BYTES = 16u << 20;
-    // tensor path (f32 input only): augmented FP16 operands, see tc_filter.cuh
-    DevBuf d_baug, d_center, w_aaug, w_qmargin, w_trace, w_gbound;
-    bool tensor_ready = false, last_used_tensor = false;
-    // pruned tensor scan (tc_prune.cuh): tile balls, the build-time estimate of what pruning can do, per-call workspaces
-    DevBuf d_tcen, d_trad, w_qs, w_seed, w_bits, w_tcnt;
-    DevBuf w_bcen, w_brad, w_bmu, w_qth, w_bbits, w_bcnt, w_wslot, w_wlist, w_wbits, w_nwide;   // tile-bitmap pass: query balls, their bitmaps, wide balls
-    double prune_frac = 0.0;      // estimated fraction of (query group, tile) pairs that are out of reach
-    double seed_candidates = 0.0; // estimated candidates per query that survive a seed threshold
-    double tile_frac = 0.0;       // estimated share of tiles beyond a single query's seed
-    bool prune_on = false, tiles_on = false, last_pruned = false;   // prune_on: sorted + seeded scan; tiles_on: with tile bitmaps
-    uint32_t prune_opt = 0;       // pn_prune
-    // Vantage-point trees: the tensor path never used the VP bounds (a dense scan over the stored order), and the VP order
-    // -- shells around vantage points -- gives tiles that no ball can bound tightly.  A VP handle with a device therefore
-    // also keeps the BALL partition of the same points (built on the device) and answers tensor-path queries from it:
-    // exact 1-NN does not depend on the partition; the VP arrays serve the pruned SIMT traversal (PN_ALGO_SIMT), the layout
-    // accessors and trees the tensor path does not take (f64, d < 16).
-    std::unique_ptr<Engine<A>> aux;
-    // Ball handles (and the ball partition of a VP handle) on CLUSTERED data: the reference's split -- the median of the
-    // widest coordinate -- cuts through clusters, so in d >= 32 most 128-row tiles of the stored order mix fragments of
-    // several clusters and no ball bounds them tightly (BASELINE config 3: 88 % of all (query group, tile) pairs stay).
-    // Such a handle keeps a second ball tree over the same rows, partitioned by the TWO-MEANS rule of gpu_build.cu
-    // (partition_rule 1), and answers its k-NN batches from it: exact results do not depend on the partition, the tile
-    // bitmaps of tc_prune.cuh do.  two_means_partition() decides from the build-time estimates of both partitions.
-    uint32_t partition_rule = 0;  // gb::build_ball_tree rule of THIS engine's arrays
-    static constexpr uint32_t TWO_MEANS_ORDER_LEVELS = 1;
+    uint32_t algo = PN_ALGO_AUTO;
+    uint32_t prune_opt = 0;  // pn_prune
     bool gpu_built = false;  // the tree arrays were produced on the device (gpu_build.cu); host copies are fetched on demand
+    DevBuf d_pts, d_ids, d_blo, d_bhi, d_centers, d_radii, d_vpids, d_plane_w, d_plane_t;
+    DevTree<A> dt{};
+    uint64_t bytes = 0;      // device memory of this tree's arrays (not counting `part`)
+    // tensor path (f32 input only): augmented FP16 operands, see tc_filter.cuh
+    DevBuf d_baug, d_center;
+    bool tensor_ready = false;
     uint32_t kp = 0;       // padded K of the augmented operands (multiple of 32)
     float pmax = 0.f;      // max |s (p - center)|
     float tscale = 1.f;    // s: power of two bringing the centred coordinates into [-1, 1]
-    uint32_t algo = PN_ALGO_AUTO;
+    // pruned tensor scan (tc_prune.cuh): tile balls and the build-time estimate of what pruning can do
+    DevBuf d_tcen, d_trad;
+    double prune_frac = 0.0;      // estimated fraction of (query group, tile) pairs that are out of reach
+    double seed_candidates = 0.0; // estimated candidates per query that survive a seed threshold
+    double tile_frac = 0.0;       // estimated share of tiles beyond a single query's seed
+    bool prune_on = false, tiles_on = false;   // prune_on: sorted + seeded scan; tiles_on: with tile bitmaps
+    // Vantage-point trees: the tensor path never used the VP bounds (a dense scan over the stored order), and the VP order
+    // -- shells around vantage points -- gives tiles that no ball can bound tightly.  A VP tree with a device therefore
+    // also keeps the BALL partition of the same points (built on the device) and answers tensor-path queries from it:
+    // exact 1-NN does not depend on the partition; the VP arrays serve the pruned SIMT traversal (PN_ALGO_SIMT), the layout
+    // accessors and trees the tensor path does not take (f64, d < 16).
+    // Ball trees (and the ball partition of a VP tree) on CLUSTERED data: the reference's split -- the median of the
+    // widest coordinate -- cuts through clusters, so in d >= 32 most 128-row tiles of the stored order mix fragments of
+    // several clusters and no ball bounds them tightly (BASELINE config 3: 88 % of all (query group, tile) pairs stay).
+    // Such a tree keeps a second ball tree over the same rows, partitioned by the TWO-MEANS rule of gpu_build.cu
+    // (partition_rule 1), and answers its k-NN batches from it: exact results do not depend on the partition, the tile
+    // bitmaps of tc_prune.cuh do.  two_means_partition() decides from the build-time estimates of both partitions.
+    // `part` is set when the tree is built, or once later by companion(); read it with partition().
+    std::shared_ptr<DeviceTree> part;
+    std::mutex part_mu;           // serialises companion() builds
+    uint32_t partition_rule = 0;  // gb::build_ball_tree rule of THIS tree's arrays
+    static constexpr uint32_t TWO_MEANS_ORDER_LEVELS = 1;
 
-    ~Engine() override {
-        if (!host_only) {
-            DeviceGuard g(device);
-            for (DevBuf* b : {&d_pts, &d_ids, &d_blo, &d_bhi, &d_centers, &d_radii, &d_vpids, &d_plane_w, &d_plane_t, &w_qraw, &w_q, &w_home,
-                              &w_hist, &w_cursor, &w_order, &w_part_d, &w_part_i, &w_floor_d, &w_floor_i, &w_counters,
-                              &w_out_i, &w_out_d, &w_counts, &w_offsets, &w_hits, &d_baug, &d_center, &w_aaug, &w_qmargin, &w_trace, &w_gbound,
-                              &d_tcen, &d_trad, &w_qs, &w_seed, &w_bits, &w_tcnt,
-                              &w_bcen, &w_brad, &w_bmu, &w_qth, &w_bbits, &w_bcnt, &w_wslot, &w_wlist, &w_wbits, &w_nwide})
-                b->release();
-            for (auto& e : ev) if (e) cudaEventDestroy(e);
-            for (int i = 0; i < 2; ++i) {
-                if (pin_stage[i]) cudaFreeHost(pin_stage[i]);
-                if (pin_ev[i]) cudaEventDestroy(pin_ev[i]);
-                w_qraw2[i].release(); w_oi2[i].release(); w_od2[i].release();
-                r_qraw[i].release(); r_q[i].release(); r_counts[i].release(); r_offsets[i].release(); r_hits[i].release(); r_sums[i].release();
-                r_slab[i].release(); r_qlist[i].release(); r_nlist[i].release();
-                sh_li[i].release(); sh_ld[i].release(); sh_pack[i].release(); sh_gat[i].release(); sh_gat_d[i].release();
-                for (cudaEvent_t e : {e_in[i], e_cmp[i], e_out[i]}) if (e) cudaEventDestroy(e);
-            }
-            for (cudaEvent_t e : sh_ev) cudaEventDestroy(e);
-            if (pin_tot) cudaFreeHost(pin_tot);
-            if (s_in) cudaStreamDestroy(s_in);
-            if (s_out) cudaStreamDestroy(s_out);
-            if (stream) cudaStreamDestroy(stream);
-        }
-    }
-
-    int open_device() {
-        CU(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, device));
-        CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        for (auto& e : ev) CU(cudaEventCreate(&e));
-        return PN_OK;
-    }
+    std::shared_ptr<DeviceTree> partition() const { return std::atomic_load(&part); }
 
     // ---- device-side construction (gpu_build.cu): raw rows on the device -> the same arrays upload() would have sent
     static gb::BallOut<A> alloc_tree_arrays(void* ctx, uint64_t n, const gb::TreeShape& shape) {
-        Engine* e = static_cast<Engine*>(ctx);
+        DeviceTree* e = static_cast<DeviceTree*>(ctx);
         FlatTree<A>& t = e->ft;
         t.kind = 0; t.n = n;
         t.dpad = (uint32_t)((t.d + VT<A>::N - 1) / VT<A>::N * VT<A>::N);
@@ -248,7 +219,7 @@ struct Engine final : pn_tree {
         return o;
     }
     static gb::VpOut<A> alloc_vp_arrays(void* ctx, uint64_t n, const gb::VpShape& shape) {
-        Engine* e = static_cast<Engine*>(ctx);
+        DeviceTree* e = static_cast<DeviceTree*>(ctx);
         FlatTree<A>& t = e->ft;
         t.kind = 1; t.n = n; t.n_total = n;
         t.dpad = (uint32_t)((t.d + VT<A>::N - 1) / VT<A>::N * VT<A>::N);
@@ -266,31 +237,29 @@ struct Engine final : pn_tree {
         return o;
     }
     // vantage-point tree on the device (gb::build_vp_tree): the same arrays the host VpBuilder + upload() produce
-    int build_vp_on_device(const A* raw_dev, size_t n, size_t d, size_t stride, uint32_t bucket) {
+    int build_vp_on_device(const A* raw_dev, size_t n, size_t d, size_t stride, uint32_t bucket, cudaStream_t st) {
         DeviceGuard g(device);
         if (!g.ok) return fail(PN_CUDA, "no usable CUDA device (there is no CPU fallback)");
-        TRY(open_device());
         ft.d = (uint32_t)d;
         gb::VpShape shape;
         std::string err;
-        const int rc = gb::build_vp_tree<A>(raw_dev, n, (uint32_t)d, stride, bucket, shape, &Engine::alloc_vp_arrays, this, stream, err);
+        const int rc = gb::build_vp_tree<A>(raw_dev, n, (uint32_t)d, stride, bucket, shape, &DeviceTree::alloc_vp_arrays, this, st, err);
         if (rc) return fail(rc == (int)cudaErrorMemoryAllocation ? PN_OOM : PN_CUDA, "device tree build: " + err);
         gpu_built = true;
         TRY(d_blo.ensure(ft.bucket_lo.size() * 4));
         TRY(d_bhi.ensure(ft.bucket_hi.size() * 4));
         CU(cudaMemcpy(d_blo.p, ft.bucket_lo.data(), ft.bucket_lo.size() * 4, cudaMemcpyHostToDevice));
         CU(cudaMemcpy(d_bhi.p, ft.bucket_hi.data(), ft.bucket_hi.size() * 4, cudaMemcpyHostToDevice));
-        info.device_bytes = d_pts.cap + d_ids.cap + d_blo.cap + d_bhi.cap + d_centers.cap + d_radii.cap + d_vpids.cap;
+        bytes = d_pts.cap + d_ids.cap + d_blo.cap + d_bhi.cap + d_centers.cap + d_radii.cap + d_vpids.cap;
         fill_dev_tree();
-        TRY(prepare_tensor());
+        TRY(prepare_tensor(st));
         return PN_OK;
     }
 
     int build_on_device(const A* raw_dev, size_t n_all, size_t d, size_t stride, uint32_t bucket, uint32_t shard_depth, uint32_t shard_index,
-                        uint32_t rule = 0) {
+                        uint32_t rule, cudaStream_t st) {
         DeviceGuard g(device);
         if (!g.ok) return fail(PN_CUDA, "no usable CUDA device (there is no CPU fallback)");
-        TRY(open_device());
         ft.d = (uint32_t)d; ft.n_total = n_all;
         partition_rule = rule;
         gb::TreeShape shape;
@@ -299,7 +268,7 @@ struct Engine final : pn_tree {
         // two-means partition: the rows of a bucket follow one more level of the split (a bucket is about two tiles of the
         // tensor path's point image)
         const int rc = gb::build_ball_tree<A>(raw_dev, n_all, (uint32_t)d, stride, bucket, shard_depth, shard_index, shape, &n,
-                                              &Engine::alloc_tree_arrays, this, stream, err, rule, rule == 1 ? TWO_MEANS_ORDER_LEVELS : 0u);
+                                              &DeviceTree::alloc_tree_arrays, this, st, err, rule, rule == 1 ? TWO_MEANS_ORDER_LEVELS : 0u);
         if (rc) return fail(rc == (int)cudaErrorMemoryAllocation ? PN_OOM : PN_CUDA, "device tree build: " + err);
         if (n == 0) return fail(PN_EMPTY, "shard holds no points");
         gpu_built = true;
@@ -308,16 +277,15 @@ struct Engine final : pn_tree {
         TRY(d_vpids.ensure(16));
         CU(cudaMemcpy(d_blo.p, ft.bucket_lo.data(), ft.bucket_lo.size() * 4, cudaMemcpyHostToDevice));
         CU(cudaMemcpy(d_bhi.p, ft.bucket_hi.data(), ft.bucket_hi.size() * 4, cudaMemcpyHostToDevice));
-        info.device_bytes = d_pts.cap + d_ids.cap + d_blo.cap + d_bhi.cap + d_centers.cap + d_radii.cap + d_vpids.cap + d_plane_w.cap + d_plane_t.cap;
+        bytes = d_pts.cap + d_ids.cap + d_blo.cap + d_bhi.cap + d_centers.cap + d_radii.cap + d_vpids.cap + d_plane_w.cap + d_plane_t.cap;
         fill_dev_tree();
-        TRY(prepare_tensor());
+        TRY(prepare_tensor(st));
         return PN_OK;
     }
 
-    int upload() {
+    int upload(cudaStream_t st) {
         DeviceGuard g(device);
         if (!g.ok) return fail(PN_CUDA, "no usable CUDA device (there is no CPU fallback)");
-        TRY(open_device());
         auto up = [&](DevBuf& b, const void* src, size_t bytes) -> int {
             TRY(b.ensure(bytes ? bytes : 16));
             if (bytes) CU(cudaMemcpy(b.p, src, bytes, cudaMemcpyHostToDevice));
@@ -330,9 +298,9 @@ struct Engine final : pn_tree {
         TRY(up(d_centers, ft.centers.data(), ft.centers.size() * sizeof(A)));
         TRY(up(d_radii, ft.radii.data(), ft.radii.size() * sizeof(A)));
         TRY(up(d_vpids, ft.vp_ids.data(), ft.vp_ids.size() * 4));
-        info.device_bytes = d_pts.cap + d_ids.cap + d_blo.cap + d_bhi.cap + d_centers.cap + d_radii.cap + d_vpids.cap;
+        bytes = d_pts.cap + d_ids.cap + d_blo.cap + d_bhi.cap + d_centers.cap + d_radii.cap + d_vpids.cap;
         fill_dev_tree();
-        TRY(prepare_tensor());
+        TRY(prepare_tensor(st));
         std::vector<A>().swap(ft.pts);  // the device copy is the point store from here on
         return PN_OK;
     }
@@ -350,63 +318,9 @@ struct Engine final : pn_tree {
         dt.slack = (A)((2.0 * ft.d + 8.0) * u);
     }
 
-    // ------------------------------------------------------------------------------------------
-    template <int DVR, int K, int KIND>
-    int launch_knn_t(const KnnArgs<A>& a, dim3 grid, cudaStream_t st) {
-        size_t smem = DVR < 0 ? 0 : 2 * TILE_BYTES + (DVR == 0 ? (size_t)TQ * ft.dpad * sizeof(A) : 0);
-        auto kern = knn_tile_kernel<A, DVR, K, KIND>;
-        if (smem > 32 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<grid, TQ, smem, st>>>(a);
-        CU(cudaGetLastError());
-        return PN_OK;
-    }
-    template <int K, int KIND>
-    int launch_knn_k(const KnnArgs<A>& a, dim3 grid, cudaStream_t st) {
-        switch (dt.dv) {
-            case 1: return launch_knn_t<1, K, KIND>(a, grid, st);
-            case 2: return launch_knn_t<2, K, KIND>(a, grid, st);
-            case 4: return launch_knn_t<4, K, KIND>(a, grid, st);
-            case 8: return launch_knn_t<8, K, KIND>(a, grid, st);
-            default:
-                if ((size_t)ft.dpad * sizeof(A) > 1024) return launch_knn_t<-1, K, KIND>(a, grid, st);  // wide rows: unstaged
-                return launch_knn_t<0, K, KIND>(a, grid, st);
-        }
-    }
-    int launch_knn(const KnnArgs<A>& a, dim3 grid, cudaStream_t st, bool k1) {
-        if (ft.kind == 0) return k1 ? launch_knn_k<1, 0>(a, grid, st) : launch_knn_k<16, 0>(a, grid, st);
-        return k1 ? launch_knn_k<1, 1>(a, grid, st) : launch_knn_k<16, 1>(a, grid, st);
-    }
-
-
-    // ------------------------------------------------------------------------------------------
-    // tensor path set-up (f32, d >= 8 worth of contraction): centred, augmented B operand + its TMA map
-    typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                      const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-    static EncodeTiledFn encode_fn() {
-        static EncodeTiledFn fn = [] {
-            void* p = nullptr;
-            cudaDriverEntryPointQueryResult q;
-            if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess) { (void)cudaGetLastError(); p = nullptr; }
-            return (EncodeTiledFn)p;
-        }();
-        return fn;
-    }
-    int make_map(CUtensorMap* m, void* base, uint64_t rows, uint32_t box_rows) {
-        EncodeTiledFn fn = encode_fn();
-        if (!fn) return fail(PN_CUDA, "cuTensorMapEncodeTiled entry point not found");
-        cuuint64_t dims[2] = {kp, rows};
-        cuuint64_t strides[1] = {(cuuint64_t)kp * 2};
-        cuuint32_t box[2] = {(cuuint32_t)tc::KC, (cuuint32_t)box_rows};
-        cuuint32_t estr[2] = {1, 1};
-        CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(PN_CUDA, "cuTensorMapEncodeTiled failed with code " + std::to_string((int)r));
-        return PN_OK;
-    }
     // the resident A operand (nkc chunks of 8 KB per 128-query subtile) must fit shared memory: Kp <= 384
     bool tensor_eligible() const { return sizeof(A) == 4 && algo != PN_ALGO_SIMT && (algo == PN_ALGO_TENSOR || ft.d >= 16) && ft.d + tc::NSLOT <= 384; }
-    int prepare_tensor() {
+    int prepare_tensor(cudaStream_t st) {
         if constexpr (sizeof(A) == 4) {
             if (!tensor_eligible()) return PN_OK;
             kp = (ft.d + tc::NSLOT + tc::KC - 1) / tc::KC * tc::KC;
@@ -419,7 +333,7 @@ struct Engine final : pn_tree {
             TRY(d_center.ensure(ft.dpad * 4));
             if (gpu_built) {
                 std::string err;
-                if (gb::centre_and_range_f32(d_pts.as<float>(), ft.n, ft.d, ft.dpad, d_center.as<float>(), c.data(), &maxabs, stream, err))
+                if (gb::centre_and_range_f32(d_pts.as<float>(), ft.n, ft.d, ft.dpad, d_center.as<float>(), c.data(), &maxabs, st, err))
                     return fail(PN_CUDA, "tensor path set-up: " + err);
             } else {
                 const size_t CH = 4096, n_ch = (ft.n + CH - 1) / CH;
@@ -458,32 +372,33 @@ struct Engine final : pn_tree {
             if (!std::isnormal(tscale) || !std::isnormal(tscale * tscale) || !std::isfinite(maxabs)) { tensor_ready = false; return PN_OK; }
             const size_t baug_bytes = (ft.n + tc::BN - 1) / tc::BN * tc::BN * (size_t)kp * 2;  // whole tiles
             TRY(d_baug.ensure(baug_bytes));
-            CU(cudaMemsetAsync(d_baug.p, 0, baug_bytes, stream));
-            TRY(w_counters.ensure(256));
-            CU(cudaMemset(w_counters.p, 0, 256));
-            tc::build_baug_kernel<<<(unsigned)((ft.n + 127) / 128), 128, 0, stream>>>(d_pts.as<float>(), d_center.as<float>(), tscale, (uint32_t)ft.n, ft.d,
-                                                                                     ft.dpad, kp, d_baug.as<__half>(), w_counters.as<unsigned int>());
+            CU(cudaMemsetAsync(d_baug.p, 0, baug_bytes, st));
+            DevBuf cnt;   // device-side results of the set-up kernels
+            TRY(cnt.ensure(256));
+            CU(cudaMemset(cnt.p, 0, 256));
+            tc::build_baug_kernel<<<(unsigned)((ft.n + 127) / 128), 128, 0, st>>>(d_pts.as<float>(), d_center.as<float>(), tscale, (uint32_t)ft.n, ft.d,
+                                                                                     ft.dpad, kp, d_baug.as<__half>(), cnt.as<unsigned int>());
             CU(cudaGetLastError());
             unsigned int bits = 0;
-            CU(cudaMemcpyAsync(&bits, w_counters.p, 4, cudaMemcpyDeviceToHost, stream));
-            CU(cudaStreamSynchronize(stream));
+            CU(cudaMemcpyAsync(&bits, cnt.p, 4, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
             memcpy(&pmax, &bits, 4);
-            info.device_bytes += d_baug.cap;
+            bytes += d_baug.cap;
             tensor_ready = true;
             // tile balls for the pruned scan, and the estimate that decides whether pruning is worth its set-up passes
             const uint32_t n_tiles = (uint32_t)((ft.n + tc::BN - 1) / tc::BN);
             TRY(d_tcen.ensure((size_t)n_tiles * ft.dpad * 4));
             TRY(d_trad.ensure((size_t)n_tiles * 4));
-            tc::tile_balls_kernel<<<n_tiles, 128, ft.dpad * 4, stream>>>(d_pts.as<float>(), (uint32_t)ft.n, ft.d, ft.dpad, d_tcen.as<float>(), d_trad.as<float>());
+            tc::tile_balls_kernel<<<n_tiles, 128, ft.dpad * 4, st>>>(d_pts.as<float>(), (uint32_t)ft.n, ft.d, ft.dpad, d_tcen.as<float>(), d_trad.as<float>());
             CU(cudaGetLastError());
-            CU(cudaMemsetAsync(w_counters.p, 0, 256, stream));
+            CU(cudaMemsetAsync(cnt.p, 0, 256, st));
             const uint32_t n_samples = std::min<uint32_t>(64u, n_tiles);
-            tc::prune_estimate_kernel<<<n_samples, 256, 0, stream>>>(d_tcen.as<float>(), d_trad.as<float>(), n_tiles, ft.dpad, n_samples,
-                                                                     w_counters.as<unsigned long long>());
+            tc::prune_estimate_kernel<<<n_samples, 256, 0, st>>>(d_tcen.as<float>(), d_trad.as<float>(), n_tiles, ft.dpad, n_samples,
+                                                                     cnt.as<unsigned long long>());
             CU(cudaGetLastError());
             unsigned long long est[2] = {0, 0};
-            CU(cudaMemcpyAsync(est, w_counters.p, 16, cudaMemcpyDeviceToHost, stream));
-            CU(cudaStreamSynchronize(stream));
+            CU(cudaMemcpyAsync(est, cnt.p, 16, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
             prune_frac = est[1] ? (double)est[0] / (double)est[1] : 0.0;
             // ... and whether seeding is: candidates a query still reranks when it starts from its home-bucket seed
             {
@@ -497,16 +412,14 @@ struct Engine final : pn_tree {
                 }
                 DevBuf sr, sb;
                 TRY(sr.ensure(S * 4)); TRY(sb.ensure(S * 4));
-                CU(cudaMemcpyAsync(sr.p, rows.data(), S * 4, cudaMemcpyHostToDevice, stream));
-                CU(cudaMemcpyAsync(sb.p, bks.data(), S * 4, cudaMemcpyHostToDevice, stream));
-                tc::seed_estimate_kernel<<<S, 256, 0, stream>>>(*reinterpret_cast<DevTree<float>*>(&dt), sr.as<uint32_t>(), sb.as<uint32_t>(), M,
-                                                               d_tcen.as<float>(), d_trad.as<float>(), n_tiles, w_counters.as<unsigned long long>());
-                cudaError_t ke = cudaGetLastError();
+                CU(cudaMemcpyAsync(sr.p, rows.data(), S * 4, cudaMemcpyHostToDevice, st));
+                CU(cudaMemcpyAsync(sb.p, bks.data(), S * 4, cudaMemcpyHostToDevice, st));
+                tc::seed_estimate_kernel<<<S, 256, 0, st>>>(*reinterpret_cast<DevTree<float>*>(&dt), sr.as<uint32_t>(), sb.as<uint32_t>(), M,
+                                                               d_tcen.as<float>(), d_trad.as<float>(), n_tiles, cnt.as<unsigned long long>());
+                CU(cudaGetLastError());
                 unsigned long long se[4] = {0, 0, 0, 0};
-                if (ke == cudaSuccess) ke = cudaMemcpyAsync(se, (char*)w_counters.p + 16, 32, cudaMemcpyDeviceToHost, stream);
-                if (ke == cudaSuccess) ke = cudaStreamSynchronize(stream);
-                sr.release(); sb.release();
-                if (ke != cudaSuccess) return fail(PN_CUDA, std::string("seed estimate: ") + cudaGetErrorString(ke));
+                CU(cudaMemcpyAsync(se, (char*)cnt.p + 16, 32, cudaMemcpyDeviceToHost, st));
+                CU(cudaStreamSynchronize(st));
                 seed_candidates = se[1] ? (double)se[0] / (double)se[1] * (double)ft.n : (double)ft.n;
                 tile_frac = se[3] ? (double)se[2] / (double)se[3] : 0.0;
             }
@@ -517,31 +430,11 @@ struct Engine final : pn_tree {
             // tile bitmaps: worth their pass when a single query could skip most tiles (a CTA needs the union over its queries)
             tiles_on = can && (prune_opt == PN_PRUNE_ON || (prune_opt == PN_PRUNE_AUTO && (prune_frac >= 0.25 || tile_frac >= 0.6)));
             prune_on = can && (tiles_on || (prune_opt == PN_PRUNE_AUTO && seed_candidates <= 4.0 * stream_candidates));
-            info.device_bytes += d_tcen.cap + d_trad.cap;
+            bytes += d_tcen.cap + d_trad.cap;
         }
         return PN_OK;
     }
 
-    static constexpr size_t filter_fixed_smem(int mt, uint32_t k) {
-        // alignment slack + barriers / TMEM slot + per-warp queues + per-warp top-k lists (k entries per query)
-        return 1024 + 1024 + (size_t)4 * mt * 192 * 4 + (size_t)4 * mt * k * 32 * 8;
-    }
-    template <int DVR, int K, int MT, int NACC, int SW = tc::BN>
-    int launch_filter_t(const CUtensorMap& map_a, const tc::FilterArgs& fa, cudaStream_t st) {
-        if (fa.tile_bits) return launch_filter_s<DVR, K, MT, NACC, false, SW, true>(map_a, fa, st);
-        return fa.g_bound ? launch_filter_s<DVR, K, MT, NACC, true, SW, false>(map_a, fa, st) : launch_filter_s<DVR, K, MT, NACC, false, SW, false>(map_a, fa, st);
-    }
-    template <int DVR, int K, int MT, int NACC, bool SHARED, int SW, bool PRUNE>
-    int launch_filter_s(const CUtensorMap& map_a, const tc::FilterArgs& fa, cudaStream_t st) {
-        const size_t smem = filter_fixed_smem(MT, fa.k) + (size_t)MT * fa.nkc * tc::A_CHUNK_BYTES + (size_t)fa.stages * fa.gs * tc::CHUNK_BYTES;
-        auto kern = tc::knn_filter_kernel<DVR, K, MT, NACC, SHARED, SW, PRUNE>;
-        CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        const unsigned gx = (fa.nq - fa.row0 + MT * tc::BM - 1) / (MT * tc::BM);
-        const unsigned gy = PRUNE ? 1u : (fa.n_tiles + fa.tiles_per_split - 1) / fa.tiles_per_split;
-        kern<<<dim3(gx, gy), (5 * MT + 2) * 32, smem, st>>>(map_a, d_baug.as<unsigned char>(), fa);
-        CU(cudaGetLastError());
-        return PN_OK;
-    }
     // subtiles per CTA: 4 (one accumulator stage each) for narrow rows, where the epilogue is the bound; 2 (two
     // stages each) where the tensor pipe is; 1 when the resident A operand of two subtiles no longer fits
     int filter_subtiles(uint32_t nkc) const {
@@ -560,14 +453,276 @@ struct Engine final : pn_tree {
 #endif
         return nkc <= 3 ? 4 : (nkc <= 6 ? 2 : 1);
     }
-    // queries per CTA of the scan this handle (or the ball tree behind a vantage-point handle) runs
+    // queries per CTA of the scan a k-NN batch on this tree runs (on the partition, when there is one)
     size_t query_tile() const {
-        const Engine* e = aux ? aux.get() : this;
-        return e->tensor_ready ? (size_t)128 * e->filter_subtiles(e->kp / tc::KC) : 512;
+        const auto p = partition();
+        const DeviceTree& s = p ? *p : *this;
+        return s.tensor_ready ? (size_t)128 * s.filter_subtiles(s.kp / tc::KC) : 512;
+    }
+
+    // A ball tree over the points of this tree, for `part`.  `rows` (n x d, row stride `stride`) are either the
+    // original-order rows or this tree's stored rows (d_pts); then the new tree's ids (positions in this tree's stored
+    // order) are translated to the original point indices.
+    int build_partition(const A* rows, size_t stride, uint32_t bucket, uint32_t rule, cudaStream_t st, std::shared_ptr<DeviceTree>& out) const {
+        auto p = std::make_shared<DeviceTree>();
+        p->device = device; p->algo = algo; p->prune_opt = prune_opt;
+        TRY(p->build_on_device(rows, ft.n, ft.d, stride, bucket, 0, 0, rule, st));
+        if (rows == d_pts.as<A>()) {
+            translate_ids_kernel<<<(unsigned)((ft.n + 255) / 256), 256, 0, st>>>(p->d_ids.template as<uint32_t>(), d_ids.as<uint32_t>(), (uint32_t)ft.n);
+            CU(cudaGetLastError());
+            CU(cudaStreamSynchronize(st));
+        }
+        p->ft.n_total = ft.n_total;
+        out = std::move(p);
+        return PN_OK;
+    }
+
+    // A second ball tree over this tree's stored rows, split by the two-means rule, when that pays (see `part`):
+    // AUTO tries it where seeding already pays and the tile balls of the reference partition leave a single query more than
+    // a tenth of the tiles, and keeps it when its own estimates turn the bitmaps on and a single query can skip at least a
+    // tenth of all tiles more; PN_PARTITION_TWO_MEANS keeps it regardless.  Returns the new
+    // tree in `out` (null: stay with this partition); a failure on the way only loses the speed-up.
+    void two_means_partition(uint32_t partition_opt, uint32_t bucket, cudaStream_t st, std::shared_ptr<DeviceTree>& out) const {
+        out.reset();
+        if constexpr (sizeof(A) == 4) {
+            if (partition_opt == PN_PARTITION_REFERENCE || ft.kind != 0 || !tensor_ready || ft.n != ft.n_total) return;
+            const bool forced = partition_opt == PN_PARTITION_TWO_MEANS;
+            // AUTO: seeding pays (clustered data), a single query could skip some tiles but not nearly all of them
+            if (forced ? ft.n < 1024 : !(ft.n >= 32768 && prune_opt == PN_PRUNE_AUTO && prune_on && tile_frac >= 0.1 && tile_frac < 0.9)) return;
+            DeviceGuard g(device);
+            if (!g.ok) return;
+            std::shared_ptr<DeviceTree> tm;
+            if (build_partition(d_pts.as<A>(), ft.dpad, bucket, 1, st, tm) != PN_OK || !tm->tensor_ready) { (void)cudaGetLastError(); return; }
+            if (forced || (tm->tiles_on && tm->tile_frac >= tile_frac + 0.1)) out = std::move(tm);
+        }
+    }
+
+    // A vantage-point tree's ball partition of the same points (`part`).  Tensor-eligible trees get it when they are
+    // created; the others on the first query the VP arrays do not serve (radius search), whichever handle of the tree asks
+    // first: built once, on the device, from the stored rows.  A failed build publishes nothing.
+    int companion(cudaStream_t st, std::shared_ptr<DeviceTree>& out) {
+        out = partition();
+        if (out) return PN_OK;
+        std::lock_guard<std::mutex> lk(part_mu);
+        out = partition();
+        if (out) return PN_OK;
+        TRY(build_partition(d_pts.as<A>(), ft.dpad, 256, 0, st, out));
+        std::atomic_store(&part, out);
+        return PN_OK;
+    }
+
+    // ---- replication of the flattened tree over NCCL (query sharding: build once, broadcast) ------------------------------
+    struct ReplicaHeader {
+        uint64_t n, n_total;
+        uint32_t d, dpad, L, n_internal, n_buckets, n_nodes, bucket_max, kp;
+        int32_t kind;
+        uint32_t algo, tensor_ready, prune_on;
+        float pmax, tscale;
+    };
+    std::vector<std::pair<DevBuf*, size_t>> replica_arrays() {
+        std::vector<std::pair<DevBuf*, size_t>> v = {
+            {&d_pts, (size_t)ft.n * ft.dpad * sizeof(A)}, {&d_ids, (size_t)ft.n * 4}, {&d_blo, (size_t)ft.n_buckets * 4}, {&d_bhi, (size_t)ft.n_buckets * 4},
+            {&d_centers, (size_t)std::max<uint32_t>(ft.n_nodes, 1) * ft.dpad * sizeof(A)}, {&d_radii, (size_t)std::max<uint32_t>(ft.n_nodes, 1) * sizeof(A)},
+            {&d_vpids, ft.kind == 1 ? (size_t)std::max<uint32_t>(ft.n_nodes, 1) * 4 : 16}};
+        if (partition_rule == 1 && ft.n_internal) {   // (never replicated: a tree's second partition stays on its device)
+            v.push_back({&d_plane_w, (size_t)ft.n_internal * ft.dpad * sizeof(A)});
+            v.push_back({&d_plane_t, (size_t)ft.n_internal * sizeof(A)});
+        }
+        if (tensor_ready) {
+            v.push_back({&d_center, (size_t)ft.dpad * 4});
+            v.push_back({&d_baug, (ft.n + tc::BN - 1) / tc::BN * tc::BN * (size_t)kp * 2});
+            const size_t n_tiles = (ft.n + tc::BN - 1) / tc::BN;
+            v.push_back({&d_tcen, n_tiles * ft.dpad * 4});
+            v.push_back({&d_trad, n_tiles * 4});
+        }
+        return v;
+    }
+    int replicate_send(pn_comm* cm, int root) {
+        ReplicaHeader h{ft.n, ft.n_total, ft.d, ft.dpad, ft.L, ft.n_internal, ft.n_buckets, ft.n_nodes, ft.bucket_max, kp, ft.kind, algo,
+                        tensor_ready ? 1u : 0u, (prune_on ? 1u : 0u) | (tiles_on ? 2u : 0u), pmax, tscale};
+        DevBuf hb;
+        TRY(hb.ensure(sizeof(h)));
+        CU(cudaMemcpyAsync(hb.p, &h, sizeof(h), cudaMemcpyHostToDevice, cm->stream));
+        NC(cm->api->Broadcast(hb.p, hb.p, sizeof(h), ncclUint8, root, cm->comm, cm->stream));
+        for (auto& a : replica_arrays()) NC(cm->api->Broadcast(a.first->p, a.first->p, a.second, ncclUint8, root, cm->comm, cm->stream));
+        CU(cudaStreamSynchronize(cm->stream));
+        return PN_OK;
+    }
+    int replicate_recv(pn_comm* cm, int root) {
+        device = cm->device;
+        DeviceGuard g(device);
+        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
+        ReplicaHeader h{};
+        DevBuf hb;
+        TRY(hb.ensure(sizeof(h)));
+        NC(cm->api->Broadcast(hb.p, hb.p, sizeof(h), ncclUint8, root, cm->comm, cm->stream));
+        CU(cudaMemcpyAsync(&h, hb.p, sizeof(h), cudaMemcpyDeviceToHost, cm->stream));
+        CU(cudaStreamSynchronize(cm->stream));
+        ft.n = h.n; ft.n_total = h.n_total; ft.d = h.d; ft.dpad = h.dpad; ft.L = h.L; ft.n_internal = h.n_internal; ft.n_buckets = h.n_buckets;
+        ft.n_nodes = h.n_nodes; ft.bucket_max = h.bucket_max; ft.kind = h.kind; kp = h.kp; algo = h.algo; tensor_ready = h.tensor_ready != 0;
+        pmax = h.pmax; tscale = h.tscale; prune_on = (h.prune_on & 1u) != 0; tiles_on = (h.prune_on & 2u) != 0;
+        gpu_built = true;  // no host copies: layout() reads the device arrays
+        bytes = 0;
+        for (auto& a : replica_arrays()) {
+            TRY(a.first->ensure(a.second));
+            NC(cm->api->Broadcast(a.first->p, a.first->p, a.second, ncclUint8, root, cm->comm, cm->stream));
+            bytes += a.first->cap;
+        }
+        CU(cudaStreamSynchronize(cm->stream));
+        ft.bucket_lo.resize(ft.n_buckets); ft.bucket_hi.resize(ft.n_buckets);
+        CU(cudaMemcpy(ft.bucket_lo.data(), d_blo.p, (size_t)ft.n_buckets * 4, cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(ft.bucket_hi.data(), d_bhi.p, (size_t)ft.n_buckets * 4, cudaMemcpyDeviceToHost));
+        if (ft.kind == 1) {
+            ft.vp_ids.resize(std::max<uint32_t>(ft.n_nodes, 1));
+            CU(cudaMemcpy(ft.vp_ids.data(), d_vpids.p, ft.vp_ids.size() * 4, cudaMemcpyDeviceToHost));
+        }
+        fill_dev_tree();
+        return PN_OK;
+    }
+};
+
+template <typename A>
+struct Engine final : pn_tree {
+    using V = typename VT<A>::V;
+    // the tree this handle queries, shared with the handle's sessions (pn_tree_session) and never written after its build,
+    // except that DeviceTree::companion() may publish a partition
+    std::shared_ptr<DeviceTree<A>> tree;
+    bool owns_tree = true;   // false for a session: device_bytes are reported by the handle that built the tree
+    int n_sms = 148;
+    cudaStream_t stream = nullptr, last_stream = nullptr;
+    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    DevBuf w_qraw, w_q, w_home, w_hist, w_cursor, w_order, w_part_d, w_part_i, w_floor_d, w_floor_i,
+        w_counters, w_out_i, w_out_d, w_counts, w_offsets, w_hits;
+    // host-buffer calls are software-pipelined over chunks of queries: H2D of chunk i+1 and D2H of chunk i-1 run on their own
+    // streams under the kernels of chunk i (two sets of raw-query / result buffers)
+    cudaStream_t s_in = nullptr, s_out = nullptr;
+    cudaEvent_t e_in[2] = {nullptr, nullptr}, e_cmp[2] = {nullptr, nullptr}, e_out[2] = {nullptr, nullptr};
+    DevBuf w_qraw2[2], w_oi2[2], w_od2[2];
+    DevBuf sh_li[2], sh_ld[2], sh_pack[2], sh_gat[2], sh_gat_d[2];   // sharded k-NN: local lists, packed keys, gathered lists
+    std::vector<cudaEvent_t> sh_ev;                                    // timing events of the sharded pipeline (reused)
+    DevBuf r_qraw[2], r_q[2], r_counts[2], r_offsets[2], r_hits[2], r_slab[2], r_qlist[2], r_nlist[2], r_sums[2];  // radius pipeline workspaces
+    unsigned long long* pin_tot = nullptr;                            // pinned: chunk totals of the radius count pass
+    void* pin_stage[2] = {nullptr, nullptr};  // pinned D2H staging for the variable-length radius output
+    cudaEvent_t pin_ev[2] = {nullptr, nullptr};
+    static constexpr size_t PIN_BYTES = 16u << 20;
+    // tensor path (f32 input only): per-call workspaces, see tc_filter.cuh
+    DevBuf w_aaug, w_qmargin, w_trace, w_gbound;
+    bool last_used_tensor = false;
+    // pruned tensor scan (tc_prune.cuh): per-call workspaces
+    DevBuf w_qs, w_seed, w_bits, w_tcnt;
+    DevBuf w_bcen, w_brad, w_bmu, w_qth, w_bbits, w_bcnt, w_wslot, w_wlist, w_wbits, w_nwide;   // tile-bitmap pass: query balls, their bitmaps, wide balls
+    bool last_pruned = false, last_tiles = false;   // the last k-NN scan was seeded / also used tile bitmaps
+
+    explicit Engine(std::shared_ptr<DeviceTree<A>> t) : tree(std::move(t)) {}
+    ~Engine() override {
+        if (!host_only) {
+            DeviceGuard g(tree->device);
+            for (auto& e : ev) if (e) cudaEventDestroy(e);
+            for (int i = 0; i < 2; ++i) {
+                if (pin_stage[i]) cudaFreeHost(pin_stage[i]);
+                if (pin_ev[i]) cudaEventDestroy(pin_ev[i]);
+                for (cudaEvent_t e : {e_in[i], e_cmp[i], e_out[i]}) if (e) cudaEventDestroy(e);
+            }
+            for (cudaEvent_t e : sh_ev) cudaEventDestroy(e);
+            if (pin_tot) cudaFreeHost(pin_tot);
+            if (s_in) cudaStreamDestroy(s_in);
+            if (s_out) cudaStreamDestroy(s_out);
+            if (stream) cudaStreamDestroy(stream);
+        }
+    }
+
+    int open_device() {
+        DeviceGuard g(tree->device);
+        if (!g.ok) return fail(PN_CUDA, "no usable CUDA device (there is no CPU fallback)");
+        CU(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, tree->device));
+        CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+        for (auto& e : ev) CU(cudaEventCreate(&e));
+        return PN_OK;
+    }
+
+    uint64_t device_bytes() const override {
+        if (!owns_tree) return 0;
+        const auto p = tree->partition();
+        return tree->bytes + (p ? p->bytes : 0);
+    }
+
+    // ------------------------------------------------------------------------------------------
+    template <int DVR, int K, int KIND>
+    int launch_knn_t(const DeviceTree<A>& t, const KnnArgs<A>& a, dim3 grid, cudaStream_t st) {
+        size_t smem = DVR < 0 ? 0 : 2 * TILE_BYTES + (DVR == 0 ? (size_t)TQ * t.ft.dpad * sizeof(A) : 0);
+        auto kern = knn_tile_kernel<A, DVR, K, KIND>;
+        if (smem > 32 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        kern<<<grid, TQ, smem, st>>>(a);
+        CU(cudaGetLastError());
+        return PN_OK;
+    }
+    template <int K, int KIND>
+    int launch_knn_k(const DeviceTree<A>& t, const KnnArgs<A>& a, dim3 grid, cudaStream_t st) {
+        switch (t.dt.dv) {
+            case 1: return launch_knn_t<1, K, KIND>(t, a, grid, st);
+            case 2: return launch_knn_t<2, K, KIND>(t, a, grid, st);
+            case 4: return launch_knn_t<4, K, KIND>(t, a, grid, st);
+            case 8: return launch_knn_t<8, K, KIND>(t, a, grid, st);
+            default:
+                if ((size_t)t.ft.dpad * sizeof(A) > 1024) return launch_knn_t<-1, K, KIND>(t, a, grid, st);  // wide rows: unstaged
+                return launch_knn_t<0, K, KIND>(t, a, grid, st);
+        }
+    }
+    int launch_knn(const DeviceTree<A>& t, const KnnArgs<A>& a, dim3 grid, cudaStream_t st, bool k1) {
+        if (t.ft.kind == 0) return k1 ? launch_knn_k<1, 0>(t, a, grid, st) : launch_knn_k<16, 0>(t, a, grid, st);
+        return k1 ? launch_knn_k<1, 1>(t, a, grid, st) : launch_knn_k<16, 1>(t, a, grid, st);
+    }
+
+
+    // ------------------------------------------------------------------------------------------
+    // tensor path set-up (f32, d >= 8 worth of contraction): centred, augmented B operand + its TMA map
+    typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                      const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+    static EncodeTiledFn encode_fn() {
+        static EncodeTiledFn fn = [] {
+            void* p = nullptr;
+            cudaDriverEntryPointQueryResult q;
+            if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess) { (void)cudaGetLastError(); p = nullptr; }
+            return (EncodeTiledFn)p;
+        }();
+        return fn;
+    }
+    static int make_map(CUtensorMap* m, void* base, uint64_t rows, uint32_t box_rows, uint32_t kp) {
+        EncodeTiledFn fn = encode_fn();
+        if (!fn) return fail(PN_CUDA, "cuTensorMapEncodeTiled entry point not found");
+        cuuint64_t dims[2] = {kp, rows};
+        cuuint64_t strides[1] = {(cuuint64_t)kp * 2};
+        cuuint32_t box[2] = {(cuuint32_t)tc::KC, (cuuint32_t)box_rows};
+        cuuint32_t estr[2] = {1, 1};
+        CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                        CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+        if (r != CUDA_SUCCESS) return fail(PN_CUDA, "cuTensorMapEncodeTiled failed with code " + std::to_string((int)r));
+        return PN_OK;
+    }
+    static constexpr size_t filter_fixed_smem(int mt, uint32_t k) {
+        // alignment slack + barriers / TMEM slot + per-warp queues + per-warp top-k lists (k entries per query)
+        return 1024 + 1024 + (size_t)4 * mt * 192 * 4 + (size_t)4 * mt * k * 32 * 8;
+    }
+    template <int DVR, int K, int MT, int NACC, int SW = tc::BN>
+    int launch_filter_t(const DeviceTree<A>& t, const CUtensorMap& map_a, const tc::FilterArgs& fa, cudaStream_t st) {
+        if (fa.tile_bits) return launch_filter_s<DVR, K, MT, NACC, false, SW, true>(t, map_a, fa, st);
+        return fa.g_bound ? launch_filter_s<DVR, K, MT, NACC, true, SW, false>(t, map_a, fa, st) : launch_filter_s<DVR, K, MT, NACC, false, SW, false>(t, map_a, fa, st);
+    }
+    template <int DVR, int K, int MT, int NACC, bool SHARED, int SW, bool PRUNE>
+    int launch_filter_s(const DeviceTree<A>& t, const CUtensorMap& map_a, const tc::FilterArgs& fa, cudaStream_t st) {
+        const size_t smem = filter_fixed_smem(MT, fa.k) + (size_t)MT * fa.nkc * tc::A_CHUNK_BYTES + (size_t)fa.stages * fa.gs * tc::CHUNK_BYTES;
+        auto kern = tc::knn_filter_kernel<DVR, K, MT, NACC, SHARED, SW, PRUNE>;
+        CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const unsigned gx = (fa.nq - fa.row0 + MT * tc::BM - 1) / (MT * tc::BM);
+        const unsigned gy = PRUNE ? 1u : (fa.n_tiles + fa.tiles_per_split - 1) / fa.tiles_per_split;
+        kern<<<dim3(gx, gy), (5 * MT + 2) * 32, smem, st>>>(map_a, t.d_baug.template as<unsigned char>(), fa);
+        CU(cudaGetLastError());
+        return PN_OK;
     }
     template <int K>
-    int launch_filter_k(const CUtensorMap& map_a, tc::FilterArgs& fa, cudaStream_t st) {
-        const int mt = filter_subtiles(fa.nkc);
+    int launch_filter_k(const DeviceTree<A>& t, const CUtensorMap& map_a, tc::FilterArgs& fa, cudaStream_t st) {
+        const int mt = t.filter_subtiles(fa.nkc);
         const size_t budget = 224 * 1024;
         // ring groups of 16 KB (one full/empty barrier pair per group): 2 tiles at Kp = 32, 1 tile at Kp = 64, chunks beyond
         fa.gs = fa.nkc == 1 ? 2 : (fa.nkc == 2 ? 2 : 1);
@@ -584,24 +739,24 @@ struct Engine final : pn_tree {
             if (getenv("PN_TC_HALF")) half = atoi(getenv("PN_TC_HALF")) != 0;
 #endif
             if (half) {
-                if (dt.dv == 4) return launch_filter_t<4, K, 4, 2, 64>(map_a, fa, st);
-                if (dt.dv == 8) return launch_filter_t<8, K, 4, 2, 64>(map_a, fa, st);
-                return launch_filter_t<0, K, 4, 2, 64>(map_a, fa, st);
+                if (t.dt.dv == 4) return launch_filter_t<4, K, 4, 2, 64>(t, map_a, fa, st);
+                if (t.dt.dv == 8) return launch_filter_t<8, K, 4, 2, 64>(t, map_a, fa, st);
+                return launch_filter_t<0, K, 4, 2, 64>(t, map_a, fa, st);
             }
-            if (dt.dv == 4) return launch_filter_t<4, K, 4, 1>(map_a, fa, st);
-            if (dt.dv == 8) return launch_filter_t<8, K, 4, 1>(map_a, fa, st);
-            return launch_filter_t<0, K, 4, 1>(map_a, fa, st);
+            if (t.dt.dv == 4) return launch_filter_t<4, K, 4, 1>(t, map_a, fa, st);
+            if (t.dt.dv == 8) return launch_filter_t<8, K, 4, 1>(t, map_a, fa, st);
+            return launch_filter_t<0, K, 4, 1>(t, map_a, fa, st);
         }
 #if defined(PN_TC_PROFILE) || defined(PN_TC_EXPERIMENTS)
         if (mt == 3) {
             // one chunk: two half-tile stages per subtile (3 x 2 x 64 accumulator columns + 3 x 16 operand columns)
-            if (fa.nkc == 1) return dt.dv == 4 ? launch_filter_t<4, K, 3, 2, 64>(map_a, fa, st) : launch_filter_t<0, K, 3, 2, 64>(map_a, fa, st);
-            return launch_filter_t<0, K, 3, 1>(map_a, fa, st);
+            if (fa.nkc == 1) return t.dt.dv == 4 ? launch_filter_t<4, K, 3, 2, 64>(t, map_a, fa, st) : launch_filter_t<0, K, 3, 2, 64>(t, map_a, fa, st);
+            return launch_filter_t<0, K, 3, 1>(t, map_a, fa, st);
         }
 #endif
         if (mt == 2) {
-            if (dt.dv == 4) return launch_filter_t<4, K, 2, 2>(map_a, fa, st);
-            if (dt.dv == 8) return launch_filter_t<8, K, 2, 2>(map_a, fa, st);
+            if (t.dt.dv == 4) return launch_filter_t<4, K, 2, 2>(t, map_a, fa, st);
+            if (t.dt.dv == 8) return launch_filter_t<8, K, 2, 2>(t, map_a, fa, st);
 #if defined(PN_TC_PROFILE) || defined(PN_TC_EXPERIMENTS)
             // Experiments (diagnostic builds): the A operand in tensor memory (TS-form MMA).  scripts/mma_rate.cu, two
             // issuers, cycles per 128 accumulator columns: SS N=128 86.5 (= the 64-cycle floor + 22 of operand fetch),
@@ -612,41 +767,41 @@ struct Engine final : pn_tree {
             //               (151 552 queries; profiles/r02_mma_rate.md).  Both bit-exact.
             {
                 static const int ts = getenv("PN_TC_TS") ? atoi(getenv("PN_TC_TS")) : 0;
-                if (ts == 1 && fa.nkc <= 8) return launch_filter_t<0, K, 2, 2, 64>(map_a, fa, st);
-                if (ts == 2) return launch_filter_t<0, K, 2, 1>(map_a, fa, st);
+                if (ts == 1 && fa.nkc <= 8) return launch_filter_t<0, K, 2, 2, 64>(t, map_a, fa, st);
+                if (ts == 2) return launch_filter_t<0, K, 2, 1>(t, map_a, fa, st);
             }
 #endif
-            return launch_filter_t<0, K, 2, 2>(map_a, fa, st);
+            return launch_filter_t<0, K, 2, 2>(t, map_a, fa, st);
         }
-        return launch_filter_t<0, K, 1, 2>(map_a, fa, st);
+        return launch_filter_t<0, K, 1, 2>(t, map_a, fa, st);
     }
 
     // Prepass of the seeded scans (k <= 16): queries sorted by home bucket (self query: the stored order is that order
     // already) and every query's seed threshold from its home bucket.  *qsorted: padded query rows in sorted order; *order:
     // sorted slot -> query id (null for the self query).
-    int sort_and_seed(const A* qraw, uint32_t nq, size_t stride, uint32_t k, cudaStream_t st, bool self_query, const float4** qsorted,
+    int sort_and_seed(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, uint32_t k, cudaStream_t st, bool self_query, const float4** qsorted,
                       const uint32_t** order) {
         if constexpr (sizeof(A) == 4) {
             *order = nullptr;
             TRY(w_home.ensure((size_t)nq * 4));
             if (self_query) {
-                TRY(w_hist.ensure((size_t)ft.n_buckets * 4));
-                home_bucket_kernel<A><<<(nq + 127) / 128, 128, 0, st>>>(dt, d_pts.as<V>(), nq, w_home.as<uint32_t>(), w_hist.as<uint32_t>());
+                TRY(w_hist.ensure((size_t)t.ft.n_buckets * 4));
+                home_bucket_kernel<A><<<(nq + 127) / 128, 128, 0, st>>>(t.dt, t.d_pts.template as<V>(), nq, w_home.as<uint32_t>(), w_hist.as<uint32_t>());
                 CU(cudaGetLastError());
                 ++counters.kernel_launches;
-                *qsorted = d_pts.as<float4>();
+                *qsorted = t.d_pts.template as<float4>();
             } else {
-                TRY(stage_queries(qraw, nq, stride, st, true));  // padded rows, home buckets, counting sort -> w_order
-                TRY(w_qs.ensure((size_t)nq * ft.dpad * 4));
-                const size_t tot = (size_t)nq * dt.dv;
-                tc::gather_queries_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(w_q.as<float4>(), w_order.as<uint32_t>(), nq, dt.dv, w_qs.as<float4>());
+                TRY(stage_queries(t, qraw, nq, stride, st, true));  // padded rows, home buckets, counting sort -> w_order
+                TRY(w_qs.ensure((size_t)nq * t.ft.dpad * 4));
+                const size_t tot = (size_t)nq * t.dt.dv;
+                tc::gather_queries_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(w_q.as<float4>(), w_order.as<uint32_t>(), nq, t.dt.dv, w_qs.as<float4>());
                 CU(cudaGetLastError());
                 ++counters.kernel_launches;
                 *qsorted = w_qs.as<float4>();
                 *order = w_order.as<uint32_t>();
             }
             TRY(w_seed.ensure((size_t)nq * 4));
-            const DevTree<float>& dtf = *reinterpret_cast<DevTree<float>*>(&dt);
+            const DevTree<float>& dtf = *reinterpret_cast<const DevTree<float>*>(&t.dt);
             tc::seed_bound_kernel<<<(nq + 7) / 8, 256, 0, st>>>(dtf, *qsorted, *order, w_home.as<uint32_t>(), nq, k, w_seed.as<float>());
             CU(cudaGetLastError());
             ++counters.kernel_launches;
@@ -660,13 +815,13 @@ struct Engine final : pn_tree {
     // Pruned tensor k-NN (tc_prune.cuh; k <= 16): queries sorted by home bucket, seed bounds from the home bucket, one tile
     // bitmap per CTA, then ONE launch of the filter over all query groups -- the groups have lists of very different
     // lengths, so the hardware block scheduler does the load balancing that whole waves do for the dense scan.
-    int knn_device_pruned(const A* qraw, uint32_t nq, size_t stride, uint32_t k, uint32_t kstride, uint64_t* idx_out, A* dist_out, cudaStream_t st,
+    int knn_device_pruned(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, uint32_t k, uint32_t kstride, uint64_t* idx_out, A* dist_out, cudaStream_t st,
                           bool self_query) {
         if constexpr (sizeof(A) == 4) {
             const bool k1 = (k == 1);
             const uint32_t KP = k1 ? 1 : 16;
-            const uint32_t n_tiles = (uint32_t)((ft.n + tc::BN - 1) / tc::BN), words = (n_tiles + 31) / 32;
-            const uint32_t QT = 128u * (uint32_t)filter_subtiles(kp / tc::KC), n_qt = (nq + QT - 1) / QT;
+            const uint32_t n_tiles = (uint32_t)((t.ft.n + tc::BN - 1) / tc::BN), words = (n_tiles + 31) / 32;
+            const uint32_t QT = 128u * (uint32_t)t.filter_subtiles(t.kp / tc::KC), n_qt = (nq + QT - 1) / QT;
             const float4* qsorted;
             const uint32_t* order = nullptr;
             CU(cudaEventRecord(ev[2], st));   // scan_ms covers the whole scan: sort + seeds, bitmaps, filter, merge
@@ -674,17 +829,17 @@ struct Engine final : pn_tree {
             static const bool stage_timing = getenv("PN_STAGE_TIMING") != nullptr;
             cudaEvent_t se[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
             if (stage_timing) { for (auto& e : se) CU(cudaEventCreate(&e)); CU(cudaEventRecord(se[0], st)); }
-            TRY(sort_and_seed(qraw, nq, stride, k, st, self_query, &qsorted, &order));
+            TRY(sort_and_seed(t, qraw, nq, stride, k, st, self_query, &qsorted, &order));
             if (stage_timing) CU(cudaEventRecord(se[1], st));
-            TRY(w_aaug.ensure((size_t)nq * kp * 2));
+            TRY(w_aaug.ensure((size_t)nq * t.kp * 2));
             TRY(w_qmargin.ensure((size_t)nq * 4));
             TRY(w_bits.ensure((size_t)n_qt * words * 4));
             TRY(w_tcnt.ensure((size_t)n_qt * 4));
             TRY(w_part_d.ensure((size_t)nq * KP * 4));
             TRY(w_part_i.ensure((size_t)nq * KP * 4));
-            const DevTree<float>& dtf = *reinterpret_cast<DevTree<float>*>(&dt);
-            tc::build_aaug_kernel<<<(nq + 127) / 128, 128, 0, st>>>(reinterpret_cast<const float*>(qsorted), d_center.as<float>(), tscale, nq, ft.d, ft.dpad,
-                                                                    kp, pmax, w_aaug.as<__half>(), w_qmargin.as<float>());
+            const DevTree<float>& dtf = *reinterpret_cast<const DevTree<float>*>(&t.dt);
+            tc::build_aaug_kernel<<<(nq + 127) / 128, 128, 0, st>>>(reinterpret_cast<const float*>(qsorted), t.d_center.template as<float>(), t.tscale, nq, t.ft.d, t.ft.dpad,
+                                                                    t.kp, t.pmax, w_aaug.as<__half>(), w_qmargin.as<float>());
             CU(cudaGetLastError());
             {
                 // tile bitmaps (tc_prune.cuh): balls of 32 sorted queries against the tile balls, wide balls refined query by query
@@ -692,8 +847,8 @@ struct Engine final : pn_tree {
                 static const int wide_div = getenv("PN_WIDE_DIV") ? atoi(getenv("PN_WIDE_DIV")) : 4;
                 const uint32_t n_sub = QT / 32, n_warps = n_qt * n_sub, n_balls = 2 * n_warps;
                 const uint32_t wide_cap = wide_div > 0 ? std::max<uint32_t>(1u, n_warps / (uint32_t)wide_div) : 1u;
-                const size_t smem = (size_t)32 * dt.dv * 16;
-                TRY(w_bcen.ensure((size_t)n_balls * ft.dpad * 4)); TRY(w_brad.ensure((size_t)n_balls * 4)); TRY(w_bmu.ensure((size_t)n_balls * 4));
+                const size_t smem = (size_t)32 * t.dt.dv * 16;
+                TRY(w_bcen.ensure((size_t)n_balls * t.ft.dpad * 4)); TRY(w_brad.ensure((size_t)n_balls * 4)); TRY(w_bmu.ensure((size_t)n_balls * 4));
                 TRY(w_qth.ensure((size_t)n_warps * 32 * 4)); TRY(w_bbits.ensure((size_t)n_balls * words * 4)); TRY(w_bcnt.ensure((size_t)n_balls * 4));
                 TRY(w_wslot.ensure((size_t)n_warps * 4)); TRY(w_wlist.ensure((size_t)wide_cap * 4)); TRY(w_wbits.ensure((size_t)wide_cap * words * 4));
                 TRY(w_nwide.ensure(4));
@@ -702,18 +857,18 @@ struct Engine final : pn_tree {
                     CU(cudaFuncSetAttribute(tc::ball_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
                 }
                 CU(cudaMemsetAsync(w_nwide.p, 0, 4, st));
-                tc::warp_balls_kernel<<<(n_warps + 7) / 8, 256, 0, st>>>(qsorted, w_seed.as<float>(), nq, n_warps, dt.dv, w_bcen.as<float4>(), w_brad.as<float>(),
+                tc::warp_balls_kernel<<<(n_warps + 7) / 8, 256, 0, st>>>(qsorted, w_seed.as<float>(), nq, n_warps, t.dt.dv, w_bcen.as<float4>(), w_brad.as<float>(),
                                                                          w_bmu.as<float>(), w_qth.as<float>());
                 CU(cudaGetLastError());
                 tc::ball_tile_kernel<false><<<(n_balls + 31) / 32, 256, smem, st>>>(w_bcen.as<float4>(), w_brad.as<float>(), w_bmu.as<float>(), n_balls, nullptr, nullptr, 0u,
-                                                                                   d_tcen.as<float>(), d_trad.as<float>(), n_tiles, dt.dv, (float)dt.slack, words,
+                                                                                   t.d_tcen.template as<float>(), t.d_trad.template as<float>(), n_tiles, t.dt.dv, (float)t.dt.slack, words,
                                                                                    w_bbits.as<uint32_t>(), w_bcnt.as<uint32_t>());
                 CU(cudaGetLastError());
                 tc::wide_select_kernel<<<(n_qt + 127) / 128, 128, 0, st>>>(w_bcnt.as<uint32_t>(), w_bmu.as<float>(), n_qt, n_sub, wide_div > 0 ? wide_cap : 0u, w_wslot.as<uint32_t>(),
                                                                           w_wlist.as<uint32_t>(), w_nwide.as<uint32_t>());
                 CU(cudaGetLastError());
                 tc::ball_tile_kernel<true><<<wide_cap, 256, smem, st>>>(qsorted, nullptr, w_qth.as<float>(), nq, w_wlist.as<uint32_t>(), w_nwide.as<uint32_t>(), wide_div > 0 ? wide_cap : 0u,
-                                                                       d_tcen.as<float>(), d_trad.as<float>(), n_tiles, dt.dv, (float)dt.slack, words,
+                                                                       t.d_tcen.template as<float>(), t.d_trad.template as<float>(), n_tiles, t.dt.dv, (float)t.dt.slack, words,
                                                                        w_wbits.as<uint32_t>(), nullptr);
                 CU(cudaGetLastError());
                 tc::group_bits_kernel<<<n_qt, 256, 0, st>>>(w_bbits.as<uint32_t>(), w_wbits.as<uint32_t>(), w_wslot.as<uint32_t>(), nq, QT, n_sub, words,
@@ -724,23 +879,23 @@ struct Engine final : pn_tree {
             counters.kernel_launches += 2;
             if (stage_timing) CU(cudaEventRecord(se[2], st));
             alignas(64) CUtensorMap map_a;
-            TRY(make_map(&map_a, w_aaug.p, nq, tc::BM));
+            TRY(make_map(&map_a, w_aaug.p, nq, tc::BM, t.kp));
             tc::FilterArgs fa{};
             fa.t = dtf;
             fa.q = qsorted; fa.q_margin = w_qmargin.as<float>();
             fa.k = k; fa.n_tiles = n_tiles; fa.tiles_per_split = n_tiles;
-            fa.nkc = kp / tc::KC;
-            fa.last_steps = ((ft.d + tc::NSLOT - 1) % tc::KC) / 16 + 1;
-            fa.t2_scale = tscale * tscale * (1.0f + (float)(ft.d + 4) * 1.1920928955078125e-07f);
+            fa.nkc = t.kp / tc::KC;
+            fa.last_steps = ((t.ft.d + tc::NSLOT - 1) % tc::KC) / 16 + 1;
+            fa.t2_scale = t.tscale * t.tscale * (1.0f + (float)(t.ft.d + 4) * 1.1920928955078125e-07f);
             fa.part_d = w_part_d.as<float>(); fa.part_i = w_part_i.as<uint32_t>();
             fa.counters = w_counters.as<unsigned long long>();
             fa.row0 = 0; fa.nq = nq; fa.g_bound = nullptr;
             fa.tile_bits = w_bits.as<uint32_t>(); fa.tile_cnt = w_tcnt.as<uint32_t>(); fa.tile_words = words; fa.seed_t2 = w_seed.as<float>();
-            TRY(k1 ? launch_filter_k<1>(map_a, fa, st) : launch_filter_k<16>(map_a, fa, st));
+            TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
             if (stage_timing) CU(cudaEventRecord(se[3], st));
             // results of sorted slot i belong to query order[i] (self query: to the original row of stored point i)
             CU(merge_lists<A, uint32_t>(st, w_part_d.as<A>(), w_part_i.as<uint32_t>(), 1, nq, k, idx_out, dist_out, kstride,
-                                                                            0, nullptr, nullptr, self_query ? d_ids.as<uint32_t>() : order));
+                                                                            0, nullptr, nullptr, self_query ? t.d_ids.template as<uint32_t>() : order));
             CU(cudaGetLastError());
             if (stage_timing) {
                 CU(cudaEventRecord(se[4], st));
@@ -752,7 +907,7 @@ struct Engine final : pn_tree {
                 for (auto& e : se) cudaEventDestroy(e);
             }
             counters.kernel_launches += 2;
-            counters.filter_pairs += (uint64_t)ft.n * nq;  // replaced by the device-side count of scanned pairs in fetch_counters
+            counters.filter_pairs += (uint64_t)t.ft.n * nq;  // replaced by the device-side count of scanned pairs in fetch_counters
             CU(cudaEventRecord(ev[3], st));
             return PN_OK;
         } else {
@@ -762,30 +917,31 @@ struct Engine final : pn_tree {
     }
 
     // tensor k-NN: same contract as knn_device
-    int knn_device_tensor(const A* qraw, uint32_t nq, size_t stride, uint32_t k, uint32_t kstride, uint64_t* idx_out, A* dist_out,
+    int knn_device_tensor(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, uint32_t k, uint32_t kstride, uint64_t* idx_out, A* dist_out,
                           cudaStream_t st, bool self_query = false) {
         if constexpr (sizeof(A) == 4) {
             const bool k1 = (k == 1);
             const uint32_t KP = k1 ? 1 : 16;
             const uint32_t n_pass = (k + KP - 1) / KP;
-            last_pruned = prune_on && n_pass == 1;
-            if (last_pruned && tiles_on) return knn_device_pruned(qraw, nq, stride, k, kstride, idx_out, dist_out, st, self_query);
+            last_pruned = t.prune_on && n_pass == 1;
+            last_tiles = last_pruned && t.tiles_on;
+            if (last_tiles) return knn_device_pruned(t, qraw, nq, stride, k, kstride, idx_out, dist_out, st, self_query);
             // seeded scan without tile bitmaps: the dense launch plan below over the SORTED queries, every query starting
             // from its seed threshold; results return to their rows through the merge kernel's row map
             const float4* qsorted = nullptr;
             const uint32_t* order = nullptr;
             CU(cudaEventRecord(ev[2], st));   // scan_ms covers the whole scan: staging, sort + seeds, filter, merge
-            if (last_pruned) TRY(sort_and_seed(qraw, nq, stride, k, st, self_query, &qsorted, &order));
-            else if (!self_query) TRY(stage_queries(qraw, nq, stride, st, false));
-            const float* qpad = last_pruned ? reinterpret_cast<const float*>(qsorted) : (self_query ? d_pts.as<float>() : w_q.as<float>());
-            TRY(w_aaug.ensure((size_t)nq * kp * 2));
+            if (last_pruned) TRY(sort_and_seed(t, qraw, nq, stride, k, st, self_query, &qsorted, &order));
+            else if (!self_query) TRY(stage_queries(t, qraw, nq, stride, st, false));
+            const float* qpad = last_pruned ? reinterpret_cast<const float*>(qsorted) : (self_query ? t.d_pts.template as<float>() : w_q.as<float>());
+            TRY(w_aaug.ensure((size_t)nq * t.kp * 2));
             TRY(w_qmargin.ensure((size_t)nq * 4));
             // Launch plan.  A CTA serves QT = 128 x subtiles queries against the whole point stream, so whole waves of
             // n_sms CTAs keep every SM busy; what is left (fewer query tiles than SMs: the tail of a large batch, or
             // all of a small one) runs as a second launch whose grid.y splits the point stream S ways -- each CTA scans
             // 1/S of the points for its queries and writes its own top-k list, merged by merge_lists_kernel.
-            const uint32_t n_tiles = (uint32_t)((ft.n + tc::BN - 1) / tc::BN);
-            const uint32_t QT = 128u * (uint32_t)filter_subtiles(kp / tc::KC);
+            const uint32_t n_tiles = (uint32_t)((t.ft.n + tc::BN - 1) / tc::BN);
+            const uint32_t QT = 128u * (uint32_t)t.filter_subtiles(t.kp / tc::KC);
             const uint32_t n_qt = (nq + QT - 1) / QT;
             uint32_t main_qt = n_qt / (uint32_t)n_sms * (uint32_t)n_sms, tail_qt = n_qt - main_qt, S = 1, tps = n_tiles;
             if (tail_qt) {
@@ -806,22 +962,22 @@ struct Engine final : pn_tree {
             TRY(w_part_d.ensure(((size_t)q_main + (size_t)S * q_tail) * KP * 4));
             TRY(w_part_i.ensure(((size_t)q_main + (size_t)S * q_tail) * KP * 4));
             if (n_pass > 1) { TRY(w_floor_d.ensure((size_t)nq * 4)); TRY(w_floor_i.ensure((size_t)nq * 4)); }
-            tc::build_aaug_kernel<<<(nq + 127) / 128, 128, 0, st>>>(qpad, d_center.as<float>(), tscale, nq, ft.d, ft.dpad, kp, pmax,
+            tc::build_aaug_kernel<<<(nq + 127) / 128, 128, 0, st>>>(qpad, t.d_center.template as<float>(), t.tscale, nq, t.ft.d, t.ft.dpad, t.kp, t.pmax,
                                                                     w_aaug.as<__half>(), w_qmargin.as<float>());
             CU(cudaGetLastError());
             ++counters.kernel_launches;
             alignas(64) CUtensorMap map_a;
-            TRY(make_map(&map_a, w_aaug.p, nq, tc::BM));
+            TRY(make_map(&map_a, w_aaug.p, nq, tc::BM, t.kp));
             for (uint32_t p = 0; p < n_pass; ++p) {
                 const uint32_t kk = std::min(KP, k - p * KP);
                 tc::FilterArgs fa{};
-                fa.t = *reinterpret_cast<DevTree<float>*>(&dt);
+                fa.t = *reinterpret_cast<const DevTree<float>*>(&t.dt);
                 fa.q = reinterpret_cast<const float4*>(qpad); fa.q_margin = w_qmargin.as<float>();
                 fa.k = kk;
                 fa.n_tiles = n_tiles;
-                fa.nkc = kp / tc::KC;
-                fa.last_steps = ((ft.d + tc::NSLOT - 1) % tc::KC) / 16 + 1;
-                fa.t2_scale = tscale * tscale * (1.0f + (float)(ft.d + 4) * 1.1920928955078125e-07f);
+                fa.nkc = t.kp / tc::KC;
+                fa.last_steps = ((t.ft.d + tc::NSLOT - 1) % tc::KC) / 16 + 1;
+                fa.t2_scale = t.tscale * t.tscale * (1.0f + (float)(t.ft.d + 4) * 1.1920928955078125e-07f);
                 fa.part_d = w_part_d.as<float>(); fa.part_i = w_part_i.as<uint32_t>();
                 fa.floor_d = p ? w_floor_d.as<float>() : nullptr; fa.floor_i = p ? w_floor_i.as<uint32_t>() : nullptr;
                 fa.counters = w_counters.as<unsigned long long>();
@@ -836,11 +992,11 @@ struct Engine final : pn_tree {
 #endif
                 A* fl_d = n_pass > 1 ? w_floor_d.as<A>() : nullptr;
                 uint32_t* fl_i = n_pass > 1 ? w_floor_i.as<uint32_t>() : nullptr;
-                const uint32_t* rmap = self_query ? d_ids.as<uint32_t>() : order;
+                const uint32_t* rmap = self_query ? t.d_ids.template as<uint32_t>() : order;
                 fa.seed_t2 = last_pruned ? w_seed.as<float>() : nullptr;
                 if (q_main) {
                     fa.row0 = 0; fa.nq = q_main; fa.tiles_per_split = n_tiles; fa.g_bound = nullptr;
-                    TRY(k1 ? launch_filter_k<1>(map_a, fa, st) : launch_filter_k<16>(map_a, fa, st));
+                    TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
                     CU(merge_lists<A, uint32_t>(st, w_part_d.as<A>(), w_part_i.as<uint32_t>(), 1, q_main, kk, idx_out, dist_out, kstride, p * KP, fl_d, fl_i, rmap));
                     CU(cudaGetLastError());
                     counters.kernel_launches += 2;
@@ -853,7 +1009,7 @@ struct Engine final : pn_tree {
                         fa.g_bound = w_gbound.as<float>();
                     }
                     fa.part_d = w_part_d.as<float>() + (size_t)q_main * kk; fa.part_i = w_part_i.as<uint32_t>() + (size_t)q_main * kk;
-                    TRY(k1 ? launch_filter_k<1>(map_a, fa, st) : launch_filter_k<16>(map_a, fa, st));
+                    TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
                     // with a row map (self query) the merge addresses output rows absolutely; otherwise the outputs are offset
                     CU(merge_lists<A, uint32_t>(st, reinterpret_cast<const A*>(fa.part_d), fa.part_i, S, q_tail, kk, rmap ? idx_out : idx_out + (size_t)q_main * kstride,
                         rmap ? dist_out : dist_out + (size_t)q_main * kstride, kstride, p * KP, fl_d ? fl_d + q_main : nullptr,
@@ -861,7 +1017,7 @@ struct Engine final : pn_tree {
                     CU(cudaGetLastError());
                     counters.kernel_launches += 2;
                 }
-                counters.filter_pairs += (uint64_t)ft.n * nq;
+                counters.filter_pairs += (uint64_t)t.ft.n * nq;
             }
             CU(cudaEventRecord(ev[3], st));
             return PN_OK;
@@ -878,21 +1034,21 @@ struct Engine final : pn_tree {
     }
 
     // queries (raw rows on the device) -> zero-padded rows + tile order
-    int stage_queries(const A* qraw, uint32_t nq, size_t stride, cudaStream_t st, bool sort) {
-        TRY(w_q.ensure((size_t)nq * ft.dpad * sizeof(A)));
-        const size_t tot = (size_t)nq * ft.dpad;
-        pad_queries_kernel<A><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(qraw, stride, nq, ft.d, ft.dpad, w_q.as<A>());
+    int stage_queries(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, cudaStream_t st, bool sort) {
+        TRY(w_q.ensure((size_t)nq * t.ft.dpad * sizeof(A)));
+        const size_t tot = (size_t)nq * t.ft.dpad;
+        pad_queries_kernel<A><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(qraw, stride, nq, t.ft.d, t.ft.dpad, w_q.as<A>());
         CU(cudaGetLastError());
         ++counters.kernel_launches;
         if (!sort) return PN_OK;
         TRY(w_home.ensure((size_t)nq * 4));
         TRY(w_order.ensure((size_t)nq * 4));
-        TRY(w_hist.ensure((size_t)ft.n_buckets * 4));
-        TRY(w_cursor.ensure((size_t)ft.n_buckets * 4));
-        CU(cudaMemsetAsync(w_hist.p, 0, (size_t)ft.n_buckets * 4, st));
-        home_bucket_kernel<A><<<(nq + 127) / 128, 128, 0, st>>>(dt, w_q.as<V>(), nq, w_home.as<uint32_t>(), w_hist.as<uint32_t>());
+        TRY(w_hist.ensure((size_t)t.ft.n_buckets * 4));
+        TRY(w_cursor.ensure((size_t)t.ft.n_buckets * 4));
+        CU(cudaMemsetAsync(w_hist.p, 0, (size_t)t.ft.n_buckets * 4, st));
+        home_bucket_kernel<A><<<(nq + 127) / 128, 128, 0, st>>>(t.dt, w_q.as<V>(), nq, w_home.as<uint32_t>(), w_hist.as<uint32_t>());
         CU(cudaGetLastError());
-        exclusive_scan_kernel<<<1, 1024, 0, st>>>(w_hist.as<uint32_t>(), w_cursor.as<uint32_t>(), ft.n_buckets);
+        exclusive_scan_kernel<<<1, 1024, 0, st>>>(w_hist.as<uint32_t>(), w_cursor.as<uint32_t>(), t.ft.n_buckets);
         CU(cudaGetLastError());
         scatter_order_kernel<<<(nq + 255) / 256, 256, 0, st>>>(w_home.as<uint32_t>(), w_cursor.as<uint32_t>(), nq, w_order.as<uint32_t>());
         CU(cudaGetLastError());
@@ -903,14 +1059,14 @@ struct Engine final : pn_tree {
     // k-NN for nq queries whose raw rows are already on the device; results to device buffers
     // self_query: the queries are the stored points themselves, already padded, resident and in bucket
     // order (perfect tile coherence); results are written to the ORIGINAL row of each point
-    int knn_device(const A* qraw, uint32_t nq, size_t stride, uint32_t k_req, uint64_t* idx_out, A* dist_out, cudaStream_t st,
+    int knn_device(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, uint32_t k_req, uint64_t* idx_out, A* dist_out, cudaStream_t st,
                    bool self_query = false) {
-        if (aux && aux->tensor_ready && !self_query) {
-            aux_used = true;
-            return aux->knn_device(qraw, nq, stride, k_req, idx_out, dist_out, st, false);
+        if (!self_query) {   // batches of queries are answered from the partition when the tensor path scans it (DeviceTree::part)
+            const auto p = t.partition();
+            if (p && p->tensor_ready) return knn_device(*p, qraw, nq, stride, k_req, idx_out, dist_out, st);
         }
         // k > n: only n neighbours exist; scan for those and pad the remaining columns directly
-        const uint32_t kstride = k_req, k = (uint32_t)std::min<uint64_t>(k_req, ft.n);
+        const uint32_t kstride = k_req, k = (uint32_t)std::min<uint64_t>(k_req, t.ft.n);
         if (k < kstride) {
             const size_t tot = (size_t)nq * (kstride - k);
             pad_rows_kernel<A><<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(idx_out, dist_out, nq, kstride, k);
@@ -922,20 +1078,20 @@ struct Engine final : pn_tree {
         // scripts/small_batch.py), so AUTO uses it for every batch size whenever the tree is tensor-eligible (f32, d >= 16).
         // The pruned scan can still win for single queries on tightly clustered data (it touches a few buckets only):
         // PN_ALGO_SIMT selects it.
-        last_used_tensor = tensor_ready;
-        if (last_used_tensor) return knn_device_tensor(qraw, nq, stride, k, kstride, idx_out, dist_out, st, self_query);
+        last_used_tensor = t.tensor_ready;
+        if (last_used_tensor) return knn_device_tensor(t, qraw, nq, stride, k, kstride, idx_out, dist_out, st, self_query);
         // narrow rows of a ball tree: one warp per query (knn_warp_kernel) -- every query walks its own few buckets
-        if (ft.kind == 0 && ft.d <= 8 && dt.dv <= 4) {
-            const bool wsort = !self_query && ft.n_buckets > 1 && nq >= 16384;   // neighbouring warps then share buckets in L1 / L2
-            if (!self_query) TRY(stage_queries(qraw, nq, stride, st, wsort));
+        if (t.ft.kind == 0 && t.ft.d <= 8 && t.dt.dv <= 4) {
+            const bool wsort = !self_query && t.ft.n_buckets > 1 && nq >= 16384;   // neighbouring warps then share buckets in L1 / L2
+            if (!self_query) TRY(stage_queries(t, qraw, nq, stride, st, wsort));
             const uint32_t WP = 32, w_pass = (k + WP - 1) / WP;
             if (w_pass > 1) { TRY(w_floor_d.ensure((size_t)nq * sizeof(A))); TRY(w_floor_i.ensure((size_t)nq * 4)); }
             CU(cudaEventRecord(ev[2], st));
             for (uint32_t p = 0; p < w_pass; ++p) {
                 WarpKnnArgs<A> a{};
-                a.t = dt; a.q = self_query ? d_pts.as<V>() : w_q.as<V>();
+                a.t = t.dt; a.q = self_query ? t.d_pts.template as<V>() : w_q.as<V>();
                 a.qorder = wsort ? w_order.as<uint32_t>() : nullptr;
-                a.row_map = self_query ? d_ids.as<uint32_t>() : nullptr;
+                a.row_map = self_query ? t.d_ids.template as<uint32_t>() : nullptr;
                 a.nq = nq; a.k = std::min(WP, k - p * WP);
                 a.out_i = idx_out; a.out_d = dist_out; a.out_stride = kstride; a.out_off = p * WP;
                 a.floor_d = w_pass > 1 ? w_floor_d.as<A>() : nullptr; a.floor_i = w_pass > 1 ? w_floor_i.as<uint32_t>() : nullptr;
@@ -948,11 +1104,11 @@ struct Engine final : pn_tree {
             CU(cudaEventRecord(ev[3], st));
             return PN_OK;
         }
-        const bool sort = !self_query && ft.n_buckets > 1 && nq > (uint32_t)TQ;
-        if (!self_query) TRY(stage_queries(qraw, nq, stride, st, sort));
+        const bool sort = !self_query && t.ft.n_buckets > 1 && nq > (uint32_t)TQ;
+        if (!self_query) TRY(stage_queries(t, qraw, nq, stride, st, sort));
         const uint32_t tiles = (nq + TQ - 1) / TQ;
         uint32_t sl = 0;
-        while (((uint64_t)tiles << sl) < 2ull * n_sms && sl < ft.L && (2u << sl) <= (uint32_t)MAX_LISTS) ++sl;
+        while (((uint64_t)tiles << sl) < 2ull * n_sms && sl < t.ft.L && (2u << sl) <= (uint32_t)MAX_LISTS) ++sl;
         const uint32_t n_splits = 1u << sl;
         const bool k1 = (k == 1);
         const uint32_t KP = k1 ? 1 : 16;
@@ -964,7 +1120,7 @@ struct Engine final : pn_tree {
         for (uint32_t p = 0; p < n_pass; ++p) {
             const uint32_t kk = std::min(KP, k - p * KP);
             KnnArgs<A> a{};
-            a.t = dt; a.q = self_query ? d_pts.as<V>() : w_q.as<V>(); a.qorder = sort ? w_order.as<uint32_t>() : nullptr;
+            a.t = t.dt; a.q = self_query ? t.d_pts.template as<V>() : w_q.as<V>(); a.qorder = sort ? w_order.as<uint32_t>() : nullptr;
             a.nq = nq; a.k = kk; a.split_level = sl;
             a.part_d = w_part_d.as<A>(); a.part_i = w_part_i.as<uint32_t>();
             a.floor_d = p ? w_floor_d.as<A>() : nullptr; a.floor_i = p ? w_floor_i.as<uint32_t>() : nullptr;
@@ -974,10 +1130,10 @@ struct Engine final : pn_tree {
                 CU(cudaMemsetAsync(w_gbound.p, 0x7f, (size_t)nq * sizeof(A), st));
                 a.g_bound = w_gbound.as<A>();
             }
-            TRY(launch_knn(a, dim3(tiles, n_splits), st, k1));
+            TRY(launch_knn(t, a, dim3(tiles, n_splits), st, k1));
             CU(merge_lists<A, uint32_t>(st, w_part_d.as<A>(), w_part_i.as<uint32_t>(), n_splits, nq, kk, idx_out, dist_out, kstride, p * KP,
                 n_pass > 1 ? w_floor_d.as<A>() : nullptr, n_pass > 1 ? w_floor_i.as<uint32_t>() : nullptr,
-                self_query ? d_ids.as<uint32_t>() : nullptr));
+                self_query ? t.d_ids.template as<uint32_t>() : nullptr));
             CU(cudaGetLastError());
             counters.kernel_launches += 2;
         }
@@ -985,79 +1141,14 @@ struct Engine final : pn_tree {
         return PN_OK;
     }
 
-    // A second ball tree over this engine's stored rows, split by the two-means rule, when that pays (see `aux`):
-    // AUTO tries it where seeding already pays and the tile balls of the reference partition leave a single query more than
-    // a tenth of the tiles, and keeps it when its own estimates turn the bitmaps on and a single query can skip at least a
-    // tenth of all tiles more; PN_PARTITION_TWO_MEANS keeps it regardless.  Returns the new
-    // engine in `out` (null: stay with this partition); a failure on the way only loses the speed-up.
-    int two_means_partition(uint32_t partition_opt, uint32_t bucket, std::unique_ptr<Engine<A>>& out) {
-        out.reset();
-        if constexpr (sizeof(A) == 4) {
-            if (partition_opt == PN_PARTITION_REFERENCE || host_only || ft.kind != 0 || !tensor_ready || ft.n != ft.n_total) return PN_OK;
-            const bool forced = partition_opt == PN_PARTITION_TWO_MEANS;
-            // AUTO: seeding pays (clustered data), a single query could skip some tiles but not nearly all of them
-            if (forced ? ft.n < 1024 : !(ft.n >= 32768 && prune_opt == PN_PRUNE_AUTO && prune_on && tile_frac >= 0.1 && tile_frac < 0.9)) return PN_OK;
-            DeviceGuard g(device);
-            if (!g.ok) return PN_OK;
-            std::unique_ptr<Engine<A>> ax(new Engine<A>());
-            ax->device = device; ax->algo = algo; ax->prune_opt = prune_opt;
-            if (cudaStreamSynchronize(stream) != cudaSuccess) { (void)cudaGetLastError(); return PN_OK; }
-            if (ax->build_on_device(d_pts.as<A>(), ft.n, ft.d, ft.dpad, bucket, 0, 0, 1) != PN_OK || !ax->tensor_ready) { (void)cudaGetLastError(); return PN_OK; }
-            translate_ids_kernel<<<(unsigned)((ft.n + 255) / 256), 256, 0, ax->stream>>>(ax->d_ids.template as<uint32_t>(), d_ids.as<uint32_t>(), (uint32_t)ft.n);
-            if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(ax->stream) != cudaSuccess) { (void)cudaGetLastError(); return PN_OK; }
-            ax->ft.n_total = ft.n_total;
-            if (forced || (ax->tiles_on && ax->tile_frac >= tile_frac + 0.1)) out = std::move(ax);
-        }
-        return PN_OK;
-    }
-
-    // A vantage-point handle's ball partition of the same points (Engine::aux).  Tensor-eligible trees get it when they are
-    // created; the others on the first query the VP arrays do not serve (radius search): built on the device from the
-    // stored rows, then its ids (positions in this tree's stored order) are translated to the original point indices.
-    int ensure_companion() {
-        if (aux) return PN_OK;
-        if (host_only) return fail(PN_CUDA, "this handle was built without a device (there is no CPU fallback)");
-        DeviceGuard g(device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
-        std::unique_ptr<Engine<A>> ax(new Engine<A>());
-        ax->device = device; ax->algo = algo; ax->prune_opt = prune_opt;
-        CU(cudaStreamSynchronize(stream));
-        TRY(ax->build_on_device(d_pts.as<A>(), ft.n, ft.d, ft.dpad, 256, 0, 0));
-        translate_ids_kernel<<<(unsigned)((ft.n + 255) / 256), 256, 0, ax->stream>>>(ax->d_ids.template as<uint32_t>(), d_ids.as<uint32_t>(), (uint32_t)ft.n);
-        CU(cudaGetLastError());
-        CU(cudaStreamSynchronize(ax->stream));
-        info.device_bytes += ax->info.device_bytes;
-        aux = std::move(ax);
-        return PN_OK;
-    }
-
-    // start of an API call: device-side work counters to zero (also those of the auxiliary ball engine of a VP handle)
+    // start of an API call: device-side work counters to zero
     int begin_call(cudaStream_t st) {
         TRY(w_counters.ensure(256));
         CU(cudaMemsetAsync(w_counters.p, 0, 256, st));
-        if (aux) {
-            TRY(aux->w_counters.ensure(256));
-            CU(cudaMemsetAsync(aux->w_counters.p, 0, 256, st));
-            aux->counters = pn_counters{};
-            aux->aux_used = false;
-        }
-        aux_used = false;
         return PN_OK;
     }
-    bool aux_used = false;
 
     int fetch_counters(cudaStream_t st, uint64_t nq) {
-        if (aux_used) {  // the scan ran in the auxiliary ball engine: its counters and scan events are the call's
-            const uint64_t h2d = counters.h2d_bytes, d2h = counters.d2h_bytes, kl = counters.kernel_launches;
-            TRY(aux->fetch_counters(st, nq));
-            float ms = 0.f;
-            const double dev_ms = cudaEventElapsedTime(&ms, ev[0], ev[1]) == cudaSuccess ? ms : 0.0;
-            (void)cudaGetLastError();
-            counters = aux->counters;
-            counters.h2d_bytes = h2d; counters.d2h_bytes = d2h; counters.kernel_launches += kl; counters.device_ms = dev_ms;
-            last_used_tensor = aux->last_used_tensor; last_pruned = aux->last_pruned;
-            return PN_OK;
-        }
         unsigned long long c[4] = {0, 0, 0, 0};
         CU(cudaMemcpyAsync(c, w_counters.p, 32, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
@@ -1065,7 +1156,9 @@ struct Engine final : pn_tree {
         if (last_used_tensor && w_counters.cap >= 256) {
             unsigned long long pc[20];
             CU(cudaMemcpy(pc, (char*)w_counters.p + 64, sizeof(pc), cudaMemcpyDeviceToHost));
-            const double tiles = (double)((ft.n + tc::BN - 1) / tc::BN) * (double)((nq + 128 * filter_subtiles(kp / tc::KC) - 1) / (128 * filter_subtiles(kp / tc::KC)));
+            const auto p = tree->partition();
+            const DeviceTree<A>& t = p && p->tensor_ready ? *p : *tree;
+            const double tiles = (double)((t.ft.n + tc::BN - 1) / tc::BN) * (double)((nq + 128 * t.filter_subtiles(t.kp / tc::KC) - 1) / (128 * t.filter_subtiles(t.kp / tc::KC)));
             if (getenv("PN_TC_TRACE") && w_trace.p) {
                 std::vector<long long> tr(12 * 64 * 4);
                 CU(cudaMemcpy(tr.data(), w_trace.p, tr.size() * 8, cudaMemcpyDeviceToHost));
@@ -1077,7 +1170,7 @@ struct Engine final : pn_tree {
 #endif
         counters.queries = nq;
         counters.pairs = last_used_tensor ? counters.filter_pairs : c[0];
-        if (last_used_tensor && last_pruned && tiles_on) {  // the pruned scan counts the (query, point) pairs of the tiles it really visits
+        if (last_used_tensor && last_tiles) {  // the pruned scan counts the (query, point) pairs of the tiles it really visits
             counters.pairs = std::min<uint64_t>(c[3], counters.filter_pairs);
             counters.filter_pairs = counters.pairs;
         }
@@ -1093,7 +1186,7 @@ struct Engine final : pn_tree {
         if (host_only) return fail(PN_CUDA, "tree was built with PN_FLAG_HOST_ONLY: no device, and there is no CPU fallback");
         if (nq && !q) return fail(PN_BAD_ARG, "queries is null");
         if (nq >= (1ull << 32)) return fail(PN_BAD_ARG, "nq must be < 2^32 per call");
-        if (nq > 1 && stride < ft.d) return fail(PN_BAD_ARG, "q_row_stride < dimension");
+        if (nq > 1 && stride < tree->ft.d) return fail(PN_BAD_ARG, "q_row_stride < dimension");
         return PN_OK;
     }
     // k is a u32 inside the engine; the result buffers of a chunk (w_out_*) are k * 12..16 bytes per query
@@ -1116,7 +1209,7 @@ struct Engine final : pn_tree {
     // chunks are capped at 2^20 queries (workspace size).  Measured alternative: one-wave first and last chunks (less
     // exposed copy) -- the same 107.9 ms on config 2 and 2770 instead of 2724 ms on 10M x 128 (scripts/e2e_chunks.py).
     std::vector<size_t> host_chunks(size_t nq) const {
-        const size_t wave = (size_t)n_sms * query_tile();
+        const size_t wave = (size_t)n_sms * tree->query_tile();
         std::vector<size_t> b{0};
         if (nq >= 4 * wave) {
             const size_t half = std::min<size_t>(((nq + 1) / 2 + wave - 1) / wave * wave, ((size_t)1 << 20) / wave * wave);
@@ -1132,7 +1225,7 @@ struct Engine final : pn_tree {
         if (k == 0 || nq == 0) return PN_OK;  // src/ball_tree.rs:106-108
         if (!idx || !distv) return fail(PN_BAD_ARG, "output buffer is null");
         std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(device);
+        DeviceGuard g(tree->device);
         if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
         counters = pn_counters{};
         const A* q = (const A*)qv;
@@ -1144,10 +1237,10 @@ struct Engine final : pn_tree {
         const size_t n_chunks = cb.size() - 1;
         size_t chunk = 0;   // the largest chunk sizes the buffers
         for (size_t c = 0; c < n_chunks; ++c) chunk = std::max(chunk, cb[c + 1] - cb[c]);
-        const size_t spitch = std::max<size_t>(stride, ft.d) * sizeof(A);  // a single row may come with any stride
+        const size_t spitch = std::max<size_t>(stride, tree->ft.d) * sizeof(A);  // a single row may come with any stride
         // every allocation happens before the first copy is enqueued (cudaMalloc synchronises the device)
         for (int b = 0; b < (n_chunks > 1 ? 2 : 1); ++b) {
-            TRY(w_qraw2[b].ensure(chunk * ft.d * sizeof(A)));
+            TRY(w_qraw2[b].ensure(chunk * tree->ft.d * sizeof(A)));
             TRY(w_oi2[b].ensure(chunk * k * 8));
             TRY(w_od2[b].ensure(chunk * k * sizeof(A)));
         }
@@ -1180,14 +1273,14 @@ struct Engine final : pn_tree {
             const uint32_t cq = (uint32_t)(cb[c + 1] - q0);
             // H2D: the raw-query buffer is free once the kernels of chunk c-2 are done
             if (c >= 2) CU(cudaStreamWaitEvent(s_in, e_cmp[b], 0));
-            CU(cudaMemcpy2DAsync(w_qraw2[b].p, ft.d * sizeof(A), q + q0 * stride, spitch, ft.d * sizeof(A), cq, cudaMemcpyHostToDevice, s_in));
+            CU(cudaMemcpy2DAsync(w_qraw2[b].p, tree->ft.d * sizeof(A), q + q0 * stride, spitch, tree->ft.d * sizeof(A), cq, cudaMemcpyHostToDevice, s_in));
             CU(cudaEventRecord(e_in[b], s_in));
             // kernels: need the queries, and the result buffers back from the D2H of chunk c-2
             CU(cudaStreamWaitEvent(st, e_in[b], 0));
             if (c >= 2) CU(cudaStreamWaitEvent(st, e_out[b], 0));
-            TRY(knn_device(w_qraw2[b].as<A>(), cq, ft.d, (uint32_t)k, w_oi2[b].as<uint64_t>(), w_od2[b].as<A>(), st));
+            TRY(knn_device(*tree, w_qraw2[b].as<A>(), cq, tree->ft.d, (uint32_t)k, w_oi2[b].as<uint64_t>(), w_od2[b].as<A>(), st));
             CU(cudaEventRecord(e_cmp[b], st));
-            counters.h2d_bytes += (uint64_t)cq * ft.d * sizeof(A);
+            counters.h2d_bytes += (uint64_t)cq * tree->ft.d * sizeof(A);
             if (c >= 1) TRY(d2h(c - 1));
         }
         TRY(d2h(n_chunks - 1));
@@ -1204,14 +1297,14 @@ struct Engine final : pn_tree {
         if (k == 0 || nq == 0) return PN_OK;
         if (!idx || !distv) return fail(PN_BAD_ARG, "output buffer is null");
         std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(device);
+        DeviceGuard g(tree->device);
         if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
         if (!st) st = stream;
         TRY(use_stream(st));
         counters = pn_counters{};
         TRY(begin_call(st));
         CU(cudaEventRecord(ev[0], st));
-        TRY(knn_device((const A*)qv, (uint32_t)nq, stride, (uint32_t)k, idx, (A*)distv, st));
+        TRY(knn_device(*tree, (const A*)qv, (uint32_t)nq, stride, (uint32_t)k, idx, (A*)distv, st));
         CU(cudaEventRecord(ev[1], st));
         if (sync) return fetch_counters(st, nq);
         counters.queries = nq;
@@ -1302,17 +1395,17 @@ struct Engine final : pn_tree {
     // every stored point is a query (benches/ball_tree.rs:53-59): no H2D at all
     int knn_self(size_t k, uint64_t* idx, void* distv, bool dev, cudaStream_t st, bool sync) override {
         if (host_only) return fail(PN_CUDA, "tree was built with PN_FLAG_HOST_ONLY: no device, and there is no CPU fallback");
-        if (ft.n != ft.n_total) return fail(PN_BAD_ARG, "self-query needs the whole point set in this handle (not a shard)");
+        if (tree->ft.n != tree->ft.n_total) return fail(PN_BAD_ARG, "self-query needs the whole point set in this handle (not a shard)");
         TRY(check_k(k));
         if (k == 0) return PN_OK;
         if (!idx || !distv) return fail(PN_BAD_ARG, "output buffer is null");
         std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(device);
+        DeviceGuard g(tree->device);
         if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
         if (!st || !dev) st = stream;
         TRY(use_stream(st));
         counters = pn_counters{};
-        const uint32_t nq = (uint32_t)ft.n;
+        const uint32_t nq = (uint32_t)tree->ft.n;
         uint64_t* oi = idx; A* od = (A*)distv;
         if (!dev) {
             TRY(w_out_i.ensure((size_t)nq * k * 8));
@@ -1321,7 +1414,7 @@ struct Engine final : pn_tree {
         }
         TRY(begin_call(st));
         CU(cudaEventRecord(ev[0], st));
-        TRY(knn_device(d_pts.as<A>(), nq, ft.dpad, (uint32_t)k, oi, od, st, true));
+        TRY(knn_device(*tree, tree->d_pts.template as<A>(), nq, tree->ft.dpad, (uint32_t)k, oi, od, st, true));
         if (!dev) {
             if ((is_pageable(idx) || is_pageable(distv)) && (size_t)nq * k * 8 >= ((size_t)4 << 20)) {
                 TRY(copy_out_bytes(idx, oi, (size_t)nq * k * 8, st));
@@ -1360,16 +1453,12 @@ struct Engine final : pn_tree {
         TRY(check_query_args(qv, nq, stride));
         if (!offs_out || !idx_out) return fail(PN_BAD_ARG, "output pointer is null");
         std::lock_guard<std::mutex> lk(mu);
-        if (ft.kind != 0) {
-            // an extension (the reference VP tree has no radius query): answered from the ball partition of the same points
-            TRY(ensure_companion());
-            const int rc = aux->radius_host(qv, nq, stride, rr, offs_out, idx_out);
-            counters = aux->counters;
-            last_used_tensor = false; last_pruned = false;
-            return rc;
-        }
-        DeviceGuard g(device);
+        DeviceGuard g(tree->device);
         if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
+        // an extension (the reference VP tree has no radius query): answered from the ball partition of the same points
+        std::shared_ptr<DeviceTree<A>> comp;
+        if (tree->ft.kind != 0) TRY(tree->companion(stream, comp));
+        const DeviceTree<A>& t = comp ? *comp : *tree;
         counters = pn_counters{};
         const A r = (A)rr;
         const A* q = (const A*)qv;
@@ -1391,10 +1480,10 @@ struct Engine final : pn_tree {
         last_used_tensor = false; last_pruned = false;
         if (!pin_tot) CUB(cudaHostAlloc((void**)&pin_tot, 2 * sizeof(unsigned long long), cudaHostAllocDefault));
         TRYB(w_counters.ensure(256));
-        const size_t spitch = std::max<size_t>(stride, ft.d) * sizeof(A);
+        const size_t spitch = std::max<size_t>(stride, t.ft.d) * sizeof(A);
         for (int b = 0; b < (n_chunks > 1 ? 2 : 1); ++b) {
-            TRYB(r_qraw[b].ensure(chunk * ft.d * sizeof(A)));
-            TRYB(r_q[b].ensure(chunk * ft.dpad * sizeof(A)));
+            TRYB(r_qraw[b].ensure(chunk * t.ft.d * sizeof(A)));
+            TRYB(r_q[b].ensure(chunk * t.ft.dpad * sizeof(A)));
             TRYB(r_counts[b].ensure(chunk * 4));
             TRYB(r_offsets[b].ensure((chunk + 1) * 8));
             TRYB(r_sums[b].ensure((chunk / SCAN_BLOCK + 1) * 8));
@@ -1411,13 +1500,13 @@ struct Engine final : pn_tree {
             const size_t q0 = c * chunk;
             const uint32_t cq = (uint32_t)std::min(chunk, nq - q0);
             cudaStream_t s = sx[b];
-            CU(cudaMemcpy2DAsync(r_qraw[b].p, ft.d * sizeof(A), q + q0 * stride, spitch, ft.d * sizeof(A), cq, cudaMemcpyHostToDevice, s));
-            const size_t tot = (size_t)cq * ft.dpad;
-            pad_queries_kernel<A><<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(r_qraw[b].as<A>(), ft.d, cq, ft.d, ft.dpad, r_q[b].as<A>());
+            CU(cudaMemcpy2DAsync(r_qraw[b].p, t.ft.d * sizeof(A), q + q0 * stride, spitch, t.ft.d * sizeof(A), cq, cudaMemcpyHostToDevice, s));
+            const size_t tot = (size_t)cq * t.ft.dpad;
+            pad_queries_kernel<A><<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(r_qraw[b].as<A>(), t.ft.d, cq, t.ft.d, t.ft.dpad, r_q[b].as<A>());
             CU(cudaGetLastError());
             const unsigned blocks = (cq + wpb - 1) / wpb;
             CU(cudaMemsetAsync(r_nlist[b].p, 0, 4, s));
-            radius_kernel<A, 0><<<blocks, wpb * 32, 0, s>>>(dt, r_q[b].as<V>(), cq, r, r_counts[b].as<uint32_t>(), nullptr, r_slab[b].as<uint32_t>(),
+            radius_kernel<A, 0><<<blocks, wpb * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, r_counts[b].as<uint32_t>(), nullptr, r_slab[b].as<uint32_t>(),
                                                            w_counters.as<unsigned long long>());
             CU(cudaGetLastError());
             const unsigned sblocks = std::max(1u, (cq + SCAN_BLOCK - 1) / SCAN_BLOCK);
@@ -1428,7 +1517,7 @@ struct Engine final : pn_tree {
             CU(cudaMemcpyAsync(&pin_tot[b], r_offsets[b].as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, s));
             CU(cudaEventRecord(e_in[b], s));
             counters.kernel_launches += 3;
-            counters.h2d_bytes += (uint64_t)cq * ft.d * sizeof(A);
+            counters.h2d_bytes += (uint64_t)cq * t.ft.d * sizeof(A);
             return PN_OK;
         };
         if (n_chunks) TRYB(stage_a(0));
@@ -1454,7 +1543,7 @@ struct Engine final : pn_tree {
                                                             r_hits[b].as<uint32_t>(), r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
             CUB(cudaGetLastError());
             // second traversal for the queries that overflowed their slab only (warps past the list length exit at once)
-            radius_kernel<A, 1><<<blocks, wpb * 32, 0, s>>>(dt, r_q[b].as<V>(), cq, r, nullptr, r_offsets[b].as<uint64_t>(), r_hits[b].as<uint32_t>(),
+            radius_kernel<A, 1><<<blocks, wpb * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, nullptr, r_offsets[b].as<uint64_t>(), r_hits[b].as<uint32_t>(),
                                                            nullptr, r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
             CUB(cudaGetLastError());
             ++counters.kernel_launches;
@@ -1486,16 +1575,11 @@ struct Engine final : pn_tree {
     }
 
     // ---- point sharding by subtree: local scan -> NCCL exchange -> k-way merge, pipelined over chunks of queries ----------
-#define NC(x)                                                                                                      \
-    do {                                                                                                           \
-        ncclResult_t r_ = (x);                                                                                     \
-        if (r_ != ncclSuccess) return fail(PN_NCCL, std::string(#x) + ": " + cm->api->GetErrorString(r_));         \
-    } while (0)
     int knn_sharded(pn_comm* cm, const void* qv, size_t nq, size_t stride, size_t k, uint32_t exchange, uint64_t* idx_out, void* dist_outv,
                     cudaStream_t st, pn_shard_stats* stats) override {
         TRY(check_query_args(qv, nq, stride));
         if (!cm || !cm->comm) return fail(PN_BAD_ARG, "comm is null");
-        if (cm->device != device) return fail(PN_BAD_ARG, "the communicator rank and the tree live on different devices");
+        if (cm->device != tree->device) return fail(PN_BAD_ARG, "the communicator rank and the tree live on different devices");
         if (k > 255) return fail(PN_BAD_ARG, "sharded k-NN serves k <= 255");
         if (exchange > PN_EXCHANGE_SLICE) return fail(PN_BAD_ARG, "bad exchange mode");
         if (cm->world > 64) return fail(PN_BAD_ARG, "at most 64 ranks");
@@ -1503,7 +1587,7 @@ struct Engine final : pn_tree {
         if (k == 0 || nq == 0) return PN_OK;
         if (!idx_out || !dist_outv) return fail(PN_BAD_ARG, "output buffer is null");
         std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(device);
+        DeviceGuard g(tree->device);
         if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
         if (!st) st = stream;
         TRY(use_stream(st));
@@ -1571,7 +1655,7 @@ struct Engine final : pn_tree {
             // scan: the local lists of chunk c (the buffers of chunk c-2 have been sent: the exchange of c-2 is awaited)
             if (c >= 2) CU(cudaStreamWaitEvent(st, EV(c - 2, 3), 0));
             CU(cudaEventRecord(EV(c, 0), st));
-            TRY(knn_device(q + c0 * stride, cq, stride, (uint32_t)k, sh_li[b].as<uint64_t>(), sh_ld[b].as<A>(), st));
+            TRY(knn_device(*tree, q + c0 * stride, cq, stride, (uint32_t)k, sh_li[b].as<uint64_t>(), sh_ld[b].as<A>(), st));
             if constexpr (PACKED) {
                 const size_t cnt = (size_t)cq * k;
                 pack_lists_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, st>>>(sh_li[b].as<uint64_t>(), (const float*)sh_ld[b].p, cnt,
@@ -1648,7 +1732,7 @@ struct Engine final : pn_tree {
 
     // whole waves per chunk, about eight chunks (see knn_sharded)
     size_t shard_chunk(size_t nq) const override {
-        const size_t wave = (size_t)n_sms * query_tile();
+        const size_t wave = (size_t)n_sms * tree->query_tile();
         return nq < 2 * wave ? nq : std::min<size_t>(std::max<size_t>(1, (nq / 8 + wave - 1) / wave) * wave, ((size_t)1 << 20) / wave * wave);
     }
     // ---- point sharding by subtree WITHOUT a collective (one process, several GPUs): the merge kernel of every rank reads
@@ -1667,7 +1751,7 @@ struct Engine final : pn_tree {
             TRY(check_query_args(qv, nq, stride));
             if (k == 0 || k > 255 || W > 64) return fail(PN_BAD_ARG, "peer exchange: 1 <= k <= 255, at most 64 ranks");
             std::lock_guard<std::mutex> lk(mu);
-            DeviceGuard g(device);
+            DeviceGuard g(tree->device);
             if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
             cudaStream_t st = stream;
             TRY(use_stream(st));
@@ -1697,7 +1781,7 @@ struct Engine final : pn_tree {
                 const size_t c0 = c * chunk, c1 = std::min(nq, c0 + chunk);
                 const uint32_t cq = (uint32_t)(c1 - c0);
                 CU(cudaEventRecord(EV(c, 0), st));
-                TRY(knn_device(q + c0 * stride, cq, stride, (uint32_t)k, sh_li[b].as<uint64_t>(), sh_ld[b].as<A>(), st));
+                TRY(knn_device(*tree, q + c0 * stride, cq, stride, (uint32_t)k, sh_li[b].as<uint64_t>(), sh_ld[b].as<A>(), st));
                 const size_t cnt = (size_t)cq * k;
                 pack_lists_kernel<<<(unsigned)((cnt + 255) / 256), 256, 0, st>>>(sh_li[b].as<uint64_t>(), (const float*)sh_ld[b].p, cnt,
                                                                                  packall.as<unsigned long long>() + c0 * k);
@@ -1747,170 +1831,56 @@ struct Engine final : pn_tree {
         }
     }
 
-    // ---- replication of the flattened tree over NCCL (query sharding: build once, broadcast) ------------------------------
-    struct ReplicaHeader {
-        uint64_t n, n_total;
-        uint32_t d, dpad, L, n_internal, n_buckets, n_nodes, bucket_max, kp;
-        int32_t kind;
-        uint32_t algo, tensor_ready, prune_on;
-        float pmax, tscale;
-    };
-    std::vector<std::pair<DevBuf*, size_t>> replica_arrays() {
-        std::vector<std::pair<DevBuf*, size_t>> v = {
-            {&d_pts, (size_t)ft.n * ft.dpad * sizeof(A)}, {&d_ids, (size_t)ft.n * 4}, {&d_blo, (size_t)ft.n_buckets * 4}, {&d_bhi, (size_t)ft.n_buckets * 4},
-            {&d_centers, (size_t)std::max<uint32_t>(ft.n_nodes, 1) * ft.dpad * sizeof(A)}, {&d_radii, (size_t)std::max<uint32_t>(ft.n_nodes, 1) * sizeof(A)},
-            {&d_vpids, ft.kind == 1 ? (size_t)std::max<uint32_t>(ft.n_nodes, 1) * 4 : 16}};
-        if (partition_rule == 1 && ft.n_internal) {   // (never replicated: a handle's second partition stays on its device; sessions alias it)
-            v.push_back({&d_plane_w, (size_t)ft.n_internal * ft.dpad * sizeof(A)});
-            v.push_back({&d_plane_t, (size_t)ft.n_internal * sizeof(A)});
-        }
-        if (tensor_ready) {
-            v.push_back({&d_center, (size_t)ft.dpad * 4});
-            v.push_back({&d_baug, (ft.n + tc::BN - 1) / tc::BN * tc::BN * (size_t)kp * 2});
-            const size_t n_tiles = (ft.n + tc::BN - 1) / tc::BN;
-            v.push_back({&d_tcen, n_tiles * ft.dpad * 4});
-            v.push_back({&d_trad, n_tiles * 4});
-        }
-        return v;
-    }
     int replicate_send(pn_comm* cm, int root) override {
         if (host_only) return fail(PN_BAD_ARG, "a host-only tree has nothing to replicate");
-        if (cm->device != device) return fail(PN_BAD_ARG, "the communicator rank and the tree live on different devices");
+        if (cm->device != tree->device) return fail(PN_BAD_ARG, "the communicator rank and the tree live on different devices");
         std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(device);
+        DeviceGuard g(tree->device);
         if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
-        ReplicaHeader h{ft.n, ft.n_total, ft.d, ft.dpad, ft.L, ft.n_internal, ft.n_buckets, ft.n_nodes, ft.bucket_max, kp, ft.kind, algo,
-                        tensor_ready ? 1u : 0u, (prune_on ? 1u : 0u) | (tiles_on ? 2u : 0u), pmax, tscale};
-        DevBuf hb;
-        TRY(hb.ensure(sizeof(h)));
-        CU(cudaMemcpyAsync(hb.p, &h, sizeof(h), cudaMemcpyHostToDevice, cm->stream));
-        NC(cm->api->Broadcast(hb.p, hb.p, sizeof(h), ncclUint8, root, cm->comm, cm->stream));
-        for (auto& a : replica_arrays()) NC(cm->api->Broadcast(a.first->p, a.first->p, a.second, ncclUint8, root, cm->comm, cm->stream));
-        CU(cudaStreamSynchronize(cm->stream));
-        hb.release();
-        return PN_OK;
+        return tree->replicate_send(cm, root);
     }
-    int replicate_recv(pn_comm* cm, int root) {
-        device = cm->device;
-        DeviceGuard g(device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
-        TRY(open_device());
-        ReplicaHeader h{};
-        DevBuf hb;
-        TRY(hb.ensure(sizeof(h)));
-        NC(cm->api->Broadcast(hb.p, hb.p, sizeof(h), ncclUint8, root, cm->comm, cm->stream));
-        CU(cudaMemcpyAsync(&h, hb.p, sizeof(h), cudaMemcpyDeviceToHost, cm->stream));
-        CU(cudaStreamSynchronize(cm->stream));
-        hb.release();
-        ft.n = h.n; ft.n_total = h.n_total; ft.d = h.d; ft.dpad = h.dpad; ft.L = h.L; ft.n_internal = h.n_internal; ft.n_buckets = h.n_buckets;
-        ft.n_nodes = h.n_nodes; ft.bucket_max = h.bucket_max; ft.kind = h.kind; kp = h.kp; algo = h.algo; tensor_ready = h.tensor_ready != 0;
-        pmax = h.pmax; tscale = h.tscale; prune_on = (h.prune_on & 1u) != 0; tiles_on = (h.prune_on & 2u) != 0;
-        gpu_built = true;  // no host copies: layout() reads the device arrays
-        info.device_bytes = 0;
-        for (auto& a : replica_arrays()) {
-            TRY(a.first->ensure(a.second));
-            NC(cm->api->Broadcast(a.first->p, a.first->p, a.second, ncclUint8, root, cm->comm, cm->stream));
-            info.device_bytes += a.first->cap;
-        }
-        CU(cudaStreamSynchronize(cm->stream));
-        ft.bucket_lo.resize(ft.n_buckets); ft.bucket_hi.resize(ft.n_buckets);
-        CU(cudaMemcpy(ft.bucket_lo.data(), d_blo.p, (size_t)ft.n_buckets * 4, cudaMemcpyDeviceToHost));
-        CU(cudaMemcpy(ft.bucket_hi.data(), d_bhi.p, (size_t)ft.n_buckets * 4, cudaMemcpyDeviceToHost));
-        if (ft.kind == 1) {
-            ft.vp_ids.resize(std::max<uint32_t>(ft.n_nodes, 1));
-            CU(cudaMemcpy(ft.vp_ids.data(), d_vpids.p, ft.vp_ids.size() * 4, cudaMemcpyDeviceToHost));
-        }
-        fill_dev_tree();
-        TRY(w_counters.ensure(256));
-        return PN_OK;
-    }
-#undef NC
 
-    // ---- sessions: a second handle onto the same device-resident tree (pn_tree_session).  The tree arrays are borrowed,
-    // everything a call writes (stream, events, workspaces, counters, the mutex) is the session's own, so calls on
-    // different sessions of one tree overlap on the device.
-    int attach(Engine& src) {
-        device = src.device;
-        DeviceGuard g(device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
-        TRY(open_device());
-        ft.n = src.ft.n; ft.n_total = src.ft.n_total; ft.d = src.ft.d; ft.dpad = src.ft.dpad; ft.L = src.ft.L;
-        ft.n_internal = src.ft.n_internal; ft.n_buckets = src.ft.n_buckets; ft.n_nodes = src.ft.n_nodes;
-        ft.bucket_max = src.ft.bucket_max; ft.kind = src.ft.kind;
-        ft.bucket_lo = src.ft.bucket_lo; ft.bucket_hi = src.ft.bucket_hi; ft.vp_ids = src.ft.vp_ids;
-        kp = src.kp; algo = src.algo; tensor_ready = src.tensor_ready; pmax = src.pmax; tscale = src.tscale;
-        prune_on = src.prune_on; tiles_on = src.tiles_on; prune_opt = src.prune_opt; partition_rule = src.partition_rule;
-        prune_frac = src.prune_frac; seed_candidates = src.seed_candidates; tile_frac = src.tile_frac;
-        gpu_built = true;   // no host copies: layout() reads the device arrays
-        auto mine = replica_arrays();
-        auto theirs = src.replica_arrays();
-        for (size_t i = 0; i < mine.size(); ++i) mine[i].first->alias(*theirs[i].first);
-        fill_dev_tree();
-        TRY(w_counters.ensure(256));
-        info = src.info;
-        info.device_bytes = 0;   // nothing of the tree is owned here
-        if (src.aux) {
-            aux.reset(new Engine<A>());
-            TRY(aux->attach(*src.aux));
-        }
-        return PN_OK;
-    }
+    // ---- sessions: a second handle onto the same tree (pn_tree_session).  The tree is shared; everything a call writes
+    // (stream, events, workspaces, counters, the mutex) is the session's own, so calls on different sessions of one tree
+    // overlap on the device.
     int session(pn_tree** out) override {
         if (host_only) return fail(PN_BAD_ARG, "a host-only tree has no device arrays to share");
-        pn_tree* root = owner ? owner : this;   // a session of a session borrows from the same owner
-        std::unique_ptr<Engine<A>> e(new Engine<A>());
-        {
-            std::lock_guard<std::mutex> lk(mu);   // no call of this handle is attaching a companion meanwhile
-            TRY(e->attach(*this));
-        }
-        e->owner = root;
-        {
-            std::lock_guard<std::mutex> lk(g_life);
-            root->n_sessions.fetch_add(1);
-        }
+        std::unique_ptr<Engine<A>> e(new Engine<A>(tree));
+        TRY(e->open_device());
+        e->info = info;
+        e->owns_tree = false;
         *out = e.release();
         return PN_OK;
     }
 
     int layout(uint32_t* ids, uint32_t* blo, uint32_t* bhi, void* rad, void* cen, void* pts) override {
-        if (gpu_built) {
-            DeviceGuard g(device);
-            if (ids) CU(cudaMemcpy(ids, d_ids.p, (size_t)ft.n * 4, cudaMemcpyDeviceToHost));
-            if (rad) CU(cudaMemcpy(rad, d_radii.p, (size_t)ft.n_nodes * sizeof(A), cudaMemcpyDeviceToHost));
-            if (cen) CU(cudaMemcpy(cen, d_centers.p, (size_t)ft.n_nodes * ft.dpad * sizeof(A), cudaMemcpyDeviceToHost));
+        const DeviceTree<A>& t = *tree;
+        if (t.gpu_built) {
+            DeviceGuard g(t.device);
+            if (ids) CU(cudaMemcpy(ids, t.d_ids.p, (size_t)t.ft.n * 4, cudaMemcpyDeviceToHost));
+            if (rad) CU(cudaMemcpy(rad, t.d_radii.p, (size_t)t.ft.n_nodes * sizeof(A), cudaMemcpyDeviceToHost));
+            if (cen) CU(cudaMemcpy(cen, t.d_centers.p, (size_t)t.ft.n_nodes * t.ft.dpad * sizeof(A), cudaMemcpyDeviceToHost));
             ids = nullptr; rad = nullptr; cen = nullptr;
         }
-        if (ids) memcpy(ids, ft.ids.data(), ft.ids.size() * 4);
-        if (blo) memcpy(blo, ft.bucket_lo.data(), ft.bucket_lo.size() * 4);
-        if (bhi) memcpy(bhi, ft.bucket_hi.data(), ft.bucket_hi.size() * 4);
-        if (rad) memcpy(rad, ft.radii.data(), (size_t)ft.n_nodes * sizeof(A));
-        if (cen) memcpy(cen, ft.centers.data(), (size_t)ft.n_nodes * ft.dpad * sizeof(A));
+        if (ids) memcpy(ids, t.ft.ids.data(), t.ft.ids.size() * 4);
+        if (blo) memcpy(blo, t.ft.bucket_lo.data(), t.ft.bucket_lo.size() * 4);
+        if (bhi) memcpy(bhi, t.ft.bucket_hi.data(), t.ft.bucket_hi.size() * 4);
+        if (rad) memcpy(rad, t.ft.radii.data(), (size_t)t.ft.n_nodes * sizeof(A));
+        if (cen) memcpy(cen, t.ft.centers.data(), (size_t)t.ft.n_nodes * t.ft.dpad * sizeof(A));
         if (pts) {
-            if (host_only) memcpy(pts, ft.pts.data(), ft.pts.size() * sizeof(A));
+            if (host_only) memcpy(pts, t.ft.pts.data(), t.ft.pts.size() * sizeof(A));
             else {
-                DeviceGuard g(device);
-                CU(cudaMemcpy(pts, d_pts.p, (size_t)ft.n * ft.dpad * sizeof(A), cudaMemcpyDeviceToHost));
+                DeviceGuard g(t.device);
+                CU(cudaMemcpy(pts, t.d_pts.p, (size_t)t.ft.n * t.ft.dpad * sizeof(A), cudaMemcpyDeviceToHost));
             }
         }
         return PN_OK;
     }
 };
+#undef NC
 
 template <typename A>
 static int finish_create(int kind, std::unique_ptr<Engine<A>>& e, const pn_build_opts& o, std::chrono::steady_clock::time_point t0, pn_tree** out);
-
-// a ball handle's two-means partition of the same rows (Engine::aux), when Engine::two_means_partition keeps one
-template <typename A>
-static int attach_two_means(Engine<A>& e, const pn_build_opts& o, uint32_t bucket) {
-    if (e.host_only || o.shard_depth) return PN_OK;
-    std::unique_ptr<Engine<A>> tm;
-    TRY(e.two_means_partition(o.partition, bucket, tm));
-    if (tm) {
-        e.info.device_bytes += tm->info.device_bytes;
-        e.aux = std::move(tm);
-    }
-    return PN_OK;
-}
 
 template <typename A>
 static int create_tree(int kind, const A* points, size_t n, size_t d, size_t row_stride, size_t col_stride,
@@ -1950,11 +1920,13 @@ static int create_tree(int kind, const A* points, size_t n, size_t d, size_t row
         }
     }
     try {
-        e.reset(new Engine<A>());
+        e.reset(new Engine<A>(std::make_shared<DeviceTree<A>>()));
         e->host_only = host_only;
-        e->device = dev;
-        e->algo = o.algo;
-        e->prune_opt = o.prune;
+        DeviceTree<A>& t = *e->tree;
+        t.device = dev;
+        t.algo = o.algo;
+        t.prune_opt = o.prune;
+        if (!host_only) TRY(e->open_device());
         if (on_device) {
             // raw rows to the device (dense n x d), partition and flatten there
             DeviceGuard g(dev);
@@ -1962,11 +1934,9 @@ static int create_tree(int kind, const A* points, size_t n, size_t d, size_t row
             DevBuf raw;
             TRY(raw.ensure(n * d * sizeof(A)));
             cudaError_t ce = cudaMemcpy2D(raw.p, d * sizeof(A), points, std::max(row_stride, d) * sizeof(A), d * sizeof(A), n, cudaMemcpyHostToDevice);
-            int rc = ce != cudaSuccess ? fail(PN_CUDA, std::string("uploading the points: ") + cudaGetErrorString(ce))
-                     : kind == PN_KIND_BALL ? e->build_on_device(raw.as<A>(), n, d, d, bucket, o.shard_depth, o.shard_index)
-                                            : e->build_vp_on_device(raw.as<A>(), n, d, d, bucket);
-            raw.release();
-            TRY(rc);
+            if (ce != cudaSuccess) return fail(PN_CUDA, std::string("uploading the points: ") + cudaGetErrorString(ce));
+            TRY(kind == PN_KIND_BALL ? t.build_on_device(raw.as<A>(), n, d, d, bucket, o.shard_depth, o.shard_index, 0, e->stream)
+                                     : t.build_vp_on_device(raw.as<A>(), n, d, d, bucket, e->stream));
         } else if (kind == PN_KIND_BALL) {
             BallBuilder<A> b(points, n, d, row_stride, threads);
             std::vector<uint32_t> idx(n);
@@ -1976,42 +1946,40 @@ static int create_tree(int kind, const A* points, size_t n, size_t d, size_t row
                 b.shard_range(idx, o.shard_depth, o.shard_index, lo, hi);
                 if (hi == lo) return fail(PN_EMPTY, "shard holds no points");
             }
-            b.build(idx, lo, hi, bucket, e->ft);
+            b.build(idx, lo, hi, bucket, t.ft);
         } else {
             VpBuilder<A> b(points, n, d, row_stride, threads);
-            b.build(bucket, e->ft);
+            b.build(bucket, t.ft);
         }
     } catch (const std::bad_alloc&) {
         return fail(PN_OOM, "host allocation failed while building the tree");
     }
-    if (!host_only && !on_device) TRY(e->upload());
-    if (kind == PN_KIND_VP && !host_only && e->tensor_ready && n >= 1024) {
-        // the ball partition of the same points for the tensor path (see Engine::aux); a failure here only loses the speed-up
-        std::unique_ptr<Engine<A>> ax(new Engine<A>());
-        ax->device = dev; ax->algo = o.algo; ax->prune_opt = o.prune;
+    DeviceTree<A>& t = *e->tree;
+    if (!host_only && !on_device) TRY(t.upload(e->stream));
+    if (kind == PN_KIND_VP && !host_only && t.tensor_ready && n >= 1024) {
+        // the ball partition of the same points for the tensor path (see DeviceTree::part); a failure here only loses the speed-up
         DeviceGuard g(dev);
         DevBuf raw;
+        std::shared_ptr<DeviceTree<A>> ball;
         if (g.ok && raw.ensure(n * d * sizeof(A)) == PN_OK &&
             cudaMemcpy2D(raw.p, d * sizeof(A), points, std::max(row_stride, d) * sizeof(A), d * sizeof(A), n, cudaMemcpyHostToDevice) == cudaSuccess &&
-            ax->build_on_device(raw.as<A>(), n, d, d, bucket, 0, 0) == PN_OK && ax->tensor_ready) {
+            t.build_partition(raw.as<A>(), d, bucket, 0, e->stream, ball) == PN_OK && ball->tensor_ready) {
             raw.release();
             // clustered points: the two-means partition of the same rows instead, when its tile bounds are the tighter ones
-            std::unique_ptr<Engine<A>> tm;
-            ax->two_means_partition(o.partition, bucket, tm);
-            if (tm) ax = std::move(tm);
-            e->info.device_bytes += ax->info.device_bytes;
-            e->aux = std::move(ax);
+            std::shared_ptr<DeviceTree<A>> tm;
+            ball->two_means_partition(o.partition, bucket, e->stream, tm);
+            t.part = tm ? tm : ball;
         }
         (void)cudaGetLastError();
-        raw.release();
     }
-    if (kind == PN_KIND_BALL) TRY(attach_two_means(*e, o, bucket));
+    if (kind == PN_KIND_BALL && !host_only && !o.shard_depth) t.two_means_partition(o.partition, bucket, e->stream, t.part);
     return finish_create(kind, e, o, t0, out);
 }
 
 template <typename A>
 static int finish_create(int kind, std::unique_ptr<Engine<A>>& e, const pn_build_opts& o, std::chrono::steady_clock::time_point t0, pn_tree** out) {
-    FlatTree<A>& ft = e->ft;
+    const DeviceTree<A>& t = *e->tree;
+    const FlatTree<A>& ft = t.ft;
     pn_tree_info& inf = e->info;
     inf.n_points = ft.n; inf.n_points_total = ft.n_total;
     inf.dim = ft.d; inf.dim_padded = ft.dpad;
@@ -2019,9 +1987,9 @@ static int finish_create(int kind, std::unique_ptr<Engine<A>>& e, const pn_build
     inf.n_levels = ft.L; inf.n_buckets = ft.n_buckets; inf.n_nodes = ft.n_nodes;
     inf.bucket_size_max = ft.bucket_max;
     inf.algo = o.algo;
-    inf.device = e->host_only ? -1 : e->device;
+    inf.device = e->host_only ? -1 : t.device;
     {
-        const Engine<A>* pe = e->aux ? e->aux.get() : e.get();   // a VP handle reports the ball partition its tensor path uses
+        const DeviceTree<A>* pe = t.part ? t.part.get() : &t;   // a VP handle reports the ball partition its tensor path uses
         inf.prune_seeded = pe->prune_on ? 1u : 0u; inf.prune_tiles = pe->tiles_on ? 1u : 0u;
         inf.est_seed_candidates = pe->seed_candidates; inf.est_tile_frac = pe->tile_frac; inf.est_group_tile_frac = pe->prune_frac;
         inf.tensor_partition = pe->partition_rule;
@@ -2056,16 +2024,30 @@ static int create_tree_dev(const A* points_dev, size_t n, size_t d, size_t row_s
     auto t0 = std::chrono::steady_clock::now();
     std::unique_ptr<Engine<A>> e;
     try {
-        e.reset(new Engine<A>());
-        e->device = dev;
-        e->algo = o.algo;
-        e->prune_opt = o.prune;
-        TRY(e->build_on_device(points_dev, n, d, row_stride, bucket, o.shard_depth, o.shard_index));
+        e.reset(new Engine<A>(std::make_shared<DeviceTree<A>>()));
+        DeviceTree<A>& t = *e->tree;
+        t.device = dev;
+        t.algo = o.algo;
+        t.prune_opt = o.prune;
+        TRY(e->open_device());
+        TRY(t.build_on_device(points_dev, n, d, row_stride, bucket, o.shard_depth, o.shard_index, 0, e->stream));
+        if (!o.shard_depth) t.two_means_partition(o.partition, bucket, e->stream, t.part);
     } catch (const std::bad_alloc&) {
         return fail(PN_OOM, "host allocation failed while building the tree");
     }
-    TRY(attach_two_means(*e, o, bucket));
     return finish_create(PN_KIND_BALL, e, o, t0, out);
+}
+
+// the receiving side of pn_tree_replicate: a new handle onto the broadcast tree
+template <typename A>
+static int receive_replica(pn_comm* cm, int root, int kind, pn_tree** out) {
+    auto t0 = std::chrono::steady_clock::now();
+    std::unique_ptr<Engine<A>> e(new Engine<A>(std::make_shared<DeviceTree<A>>()));
+    TRY(e->tree->replicate_recv(cm, root));
+    TRY(e->open_device());
+    pn_build_opts o{};
+    o.algo = e->tree->algo;
+    return finish_create<A>(kind, e, o, t0, out);
 }
 
 template <typename A>
@@ -2109,7 +2091,6 @@ static int pairwise_host(int device, const A* x, size_t n, size_t d, size_t row_
         }
         if (e != cudaSuccess) rc = fail(PN_CUDA, std::string("pairwise: ") + cudaGetErrorString(e));
     }
-    dx.release(); dout.release();
     return rc;
 }
 
@@ -2162,17 +2143,7 @@ int32_t pn_balltree_create_dev_f64(const double* p, size_t n, size_t d, size_t r
 }
 int32_t pn_tree_destroy(pn_tree* t) {
     GUARD_BEGIN
-    if (!t) return PN_OK;
-    pn_tree* owner = nullptr;
-    bool free_owner = false;
-    {
-        std::lock_guard<std::mutex> lk(g_life);   // destroys of a tree and of its sessions may race
-        if (t->n_sessions.load() > 0) { t->zombie = true; return PN_OK; }   // its sessions still read its arrays: freed with the last one
-        owner = t->owner;
-        if (owner) free_owner = owner->n_sessions.fetch_sub(1) == 1 && owner->zombie;
-    }
-    delete t;
-    if (free_owner) delete owner;
+    delete t;   // the tree itself is freed with the last handle that shares it
     return PN_OK;
     GUARD_END
 }
@@ -2359,27 +2330,15 @@ int32_t pn_tree_replicate(pn_tree* t, pn_comm* cm, int32_t root, pn_tree** out) 
     TRY(mb.ensure(sizeof(meta)));
     CU(cudaMemcpyAsync(mb.p, meta, sizeof(meta), cudaMemcpyHostToDevice, cm->stream));
     ncclResult_t r = cm->api->Broadcast(mb.p, mb.p, sizeof(meta), ncclUint8, root, cm->comm, cm->stream);
-    if (r != ncclSuccess) { mb.release(); return fail(PN_NCCL, std::string("ncclBroadcast: ") + cm->api->GetErrorString(r)); }
+    if (r != ncclSuccess) return fail(PN_NCCL, std::string("ncclBroadcast: ") + cm->api->GetErrorString(r));
     CU(cudaMemcpyAsync(meta, mb.p, sizeof(meta), cudaMemcpyDeviceToHost, cm->stream));
     CU(cudaStreamSynchronize(cm->stream));
-    mb.release();
     if (is_root) {
         TRY(t->replicate_send(cm, root));
         *out = t;
         return PN_OK;
     }
-    auto t0 = std::chrono::steady_clock::now();
-    pn_build_opts o{};
-    if (meta[0] == PN_F32) {
-        std::unique_ptr<Engine<float>> e(new Engine<float>());
-        TRY(e->replicate_recv(cm, root));
-        o.algo = e->algo;
-        return finish_create<float>(meta[1], e, o, t0, out);
-    }
-    std::unique_ptr<Engine<double>> e(new Engine<double>());
-    TRY(e->replicate_recv(cm, root));
-    o.algo = e->algo;
-    return finish_create<double>(meta[1], e, o, t0, out);
+    return meta[0] == PN_F32 ? receive_replica<float>(cm, root, meta[1], out) : receive_replica<double>(cm, root, meta[1], out);
     GUARD_END
 }
 
@@ -2403,12 +2362,6 @@ struct pn_multi {
             bool dup = false;
             for (size_t j = 0; j < i; ++j) dup |= trees[j] == trees[i];
             if (!dup) delete trees[i];
-        }
-        for (int r = 0; r < n_dev; ++r) {
-            if (r < (int)devices.size()) {
-                DeviceGuard g(devices[r]);
-                if (r < (int)q_dev.size()) { q_dev[r].release(); idx_dev[r].release(); dist_dev[r].release(); }
-            }
         }
         for (auto& v : peer.ev_scan)
             for (cudaEvent_t e : v) if (e) cudaEventDestroy(e);
@@ -2557,6 +2510,7 @@ int32_t pn_multi_destroy(pn_multi* m) {
 int32_t pn_tree_get_info(const pn_tree* t, pn_tree_info* info) {
     if (!t || !info) return fail(PN_BAD_ARG, "null pointer");
     *info = t->info;
+    info->device_bytes = t->device_bytes();
     return PN_OK;
 }
 int32_t pn_tree_get_counters(const pn_tree* t, pn_counters* c) {
