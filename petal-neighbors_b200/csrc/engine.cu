@@ -94,6 +94,64 @@ struct DevBuf {
     template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
 };
 
+// A CUDA stream, event or pinned host buffer, destroyed on the device it was created on, whichever device is current.
+// create() replaces what the wrapper held; on failure the wrapper is left empty.
+template <typename H, cudaError_t (*Destroy)(H)>
+struct CudaHandle {
+    H h = nullptr;
+    int device = -1;
+    CudaHandle() = default;
+    CudaHandle(const CudaHandle&) = delete;
+    CudaHandle& operator=(const CudaHandle&) = delete;
+    CudaHandle(CudaHandle&& o) noexcept : h(o.h), device(o.device) { o.h = nullptr; }
+    CudaHandle& operator=(CudaHandle&& o) noexcept {
+        if (this != &o) {
+            reset();
+            h = o.h; device = o.device;
+            o.h = nullptr;
+        }
+        return *this;
+    }
+    ~CudaHandle() { reset(); }
+    void reset() {
+        if (h) {
+            DeviceGuard g(device);
+            Destroy(h);
+        }
+        h = nullptr;
+    }
+    operator H() const { return h; }
+
+  protected:
+    int created(cudaError_t e, const char* what) {
+        if (e != cudaSuccess) {
+            h = nullptr;
+            return fail(e == cudaErrorMemoryAllocation ? PN_OOM : PN_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
+        }
+        if (cudaGetDevice(&device) != cudaSuccess) (void)cudaGetLastError();
+        return PN_OK;
+    }
+};
+struct Stream : CudaHandle<cudaStream_t, cudaStreamDestroy> {
+    int create() { reset(); return created(cudaStreamCreateWithFlags(&h, cudaStreamNonBlocking), "cudaStreamCreateWithFlags"); }
+};
+struct Event : CudaHandle<cudaEvent_t, cudaEventDestroy> {
+    int create(unsigned flags) { reset(); return created(cudaEventCreateWithFlags(&h, flags), "cudaEventCreateWithFlags"); }
+};
+struct PinnedBuf : CudaHandle<void*, cudaFreeHost> {
+    int create(size_t bytes) { reset(); return created(cudaHostAlloc(&h, bytes, cudaHostAllocDefault), "cudaHostAlloc"); }
+    template <typename T> T* as() const { return static_cast<T*>(h); }
+};
+// grows `v` to at least n events created with `flags` on the current device
+static int grow_events(std::vector<Event>& v, size_t n, unsigned flags) {
+    while (v.size() < n) {
+        Event e;
+        TRY(e.create(flags));
+        v.push_back(std::move(e));
+    }
+    return PN_OK;
+}
+
 }  // namespace petal
 
 using namespace petal;
@@ -104,7 +162,7 @@ struct PeerShared {
     int n = 0;
     size_t chunk = 0, n_chunks = 0;                           // the chunking of this query (the same on every rank)
     std::vector<const unsigned long long*> pack;              // [rank] packed lists of ALL queries of this call
-    std::vector<std::vector<cudaEvent_t>> ev_scan;            // [rank][chunk]: lists of that chunk are packed
+    std::vector<std::vector<Event>> ev_scan;                  // [rank][chunk]: lists of that chunk are packed
     std::mutex mu;
     std::condition_variable cv;
     int count = 0, gen = 0;
@@ -589,54 +647,50 @@ struct Engine final : pn_tree {
     std::shared_ptr<DeviceTree<A>> tree;
     bool owns_tree = true;   // false for a session: device_bytes are reported by the handle that built the tree
     int n_sms = 148;
-    cudaStream_t stream = nullptr, last_stream = nullptr;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    bool last_used_tensor = false;
+    bool last_pruned = false, last_tiles = false;   // the last k-NN scan was seeded / also used tile bitmaps
+    static constexpr size_t PIN_BYTES = 16u << 20;
+
+    // Members are destroyed in reverse order of declaration, so the order of the three groups below is the teardown
+    // order: events and pinned staging first, then the streams, then the device buffers.
     DevBuf w_qraw, w_q, w_home, w_hist, w_cursor, w_order, w_part_d, w_part_i, w_floor_d, w_floor_i,
         w_counters, w_out_i, w_out_d, w_counts, w_offsets, w_hits;
     // host-buffer calls are software-pipelined over chunks of queries: H2D of chunk i+1 and D2H of chunk i-1 run on their own
     // streams under the kernels of chunk i (two sets of raw-query / result buffers)
-    cudaStream_t s_in = nullptr, s_out = nullptr;
-    cudaEvent_t e_in[2] = {nullptr, nullptr}, e_cmp[2] = {nullptr, nullptr}, e_out[2] = {nullptr, nullptr};
     DevBuf w_qraw2[2], w_oi2[2], w_od2[2];
     DevBuf sh_li[2], sh_ld[2], sh_pack[2], sh_gat[2], sh_gat_d[2];   // sharded k-NN: local lists, packed keys, gathered lists
-    std::vector<cudaEvent_t> sh_ev;                                    // timing events of the sharded pipeline (reused)
     DevBuf r_qraw[2], r_q[2], r_counts[2], r_offsets[2], r_hits[2], r_slab[2], r_qlist[2], r_nlist[2], r_sums[2];  // radius pipeline workspaces
-    unsigned long long* pin_tot = nullptr;                            // pinned: chunk totals of the radius count pass
-    void* pin_stage[2] = {nullptr, nullptr};  // pinned D2H staging for the variable-length radius output
-    cudaEvent_t pin_ev[2] = {nullptr, nullptr};
-    static constexpr size_t PIN_BYTES = 16u << 20;
     // tensor path (f32 input only): per-call workspaces, see tc_filter.cuh
     DevBuf w_aaug, w_qmargin, w_trace, w_gbound;
-    bool last_used_tensor = false;
     // pruned tensor scan (tc_prune.cuh): per-call workspaces
     DevBuf w_qs, w_seed, w_bits, w_tcnt;
     DevBuf w_bcen, w_brad, w_bmu, w_qth, w_bbits, w_bcnt, w_wslot, w_wlist, w_wbits, w_nwide;   // tile-bitmap pass: query balls, their bitmaps, wide balls
-    bool last_pruned = false, last_tiles = false;   // the last k-NN scan was seeded / also used tile bitmaps
+
+    Stream stream, s_in, s_out;   // the handle's stream; the H2D / D2H streams of the host-buffer pipelines (ensure_io)
+    cudaStream_t last_stream = nullptr;
+
+    Event ev[4];                  // timing: call (0, 1) and scan (2, 3)
+    Event e_in[2], e_cmp[2], e_out[2];
+    std::vector<Event> sh_ev;     // timing events of the sharded pipeline (reused)
+    PinnedBuf pin_tot;            // chunk totals of the radius count pass
+    PinnedBuf pin_stage[2];       // D2H staging of copy_out_staged
+    Event pin_ev[2];
 
     explicit Engine(std::shared_ptr<DeviceTree<A>> t) : tree(std::move(t)) {}
-    ~Engine() override {
-        if (!host_only) {
-            DeviceGuard g(tree->device);
-            for (auto& e : ev) if (e) cudaEventDestroy(e);
-            for (int i = 0; i < 2; ++i) {
-                if (pin_stage[i]) cudaFreeHost(pin_stage[i]);
-                if (pin_ev[i]) cudaEventDestroy(pin_ev[i]);
-                for (cudaEvent_t e : {e_in[i], e_cmp[i], e_out[i]}) if (e) cudaEventDestroy(e);
-            }
-            for (cudaEvent_t e : sh_ev) cudaEventDestroy(e);
-            if (pin_tot) cudaFreeHost(pin_tot);
-            if (s_in) cudaStreamDestroy(s_in);
-            if (s_out) cudaStreamDestroy(s_out);
-            if (stream) cudaStreamDestroy(stream);
-        }
-    }
 
-    int open_device() {
-        DeviceGuard g(tree->device);
-        if (!g.ok) return fail(PN_CUDA, "no usable CUDA device (there is no CPU fallback)");
-        CU(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, tree->device));
-        CU(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        for (auto& e : ev) CU(cudaEventCreate(&e));
+    // A handle on `t`.  With a device, the handle's stream and timing events are created on the tree's device.
+    static int open(std::shared_ptr<DeviceTree<A>> t, bool host_only, std::unique_ptr<Engine>& out) {
+        std::unique_ptr<Engine> e(new Engine(std::move(t)));
+        e->host_only = host_only;
+        if (!host_only) {
+            const int dev = e->tree->device;
+            DeviceGuard g(dev);
+            if (!g.ok) return fail(PN_CUDA, "no usable CUDA device (there is no CPU fallback)");
+            CU(cudaDeviceGetAttribute(&e->n_sms, cudaDevAttrMultiProcessorCount, dev));
+            TRY(e->stream.create());
+            for (auto& x : e->ev) TRY(x.create(cudaEventDefault));
+        }
+        out = std::move(e);
         return PN_OK;
     }
 
@@ -776,40 +830,57 @@ struct Engine final : pn_tree {
         return launch_filter_t<0, K, 1, 2>(t, map_a, fa, st);
     }
 
+    // The members from here to knn_device_tensor serve the tensor path and are instantiated for f32 trees only (A = float,
+    // V = float4): knn_device calls them from its f32 branch.
+
     // Prepass of the seeded scans (k <= 16): queries sorted by home bucket (self query: the stored order is that order
     // already) and every query's seed threshold from its home bucket.  *qsorted: padded query rows in sorted order; *order:
     // sorted slot -> query id (null for the self query).
-    int sort_and_seed(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, uint32_t k, cudaStream_t st, bool self_query, const float4** qsorted,
+    int sort_and_seed(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, uint32_t k, cudaStream_t st, bool self_query, const V** qsorted,
                       const uint32_t** order) {
-        if constexpr (sizeof(A) == 4) {
-            *order = nullptr;
-            TRY(w_home.ensure((size_t)nq * 4));
-            if (self_query) {
-                TRY(w_hist.ensure((size_t)t.ft.n_buckets * 4));
-                home_bucket_kernel<A><<<(nq + 127) / 128, 128, 0, st>>>(t.dt, t.d_pts.template as<V>(), nq, w_home.as<uint32_t>(), w_hist.as<uint32_t>());
-                CU(cudaGetLastError());
-                ++counters.kernel_launches;
-                *qsorted = t.d_pts.template as<float4>();
-            } else {
-                TRY(stage_queries(t, qraw, nq, stride, st, true));  // padded rows, home buckets, counting sort -> w_order
-                TRY(w_qs.ensure((size_t)nq * t.ft.dpad * 4));
-                const size_t tot = (size_t)nq * t.dt.dv;
-                tc::gather_queries_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(w_q.as<float4>(), w_order.as<uint32_t>(), nq, t.dt.dv, w_qs.as<float4>());
-                CU(cudaGetLastError());
-                ++counters.kernel_launches;
-                *qsorted = w_qs.as<float4>();
-                *order = w_order.as<uint32_t>();
-            }
-            TRY(w_seed.ensure((size_t)nq * 4));
-            const DevTree<float>& dtf = *reinterpret_cast<const DevTree<float>*>(&t.dt);
-            tc::seed_bound_kernel<<<(nq + 7) / 8, 256, 0, st>>>(dtf, *qsorted, *order, w_home.as<uint32_t>(), nq, k, w_seed.as<float>());
+        *order = nullptr;
+        TRY(w_home.ensure((size_t)nq * 4));
+        if (self_query) {
+            TRY(w_hist.ensure((size_t)t.ft.n_buckets * 4));
+            home_bucket_kernel<A><<<(nq + 127) / 128, 128, 0, st>>>(t.dt, t.d_pts.template as<V>(), nq, w_home.as<uint32_t>(), w_hist.as<uint32_t>());
             CU(cudaGetLastError());
             ++counters.kernel_launches;
-            return PN_OK;
+            *qsorted = t.d_pts.template as<V>();
         } else {
-            (void)qraw; (void)nq; (void)stride; (void)k; (void)st; (void)self_query; (void)qsorted; (void)order;
-            return fail(PN_BAD_ARG, "the tensor path is f32 only");
+            TRY(stage_queries(t, qraw, nq, stride, st, true));  // padded rows, home buckets, counting sort -> w_order
+            TRY(w_qs.ensure((size_t)nq * t.ft.dpad * 4));
+            const size_t tot = (size_t)nq * t.dt.dv;
+            tc::gather_queries_kernel<<<(unsigned)((tot + 255) / 256), 256, 0, st>>>(w_q.as<V>(), w_order.as<uint32_t>(), nq, t.dt.dv, w_qs.as<V>());
+            CU(cudaGetLastError());
+            ++counters.kernel_launches;
+            *qsorted = w_qs.as<V>();
+            *order = w_order.as<uint32_t>();
         }
+        TRY(w_seed.ensure((size_t)nq * 4));
+        tc::seed_bound_kernel<<<(nq + 7) / 8, 256, 0, st>>>(t.dt, *qsorted, *order, w_home.as<uint32_t>(), nq, k, w_seed.as<float>());
+        CU(cudaGetLastError());
+        ++counters.kernel_launches;
+        return PN_OK;
+    }
+
+    // The filter arguments that come from the tree, and the query operand of the filter: the augmented FP16 rows of the
+    // nq padded query rows `qpad` (w_aaug, w_qmargin) and their TMA map.  fa.part_d / part_i point at the start of
+    // w_part_d / w_part_i.
+    int filter_operands(const DeviceTree<A>& t, const V* qpad, uint32_t nq, cudaStream_t st, CUtensorMap* map_a, tc::FilterArgs& fa) {
+        tc::build_aaug_kernel<<<(nq + 127) / 128, 128, 0, st>>>(reinterpret_cast<const float*>(qpad), t.d_center.template as<float>(), t.tscale, nq, t.ft.d,
+                                                                t.ft.dpad, t.kp, t.pmax, w_aaug.as<__half>(), w_qmargin.as<float>());
+        CU(cudaGetLastError());
+        ++counters.kernel_launches;
+        TRY(make_map(map_a, w_aaug.p, nq, tc::BM, t.kp));
+        fa.t = t.dt;
+        fa.q = qpad; fa.q_margin = w_qmargin.as<float>();
+        fa.n_tiles = (uint32_t)((t.ft.n + tc::BN - 1) / tc::BN);
+        fa.nkc = t.kp / tc::KC;
+        fa.last_steps = ((t.ft.d + tc::NSLOT - 1) % tc::KC) / 16 + 1;
+        fa.t2_scale = t.tscale * t.tscale * (1.0f + (float)(t.ft.d + 4) * 1.1920928955078125e-07f);
+        fa.part_d = w_part_d.as<float>(); fa.part_i = w_part_i.as<uint32_t>();
+        fa.counters = w_counters.as<unsigned long long>();
+        return PN_OK;
     }
 
     // Pruned tensor k-NN (tc_prune.cuh; k <= 16): queries sorted by home bucket, seed bounds from the home bucket, one tile
@@ -817,214 +888,181 @@ struct Engine final : pn_tree {
     // lengths, so the hardware block scheduler does the load balancing that whole waves do for the dense scan.
     int knn_device_pruned(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, uint32_t k, uint32_t kstride, uint64_t* idx_out, A* dist_out, cudaStream_t st,
                           bool self_query) {
-        if constexpr (sizeof(A) == 4) {
-            const bool k1 = (k == 1);
-            const uint32_t KP = k1 ? 1 : 16;
-            const uint32_t n_tiles = (uint32_t)((t.ft.n + tc::BN - 1) / tc::BN), words = (n_tiles + 31) / 32;
-            const uint32_t QT = 128u * (uint32_t)t.filter_subtiles(t.kp / tc::KC), n_qt = (nq + QT - 1) / QT;
-            const float4* qsorted;
-            const uint32_t* order = nullptr;
-            CU(cudaEventRecord(ev[2], st));   // scan_ms covers the whole scan: sort + seeds, bitmaps, filter, merge
-            // PN_STAGE_TIMING=1 (diagnostic): the stages of this call timed one by one, to stderr
-            static const bool stage_timing = getenv("PN_STAGE_TIMING") != nullptr;
-            cudaEvent_t se[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
-            if (stage_timing) { for (auto& e : se) CU(cudaEventCreate(&e)); CU(cudaEventRecord(se[0], st)); }
-            TRY(sort_and_seed(t, qraw, nq, stride, k, st, self_query, &qsorted, &order));
-            if (stage_timing) CU(cudaEventRecord(se[1], st));
-            TRY(w_aaug.ensure((size_t)nq * t.kp * 2));
-            TRY(w_qmargin.ensure((size_t)nq * 4));
-            TRY(w_bits.ensure((size_t)n_qt * words * 4));
-            TRY(w_tcnt.ensure((size_t)n_qt * 4));
-            TRY(w_part_d.ensure((size_t)nq * KP * 4));
-            TRY(w_part_i.ensure((size_t)nq * KP * 4));
-            const DevTree<float>& dtf = *reinterpret_cast<const DevTree<float>*>(&t.dt);
-            tc::build_aaug_kernel<<<(nq + 127) / 128, 128, 0, st>>>(reinterpret_cast<const float*>(qsorted), t.d_center.template as<float>(), t.tscale, nq, t.ft.d, t.ft.dpad,
-                                                                    t.kp, t.pmax, w_aaug.as<__half>(), w_qmargin.as<float>());
-            CU(cudaGetLastError());
-            {
-                // tile bitmaps (tc_prune.cuh): balls of 32 sorted queries against the tile balls, wide balls refined query by query
-                // PN_WIDE_DIV (diagnostic): the share of warps that may be refined query by query is 1 / PN_WIDE_DIV (0: none)
-                static const int wide_div = getenv("PN_WIDE_DIV") ? atoi(getenv("PN_WIDE_DIV")) : 4;
-                const uint32_t n_sub = QT / 32, n_warps = n_qt * n_sub, n_balls = 2 * n_warps;
-                const uint32_t wide_cap = wide_div > 0 ? std::max<uint32_t>(1u, n_warps / (uint32_t)wide_div) : 1u;
-                const size_t smem = (size_t)32 * t.dt.dv * 16;
-                TRY(w_bcen.ensure((size_t)n_balls * t.ft.dpad * 4)); TRY(w_brad.ensure((size_t)n_balls * 4)); TRY(w_bmu.ensure((size_t)n_balls * 4));
-                TRY(w_qth.ensure((size_t)n_warps * 32 * 4)); TRY(w_bbits.ensure((size_t)n_balls * words * 4)); TRY(w_bcnt.ensure((size_t)n_balls * 4));
-                TRY(w_wslot.ensure((size_t)n_warps * 4)); TRY(w_wlist.ensure((size_t)wide_cap * 4)); TRY(w_wbits.ensure((size_t)wide_cap * words * 4));
-                TRY(w_nwide.ensure(4));
-                if (smem > 48u * 1024u) {
-                    CU(cudaFuncSetAttribute(tc::ball_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                    CU(cudaFuncSetAttribute(tc::ball_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                }
-                CU(cudaMemsetAsync(w_nwide.p, 0, 4, st));
-                tc::warp_balls_kernel<<<(n_warps + 7) / 8, 256, 0, st>>>(qsorted, w_seed.as<float>(), nq, n_warps, t.dt.dv, w_bcen.as<float4>(), w_brad.as<float>(),
-                                                                         w_bmu.as<float>(), w_qth.as<float>());
-                CU(cudaGetLastError());
-                tc::ball_tile_kernel<false><<<(n_balls + 31) / 32, 256, smem, st>>>(w_bcen.as<float4>(), w_brad.as<float>(), w_bmu.as<float>(), n_balls, nullptr, nullptr, 0u,
-                                                                                   t.d_tcen.template as<float>(), t.d_trad.template as<float>(), n_tiles, t.dt.dv, (float)t.dt.slack, words,
-                                                                                   w_bbits.as<uint32_t>(), w_bcnt.as<uint32_t>());
-                CU(cudaGetLastError());
-                tc::wide_select_kernel<<<(n_qt + 127) / 128, 128, 0, st>>>(w_bcnt.as<uint32_t>(), w_bmu.as<float>(), n_qt, n_sub, wide_div > 0 ? wide_cap : 0u, w_wslot.as<uint32_t>(),
-                                                                          w_wlist.as<uint32_t>(), w_nwide.as<uint32_t>());
-                CU(cudaGetLastError());
-                tc::ball_tile_kernel<true><<<wide_cap, 256, smem, st>>>(qsorted, nullptr, w_qth.as<float>(), nq, w_wlist.as<uint32_t>(), w_nwide.as<uint32_t>(), wide_div > 0 ? wide_cap : 0u,
-                                                                       t.d_tcen.template as<float>(), t.d_trad.template as<float>(), n_tiles, t.dt.dv, (float)t.dt.slack, words,
-                                                                       w_wbits.as<uint32_t>(), nullptr);
-                CU(cudaGetLastError());
-                tc::group_bits_kernel<<<n_qt, 256, 0, st>>>(w_bbits.as<uint32_t>(), w_wbits.as<uint32_t>(), w_wslot.as<uint32_t>(), nq, QT, n_sub, words,
-                                                            w_bits.as<uint32_t>(), w_tcnt.as<uint32_t>(), w_counters.as<unsigned long long>() + 3);
-                CU(cudaGetLastError());
-                counters.kernel_launches += 4;
+        const bool k1 = (k == 1);
+        const uint32_t KP = k1 ? 1 : 16;
+        const uint32_t n_tiles = (uint32_t)((t.ft.n + tc::BN - 1) / tc::BN), words = (n_tiles + 31) / 32;
+        const uint32_t QT = 128u * (uint32_t)t.filter_subtiles(t.kp / tc::KC), n_qt = (nq + QT - 1) / QT;
+        const V* qsorted;
+        const uint32_t* order = nullptr;
+        CU(cudaEventRecord(ev[2], st));   // scan_ms covers the whole scan: sort + seeds, bitmaps, filter, merge
+        // PN_STAGE_TIMING=1 (diagnostic): the stages of this call timed one by one, to stderr
+        static const bool stage_timing = getenv("PN_STAGE_TIMING") != nullptr;
+        Event se[5];
+        if (stage_timing) { for (auto& e : se) TRY(e.create(cudaEventDefault)); CU(cudaEventRecord(se[0], st)); }
+        TRY(sort_and_seed(t, qraw, nq, stride, k, st, self_query, &qsorted, &order));
+        if (stage_timing) CU(cudaEventRecord(se[1], st));
+        TRY(w_aaug.ensure((size_t)nq * t.kp * 2));
+        TRY(w_qmargin.ensure((size_t)nq * 4));
+        TRY(w_bits.ensure((size_t)n_qt * words * 4));
+        TRY(w_tcnt.ensure((size_t)n_qt * 4));
+        TRY(w_part_d.ensure((size_t)nq * KP * 4));
+        TRY(w_part_i.ensure((size_t)nq * KP * 4));
+        alignas(64) CUtensorMap map_a;
+        tc::FilterArgs fa{};
+        TRY(filter_operands(t, qsorted, nq, st, &map_a, fa));
+        {
+            // tile bitmaps (tc_prune.cuh): balls of 32 sorted queries against the tile balls, wide balls refined query by query
+            // PN_WIDE_DIV (diagnostic): the share of warps that may be refined query by query is 1 / PN_WIDE_DIV (0: none)
+            static const int wide_div = getenv("PN_WIDE_DIV") ? atoi(getenv("PN_WIDE_DIV")) : 4;
+            const uint32_t n_sub = QT / 32, n_warps = n_qt * n_sub, n_balls = 2 * n_warps;
+            const uint32_t wide_cap = wide_div > 0 ? std::max<uint32_t>(1u, n_warps / (uint32_t)wide_div) : 1u;
+            const size_t smem = (size_t)32 * t.dt.dv * 16;
+            TRY(w_bcen.ensure((size_t)n_balls * t.ft.dpad * 4)); TRY(w_brad.ensure((size_t)n_balls * 4)); TRY(w_bmu.ensure((size_t)n_balls * 4));
+            TRY(w_qth.ensure((size_t)n_warps * 32 * 4)); TRY(w_bbits.ensure((size_t)n_balls * words * 4)); TRY(w_bcnt.ensure((size_t)n_balls * 4));
+            TRY(w_wslot.ensure((size_t)n_warps * 4)); TRY(w_wlist.ensure((size_t)wide_cap * 4)); TRY(w_wbits.ensure((size_t)wide_cap * words * 4));
+            TRY(w_nwide.ensure(4));
+            if (smem > 48u * 1024u) {
+                CU(cudaFuncSetAttribute(tc::ball_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                CU(cudaFuncSetAttribute(tc::ball_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             }
-            counters.kernel_launches += 2;
-            if (stage_timing) CU(cudaEventRecord(se[2], st));
-            alignas(64) CUtensorMap map_a;
-            TRY(make_map(&map_a, w_aaug.p, nq, tc::BM, t.kp));
-            tc::FilterArgs fa{};
-            fa.t = dtf;
-            fa.q = qsorted; fa.q_margin = w_qmargin.as<float>();
-            fa.k = k; fa.n_tiles = n_tiles; fa.tiles_per_split = n_tiles;
-            fa.nkc = t.kp / tc::KC;
-            fa.last_steps = ((t.ft.d + tc::NSLOT - 1) % tc::KC) / 16 + 1;
-            fa.t2_scale = t.tscale * t.tscale * (1.0f + (float)(t.ft.d + 4) * 1.1920928955078125e-07f);
-            fa.part_d = w_part_d.as<float>(); fa.part_i = w_part_i.as<uint32_t>();
-            fa.counters = w_counters.as<unsigned long long>();
-            fa.row0 = 0; fa.nq = nq; fa.g_bound = nullptr;
-            fa.tile_bits = w_bits.as<uint32_t>(); fa.tile_cnt = w_tcnt.as<uint32_t>(); fa.tile_words = words; fa.seed_t2 = w_seed.as<float>();
-            TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
-            if (stage_timing) CU(cudaEventRecord(se[3], st));
-            // results of sorted slot i belong to query order[i] (self query: to the original row of stored point i)
-            CU(merge_lists<A, uint32_t>(st, w_part_d.as<A>(), w_part_i.as<uint32_t>(), 1, nq, k, idx_out, dist_out, kstride,
-                                                                            0, nullptr, nullptr, self_query ? t.d_ids.template as<uint32_t>() : order));
+            CU(cudaMemsetAsync(w_nwide.p, 0, 4, st));
+            tc::warp_balls_kernel<<<(n_warps + 7) / 8, 256, 0, st>>>(qsorted, w_seed.as<float>(), nq, n_warps, t.dt.dv, w_bcen.as<float4>(), w_brad.as<float>(),
+                                                                     w_bmu.as<float>(), w_qth.as<float>());
             CU(cudaGetLastError());
-            if (stage_timing) {
-                CU(cudaEventRecord(se[4], st));
-                CU(cudaEventSynchronize(se[4]));
-                float t[4] = {0.f, 0.f, 0.f, 0.f};
-                for (int i = 0; i < 4; ++i) (void)cudaEventElapsedTime(&t[i], se[i], se[i + 1]);
-                fprintf(stderr, "[pn stage timing] pruned scan, %u queries, k %u: sort + seeds %.2f ms | operands + tile bitmaps %.2f ms | filter %.2f ms | merge %.2f ms\n",
-                        nq, k, t[0], t[1], t[2], t[3]);
-                for (auto& e : se) cudaEventDestroy(e);
-            }
-            counters.kernel_launches += 2;
-            counters.filter_pairs += (uint64_t)t.ft.n * nq;  // replaced by the device-side count of scanned pairs in fetch_counters
-            CU(cudaEventRecord(ev[3], st));
-            return PN_OK;
-        } else {
-            (void)qraw; (void)nq; (void)stride; (void)k; (void)kstride; (void)idx_out; (void)dist_out; (void)st; (void)self_query;
-            return fail(PN_BAD_ARG, "the tensor path is f32 only");
+            tc::ball_tile_kernel<false><<<(n_balls + 31) / 32, 256, smem, st>>>(w_bcen.as<float4>(), w_brad.as<float>(), w_bmu.as<float>(), n_balls, nullptr, nullptr, 0u,
+                                                                               t.d_tcen.template as<float>(), t.d_trad.template as<float>(), n_tiles, t.dt.dv, (float)t.dt.slack, words,
+                                                                               w_bbits.as<uint32_t>(), w_bcnt.as<uint32_t>());
+            CU(cudaGetLastError());
+            tc::wide_select_kernel<<<(n_qt + 127) / 128, 128, 0, st>>>(w_bcnt.as<uint32_t>(), w_bmu.as<float>(), n_qt, n_sub, wide_div > 0 ? wide_cap : 0u, w_wslot.as<uint32_t>(),
+                                                                      w_wlist.as<uint32_t>(), w_nwide.as<uint32_t>());
+            CU(cudaGetLastError());
+            tc::ball_tile_kernel<true><<<wide_cap, 256, smem, st>>>(qsorted, nullptr, w_qth.as<float>(), nq, w_wlist.as<uint32_t>(), w_nwide.as<uint32_t>(), wide_div > 0 ? wide_cap : 0u,
+                                                                   t.d_tcen.template as<float>(), t.d_trad.template as<float>(), n_tiles, t.dt.dv, (float)t.dt.slack, words,
+                                                                   w_wbits.as<uint32_t>(), nullptr);
+            CU(cudaGetLastError());
+            tc::group_bits_kernel<<<n_qt, 256, 0, st>>>(w_bbits.as<uint32_t>(), w_wbits.as<uint32_t>(), w_wslot.as<uint32_t>(), nq, QT, n_sub, words,
+                                                        w_bits.as<uint32_t>(), w_tcnt.as<uint32_t>(), w_counters.as<unsigned long long>() + 3);
+            CU(cudaGetLastError());
+            counters.kernel_launches += 4;
         }
+        ++counters.kernel_launches;
+        if (stage_timing) CU(cudaEventRecord(se[2], st));
+        fa.k = k; fa.tiles_per_split = n_tiles;
+        fa.row0 = 0; fa.nq = nq; fa.g_bound = nullptr;
+        fa.tile_bits = w_bits.as<uint32_t>(); fa.tile_cnt = w_tcnt.as<uint32_t>(); fa.tile_words = words; fa.seed_t2 = w_seed.as<float>();
+        TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
+        if (stage_timing) CU(cudaEventRecord(se[3], st));
+        // results of sorted slot i belong to query order[i] (self query: to the original row of stored point i)
+        CU(merge_lists<A, uint32_t>(st, w_part_d.as<A>(), w_part_i.as<uint32_t>(), 1, nq, k, idx_out, dist_out, kstride,
+                                                                        0, nullptr, nullptr, self_query ? t.d_ids.template as<uint32_t>() : order));
+        CU(cudaGetLastError());
+        if (stage_timing) {
+            CU(cudaEventRecord(se[4], st));
+            CU(cudaEventSynchronize(se[4]));
+            float t[4] = {0.f, 0.f, 0.f, 0.f};
+            for (int i = 0; i < 4; ++i) (void)cudaEventElapsedTime(&t[i], se[i], se[i + 1]);
+            fprintf(stderr, "[pn stage timing] pruned scan, %u queries, k %u: sort + seeds %.2f ms | operands + tile bitmaps %.2f ms | filter %.2f ms | merge %.2f ms\n",
+                    nq, k, t[0], t[1], t[2], t[3]);
+        }
+        counters.kernel_launches += 2;
+        counters.filter_pairs += (uint64_t)t.ft.n * nq;  // replaced by the device-side count of scanned pairs in fetch_counters
+        CU(cudaEventRecord(ev[3], st));
+        return PN_OK;
     }
 
     // tensor k-NN: same contract as knn_device
     int knn_device_tensor(const DeviceTree<A>& t, const A* qraw, uint32_t nq, size_t stride, uint32_t k, uint32_t kstride, uint64_t* idx_out, A* dist_out,
-                          cudaStream_t st, bool self_query = false) {
-        if constexpr (sizeof(A) == 4) {
-            const bool k1 = (k == 1);
-            const uint32_t KP = k1 ? 1 : 16;
-            const uint32_t n_pass = (k + KP - 1) / KP;
-            last_pruned = t.prune_on && n_pass == 1;
-            last_tiles = last_pruned && t.tiles_on;
-            if (last_tiles) return knn_device_pruned(t, qraw, nq, stride, k, kstride, idx_out, dist_out, st, self_query);
-            // seeded scan without tile bitmaps: the dense launch plan below over the SORTED queries, every query starting
-            // from its seed threshold; results return to their rows through the merge kernel's row map
-            const float4* qsorted = nullptr;
-            const uint32_t* order = nullptr;
-            CU(cudaEventRecord(ev[2], st));   // scan_ms covers the whole scan: staging, sort + seeds, filter, merge
-            if (last_pruned) TRY(sort_and_seed(t, qraw, nq, stride, k, st, self_query, &qsorted, &order));
-            else if (!self_query) TRY(stage_queries(t, qraw, nq, stride, st, false));
-            const float* qpad = last_pruned ? reinterpret_cast<const float*>(qsorted) : (self_query ? t.d_pts.template as<float>() : w_q.as<float>());
-            TRY(w_aaug.ensure((size_t)nq * t.kp * 2));
-            TRY(w_qmargin.ensure((size_t)nq * 4));
-            // Launch plan.  A CTA serves QT = 128 x subtiles queries against the whole point stream, so whole waves of
-            // n_sms CTAs keep every SM busy; what is left (fewer query tiles than SMs: the tail of a large batch, or
-            // all of a small one) runs as a second launch whose grid.y splits the point stream S ways -- each CTA scans
-            // 1/S of the points for its queries and writes its own top-k list, merged by merge_lists_kernel.
-            const uint32_t n_tiles = (uint32_t)((t.ft.n + tc::BN - 1) / tc::BN);
-            const uint32_t QT = 128u * (uint32_t)t.filter_subtiles(t.kp / tc::KC);
-            const uint32_t n_qt = (nq + QT - 1) / QT;
-            uint32_t main_qt = n_qt / (uint32_t)n_sms * (uint32_t)n_sms, tail_qt = n_qt - main_qt, S = 1, tps = n_tiles;
-            if (tail_qt) {
-                // S minimises the tail's duration in units of one full scan, ceil(tail_qt S / n_sms) / S, with a charge
-                // of 12 % per extra split (measured: every split starts its own top-k lists, so the exact reranks of a
-                // query grow ~ linearly with S, and there is one more list to merge)
-                const uint32_t s_max = std::max<uint32_t>(1u, std::min<uint32_t>({std::max<uint32_t>(16u, (uint32_t)n_sms / tail_qt), n_tiles / 64u, (uint32_t)MAX_LISTS}));
-                double best = 1e30;
-                for (uint32_t c = 1; c <= s_max; ++c) {
-                    const double cost = (double)((tail_qt * c + n_sms - 1) / n_sms) / c * (1.0 + 0.12 * (c - 1));
-                    if (cost < best) { best = cost; S = c; }
-                }
-                tps = (n_tiles + S - 1) / S;
-                S = (n_tiles + tps - 1) / tps;  // every split non-empty
+                          cudaStream_t st, bool self_query) {
+        const bool k1 = (k == 1);
+        const uint32_t KP = k1 ? 1 : 16;
+        const uint32_t n_pass = (k + KP - 1) / KP;
+        last_pruned = t.prune_on && n_pass == 1;
+        last_tiles = last_pruned && t.tiles_on;
+        if (last_tiles) return knn_device_pruned(t, qraw, nq, stride, k, kstride, idx_out, dist_out, st, self_query);
+        // seeded scan without tile bitmaps: the dense launch plan below over the SORTED queries, every query starting
+        // from its seed threshold; results return to their rows through the merge kernel's row map
+        const V* qsorted = nullptr;
+        const uint32_t* order = nullptr;
+        CU(cudaEventRecord(ev[2], st));   // scan_ms covers the whole scan: staging, sort + seeds, filter, merge
+        if (last_pruned) TRY(sort_and_seed(t, qraw, nq, stride, k, st, self_query, &qsorted, &order));
+        else if (!self_query) TRY(stage_queries(t, qraw, nq, stride, st, false));
+        const V* qpad = last_pruned ? qsorted : (self_query ? t.d_pts.template as<V>() : w_q.as<V>());
+        TRY(w_aaug.ensure((size_t)nq * t.kp * 2));
+        TRY(w_qmargin.ensure((size_t)nq * 4));
+        // Launch plan.  A CTA serves QT = 128 x subtiles queries against the whole point stream, so whole waves of
+        // n_sms CTAs keep every SM busy; what is left (fewer query tiles than SMs: the tail of a large batch, or
+        // all of a small one) runs as a second launch whose grid.y splits the point stream S ways -- each CTA scans
+        // 1/S of the points for its queries and writes its own top-k list, merged by merge_lists_kernel.
+        const uint32_t n_tiles = (uint32_t)((t.ft.n + tc::BN - 1) / tc::BN);
+        const uint32_t QT = 128u * (uint32_t)t.filter_subtiles(t.kp / tc::KC);
+        const uint32_t n_qt = (nq + QT - 1) / QT;
+        uint32_t main_qt = n_qt / (uint32_t)n_sms * (uint32_t)n_sms, tail_qt = n_qt - main_qt, S = 1, tps = n_tiles;
+        if (tail_qt) {
+            // S minimises the tail's duration in units of one full scan, ceil(tail_qt S / n_sms) / S, with a charge
+            // of 12 % per extra split (measured: every split starts its own top-k lists, so the exact reranks of a
+            // query grow ~ linearly with S, and there is one more list to merge)
+            const uint32_t s_max = std::max<uint32_t>(1u, std::min<uint32_t>({std::max<uint32_t>(16u, (uint32_t)n_sms / tail_qt), n_tiles / 64u, (uint32_t)MAX_LISTS}));
+            double best = 1e30;
+            for (uint32_t c = 1; c <= s_max; ++c) {
+                const double cost = (double)((tail_qt * c + n_sms - 1) / n_sms) / c * (1.0 + 0.12 * (c - 1));
+                if (cost < best) { best = cost; S = c; }
             }
-            if (S == 1) { main_qt = n_qt; tail_qt = 0; }
-            const uint32_t q_main = (uint32_t)std::min<uint64_t>((uint64_t)main_qt * QT, nq), q_tail = nq - q_main;
-            TRY(w_part_d.ensure(((size_t)q_main + (size_t)S * q_tail) * KP * 4));
-            TRY(w_part_i.ensure(((size_t)q_main + (size_t)S * q_tail) * KP * 4));
-            if (n_pass > 1) { TRY(w_floor_d.ensure((size_t)nq * 4)); TRY(w_floor_i.ensure((size_t)nq * 4)); }
-            tc::build_aaug_kernel<<<(nq + 127) / 128, 128, 0, st>>>(qpad, t.d_center.template as<float>(), t.tscale, nq, t.ft.d, t.ft.dpad, t.kp, t.pmax,
-                                                                    w_aaug.as<__half>(), w_qmargin.as<float>());
-            CU(cudaGetLastError());
-            ++counters.kernel_launches;
-            alignas(64) CUtensorMap map_a;
-            TRY(make_map(&map_a, w_aaug.p, nq, tc::BM, t.kp));
-            for (uint32_t p = 0; p < n_pass; ++p) {
-                const uint32_t kk = std::min(KP, k - p * KP);
-                tc::FilterArgs fa{};
-                fa.t = *reinterpret_cast<const DevTree<float>*>(&t.dt);
-                fa.q = reinterpret_cast<const float4*>(qpad); fa.q_margin = w_qmargin.as<float>();
-                fa.k = kk;
-                fa.n_tiles = n_tiles;
-                fa.nkc = t.kp / tc::KC;
-                fa.last_steps = ((t.ft.d + tc::NSLOT - 1) % tc::KC) / 16 + 1;
-                fa.t2_scale = t.tscale * t.tscale * (1.0f + (float)(t.ft.d + 4) * 1.1920928955078125e-07f);
-                fa.part_d = w_part_d.as<float>(); fa.part_i = w_part_i.as<uint32_t>();
-                fa.floor_d = p ? w_floor_d.as<float>() : nullptr; fa.floor_i = p ? w_floor_i.as<uint32_t>() : nullptr;
-                fa.counters = w_counters.as<unsigned long long>();
-#ifdef PN_TC_PROFILE
-                fa.dbg = getenv("PN_TC_DEBUG") ? (uint32_t)atoi(getenv("PN_TC_DEBUG")) : 0u;
-                if (getenv("PN_TC_TRACE")) {
-                    TRY(w_trace.ensure(12 * 64 * 4 * 8));
-                    CU(cudaMemsetAsync(w_trace.p, 0, 12 * 64 * 4 * 8, st));
-                    fa.trace = w_trace.as<long long>();
-                    fa.trace_t0 = getenv("PN_TC_TRACE_T0") ? (uint32_t)atoi(getenv("PN_TC_TRACE_T0")) : 2000u;
-                }
-#endif
-                A* fl_d = n_pass > 1 ? w_floor_d.as<A>() : nullptr;
-                uint32_t* fl_i = n_pass > 1 ? w_floor_i.as<uint32_t>() : nullptr;
-                const uint32_t* rmap = self_query ? t.d_ids.template as<uint32_t>() : order;
-                fa.seed_t2 = last_pruned ? w_seed.as<float>() : nullptr;
-                if (q_main) {
-                    fa.row0 = 0; fa.nq = q_main; fa.tiles_per_split = n_tiles; fa.g_bound = nullptr;
-                    TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
-                    CU(merge_lists<A, uint32_t>(st, w_part_d.as<A>(), w_part_i.as<uint32_t>(), 1, q_main, kk, idx_out, dist_out, kstride, p * KP, fl_d, fl_i, rmap));
-                    CU(cudaGetLastError());
-                    counters.kernel_launches += 2;
-                }
-                if (q_tail) {
-                    fa.row0 = q_main; fa.nq = nq; fa.tiles_per_split = tps;
-                    if (S > 1) {  // the splits of a query share their k-th bounds (initialised to a huge finite float)
-                        TRY(w_gbound.ensure((size_t)q_tail * 4));
-                        CU(cudaMemsetAsync(w_gbound.p, 0x7f, (size_t)q_tail * 4, st));
-                        fa.g_bound = w_gbound.as<float>();
-                    }
-                    fa.part_d = w_part_d.as<float>() + (size_t)q_main * kk; fa.part_i = w_part_i.as<uint32_t>() + (size_t)q_main * kk;
-                    TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
-                    // with a row map (self query) the merge addresses output rows absolutely; otherwise the outputs are offset
-                    CU(merge_lists<A, uint32_t>(st, reinterpret_cast<const A*>(fa.part_d), fa.part_i, S, q_tail, kk, rmap ? idx_out : idx_out + (size_t)q_main * kstride,
-                        rmap ? dist_out : dist_out + (size_t)q_main * kstride, kstride, p * KP, fl_d ? fl_d + q_main : nullptr,
-                        fl_i ? fl_i + q_main : nullptr, rmap ? rmap + q_main : nullptr));
-                    CU(cudaGetLastError());
-                    counters.kernel_launches += 2;
-                }
-                counters.filter_pairs += (uint64_t)t.ft.n * nq;
-            }
-            CU(cudaEventRecord(ev[3], st));
-            return PN_OK;
-        } else {
-            (void)qraw; (void)nq; (void)stride; (void)k; (void)idx_out; (void)dist_out; (void)st; (void)self_query;
-            return fail(PN_BAD_ARG, "the tensor path is f32 only");
+            tps = (n_tiles + S - 1) / S;
+            S = (n_tiles + tps - 1) / tps;  // every split non-empty
         }
+        if (S == 1) { main_qt = n_qt; tail_qt = 0; }
+        const uint32_t q_main = (uint32_t)std::min<uint64_t>((uint64_t)main_qt * QT, nq), q_tail = nq - q_main;
+        TRY(w_part_d.ensure(((size_t)q_main + (size_t)S * q_tail) * KP * 4));
+        TRY(w_part_i.ensure(((size_t)q_main + (size_t)S * q_tail) * KP * 4));
+        if (n_pass > 1) { TRY(w_floor_d.ensure((size_t)nq * 4)); TRY(w_floor_i.ensure((size_t)nq * 4)); }
+        alignas(64) CUtensorMap map_a;
+        tc::FilterArgs fa0{};
+        TRY(filter_operands(t, qpad, nq, st, &map_a, fa0));
+        for (uint32_t p = 0; p < n_pass; ++p) {
+            const uint32_t kk = std::min(KP, k - p * KP);
+            tc::FilterArgs fa = fa0;
+            fa.k = kk;
+            fa.floor_d = p ? w_floor_d.as<float>() : nullptr; fa.floor_i = p ? w_floor_i.as<uint32_t>() : nullptr;
+#ifdef PN_TC_PROFILE
+            fa.dbg = getenv("PN_TC_DEBUG") ? (uint32_t)atoi(getenv("PN_TC_DEBUG")) : 0u;
+            if (getenv("PN_TC_TRACE")) {
+                TRY(w_trace.ensure(12 * 64 * 4 * 8));
+                CU(cudaMemsetAsync(w_trace.p, 0, 12 * 64 * 4 * 8, st));
+                fa.trace = w_trace.as<long long>();
+                fa.trace_t0 = getenv("PN_TC_TRACE_T0") ? (uint32_t)atoi(getenv("PN_TC_TRACE_T0")) : 2000u;
+            }
+#endif
+            A* fl_d = n_pass > 1 ? w_floor_d.as<A>() : nullptr;
+            uint32_t* fl_i = n_pass > 1 ? w_floor_i.as<uint32_t>() : nullptr;
+            const uint32_t* rmap = self_query ? t.d_ids.template as<uint32_t>() : order;
+            fa.seed_t2 = last_pruned ? w_seed.as<float>() : nullptr;
+            if (q_main) {
+                fa.row0 = 0; fa.nq = q_main; fa.tiles_per_split = n_tiles; fa.g_bound = nullptr;
+                TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
+                CU(merge_lists<A, uint32_t>(st, w_part_d.as<A>(), w_part_i.as<uint32_t>(), 1, q_main, kk, idx_out, dist_out, kstride, p * KP, fl_d, fl_i, rmap));
+                CU(cudaGetLastError());
+                counters.kernel_launches += 2;
+            }
+            if (q_tail) {
+                fa.row0 = q_main; fa.nq = nq; fa.tiles_per_split = tps;
+                if (S > 1) {  // the splits of a query share their k-th bounds (initialised to a huge finite float)
+                    TRY(w_gbound.ensure((size_t)q_tail * 4));
+                    CU(cudaMemsetAsync(w_gbound.p, 0x7f, (size_t)q_tail * 4, st));
+                    fa.g_bound = w_gbound.as<float>();
+                }
+                fa.part_d = w_part_d.as<float>() + (size_t)q_main * kk; fa.part_i = w_part_i.as<uint32_t>() + (size_t)q_main * kk;
+                TRY(k1 ? launch_filter_k<1>(t, map_a, fa, st) : launch_filter_k<16>(t, map_a, fa, st));
+                // with a row map (self query) the merge addresses output rows absolutely; otherwise the outputs are offset
+                CU(merge_lists<A, uint32_t>(st, reinterpret_cast<const A*>(fa.part_d), fa.part_i, S, q_tail, kk, rmap ? idx_out : idx_out + (size_t)q_main * kstride,
+                    rmap ? dist_out : dist_out + (size_t)q_main * kstride, kstride, p * KP, fl_d ? fl_d + q_main : nullptr,
+                    fl_i ? fl_i + q_main : nullptr, rmap ? rmap + q_main : nullptr));
+                CU(cudaGetLastError());
+                counters.kernel_launches += 2;
+            }
+            counters.filter_pairs += (uint64_t)t.ft.n * nq;
+        }
+        CU(cudaEventRecord(ev[3], st));
+        return PN_OK;
     }
 
     int use_stream(cudaStream_t st) {
@@ -1078,8 +1116,10 @@ struct Engine final : pn_tree {
         // scripts/small_batch.py), so AUTO uses it for every batch size whenever the tree is tensor-eligible (f32, d >= 16).
         // The pruned scan can still win for single queries on tightly clustered data (it touches a few buckets only):
         // PN_ALGO_SIMT selects it.
-        last_used_tensor = t.tensor_ready;
-        if (last_used_tensor) return knn_device_tensor(t, qraw, nq, stride, k, kstride, idx_out, dist_out, st, self_query);
+        last_used_tensor = t.tensor_ready;   // only ever set on f32 trees (DeviceTree::prepare_tensor)
+        if constexpr (sizeof(A) == 4) {
+            if (last_used_tensor) return knn_device_tensor(t, qraw, nq, stride, k, kstride, idx_out, dist_out, st, self_query);
+        }
         // narrow rows of a ball tree: one warp per query (knn_warp_kernel) -- every query walks its own few buckets
         if (t.ft.kind == 0 && t.ft.d <= 8 && t.dt.dv <= 4) {
             const bool wsort = !self_query && t.ft.n_buckets > 1 && nq >= 16384;   // neighbouring warps then share buckets in L1 / L2
@@ -1141,12 +1181,37 @@ struct Engine final : pn_tree {
         return PN_OK;
     }
 
-    // start of an API call: device-side work counters to zero
-    int begin_call(cudaStream_t st) {
-        TRY(w_counters.ensure(256));
-        CU(cudaMemsetAsync(w_counters.p, 0, 256, st));
-        return PN_OK;
-    }
+    // One query call on this handle, made after the call's argument checks: holds the handle's mutex and makes the tree's
+    // device current until the call returns.  open() selects the call's stream (after the handle's previous stream, see
+    // use_stream) and starts a new set of counters; start() zeroes the device-side counters and starts device_ms;
+    // finish() ends device_ms and fetches the device-side counters, or for an unsynchronised call only sets `queries`.
+    struct Call {
+        Engine& e;
+        std::lock_guard<std::mutex> lk;
+        DeviceGuard g;
+        cudaStream_t st = nullptr;
+        explicit Call(Engine& en) : e(en), lk(en.mu), g(en.tree->device) {}
+        int device() const { return g.ok ? PN_OK : fail(PN_CUDA, "cudaSetDevice failed"); }
+        int open(cudaStream_t s) {
+            TRY(device());
+            st = s;
+            TRY(e.use_stream(st));
+            e.counters = pn_counters{};
+            return PN_OK;
+        }
+        int start() {
+            TRY(e.w_counters.ensure(256));
+            CU(cudaMemsetAsync(e.w_counters.p, 0, 256, st));
+            CU(cudaEventRecord(e.ev[0], st));
+            return PN_OK;
+        }
+        int finish(uint64_t nq, bool sync = true) {
+            CU(cudaEventRecord(e.ev[1], st));
+            if (sync) return e.fetch_counters(st, nq);
+            e.counters.queries = nq;
+            return PN_OK;
+        }
+    };
 
     int fetch_counters(cudaStream_t st, uint64_t nq) {
         unsigned long long c[4] = {0, 0, 0, 0};
@@ -1195,12 +1260,14 @@ struct Engine final : pn_tree {
         return PN_OK;
     }
 
+    // The pipeline streams and events, all or nothing: e_out[1] is created last, so while it is null a later call
+    // creates the whole set again.
     int ensure_io() {
-        if (s_in) return PN_OK;
-        CU(cudaStreamCreateWithFlags(&s_in, cudaStreamNonBlocking));
-        CU(cudaStreamCreateWithFlags(&s_out, cudaStreamNonBlocking));
+        if (e_out[1]) return PN_OK;
+        TRY(s_in.create());
+        TRY(s_out.create());
         for (int i = 0; i < 2; ++i)
-            for (cudaEvent_t* e : {&e_in[i], &e_cmp[i], &e_out[i]}) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+            for (Event* e : {&e_in[i], &e_cmp[i], &e_out[i]}) TRY(e->create(cudaEventDisableTiming));
         return PN_OK;
     }
     // Chunk boundaries of a host-buffer call: whole waves of the scan (n_sms CTAs x the scan's queries per CTA).  Two
@@ -1224,14 +1291,11 @@ struct Engine final : pn_tree {
         TRY(check_k(k));
         if (k == 0 || nq == 0) return PN_OK;  // src/ball_tree.rs:106-108
         if (!idx || !distv) return fail(PN_BAD_ARG, "output buffer is null");
-        std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(tree->device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
-        counters = pn_counters{};
+        Call call(*this);
+        const cudaStream_t st = stream;
+        TRY(call.open(st));
         const A* q = (const A*)qv;
         A* dist = (A*)distv;
-        cudaStream_t st = stream;
-        TRY(use_stream(st));
         TRY(ensure_io());
         const std::vector<size_t> cb = host_chunks(nq);
         const size_t n_chunks = cb.size() - 1;
@@ -1244,25 +1308,16 @@ struct Engine final : pn_tree {
             TRY(w_oi2[b].ensure(chunk * k * 8));
             TRY(w_od2[b].ensure(chunk * k * sizeof(A)));
         }
-        TRY(begin_call(st));
-        CU(cudaEventRecord(ev[0], st));
+        TRY(call.start());
         CU(cudaStreamWaitEvent(s_in, ev[0], 0));
         // Enqueue order: H2D(c), kernels(c), then D2H(c-1).  With pageable host memory a D2H copy blocks the host until it
         // is done, so it is issued only after the next chunk's kernels are already queued behind it on the device.
-        // Large results bound for pageable memory go through the engine's own pinned staging (copy_out_bytes).
-        const bool staged_out = is_pageable(idx) || is_pageable(dist);
         auto d2h = [&](size_t c) -> int {
             const int b = (int)(c & 1);
             const size_t q0 = cb[c];
             const uint32_t cq = (uint32_t)(cb[c + 1] - q0);
             CU(cudaStreamWaitEvent(s_out, e_cmp[b], 0));
-            if (staged_out && (size_t)cq * k * 8 >= ((size_t)4 << 20)) {
-                TRY(copy_out_bytes(idx + q0 * k, w_oi2[b].p, (size_t)cq * k * 8, s_out));
-                TRY(copy_out_bytes(dist + q0 * k, w_od2[b].p, (size_t)cq * k * sizeof(A), s_out));
-            } else {
-                CU(cudaMemcpyAsync(idx + q0 * k, w_oi2[b].p, (size_t)cq * k * 8, cudaMemcpyDeviceToHost, s_out));
-                CU(cudaMemcpyAsync(dist + q0 * k, w_od2[b].p, (size_t)cq * k * sizeof(A), cudaMemcpyDeviceToHost, s_out));
-            }
+            TRY(results_to_host(idx + q0 * k, dist + q0 * k, w_oi2[b].as<uint64_t>(), w_od2[b].as<A>(), (size_t)cq * k, s_out));
             CU(cudaEventRecord(e_out[b], s_out));
             counters.d2h_bytes += (uint64_t)cq * k * (8 + sizeof(A));
             return PN_OK;
@@ -1287,8 +1342,7 @@ struct Engine final : pn_tree {
         // the call ends when the last results are on the host: the tree's stream joins the D2H stream
         CU(cudaStreamWaitEvent(st, e_out[(n_chunks - 1) & 1], 0));
         if (n_chunks > 1) CU(cudaStreamWaitEvent(st, e_out[(n_chunks - 2) & 1], 0));
-        CU(cudaEventRecord(ev[1], st));
-        return fetch_counters(st, nq);
+        return call.finish(nq);
     }
 
     int knn_dev(const void* qv, size_t nq, size_t stride, size_t k, uint64_t* idx, void* distv, cudaStream_t st, bool sync) override {
@@ -1296,92 +1350,45 @@ struct Engine final : pn_tree {
         TRY(check_k(k));
         if (k == 0 || nq == 0) return PN_OK;
         if (!idx || !distv) return fail(PN_BAD_ARG, "output buffer is null");
-        std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(tree->device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
-        if (!st) st = stream;
-        TRY(use_stream(st));
-        counters = pn_counters{};
-        TRY(begin_call(st));
-        CU(cudaEventRecord(ev[0], st));
-        TRY(knn_device(*tree, (const A*)qv, (uint32_t)nq, stride, (uint32_t)k, idx, (A*)distv, st));
-        CU(cudaEventRecord(ev[1], st));
-        if (sync) return fetch_counters(st, nq);
-        counters.queries = nq;
-        return PN_OK;
+        Call call(*this);
+        TRY(call.open(st ? st : (cudaStream_t)stream));
+        TRY(call.start());
+        TRY(knn_device(*tree, (const A*)qv, (uint32_t)nq, stride, (uint32_t)k, idx, (A*)distv, call.st));
+        return call.finish(nq, sync);
     }
 
-    // Device u32 indices -> host u64 indices: D2H in 16 MB pieces through two pinned buffers; while piece
-    // p+1 is in flight, piece p is widened into the (freshly allocated, not yet faulted) destination by a
-    // few host threads -- page-faulting and widening, not the DMA, are the slow part.
-    int copy_out_widen(uint64_t* dst, const uint32_t* src_dev, size_t count, cudaStream_t st) {
-        if (count == 0) return PN_OK;
-        for (int i = 0; i < 2; ++i) {
-            if (!pin_stage[i]) CU(cudaHostAlloc(&pin_stage[i], PIN_BYTES, cudaHostAllocDefault));
-            if (!pin_ev[i]) CU(cudaEventCreateWithFlags(&pin_ev[i], cudaEventDisableTiming));
-        }
-        const size_t per = PIN_BYTES / 4;
-        const size_t pieces = (count + per - 1) / per;
-        auto issue = [&](size_t p) -> int {
-            const size_t off = p * per, cnt = std::min(per, count - off);
-            CU(cudaMemcpyAsync(pin_stage[p & 1], src_dev + off, cnt * 4, cudaMemcpyDeviceToHost, st));
-            CU(cudaEventRecord(pin_ev[p & 1], st));
-            return PN_OK;
-        };
-        TRY(issue(0));
-        const unsigned nt = std::max(1u, std::min(12u, std::thread::hardware_concurrency() / 2));
-        for (size_t p = 0; p < pieces; ++p) {
-            CU(cudaEventSynchronize(pin_ev[p & 1]));
-            if (p + 1 < pieces) TRY(issue(p + 1));  // the other buffer was consumed in the previous iteration
-            const size_t off = p * per, cnt = std::min(per, count - off);
-            const uint32_t* s32 = (const uint32_t*)pin_stage[p & 1];
-            uint64_t* d64 = dst + off;
-            std::vector<std::thread> th;
-            const size_t chunk = (cnt + nt - 1) / nt;
-            for (unsigned t = 1; t < nt; ++t) {
-                const size_t b = t * chunk, e = std::min(cnt, b + chunk);
-                if (b < e) th.emplace_back([=] { for (size_t i = b; i < e; ++i) d64[i] = s32[i]; });
-            }
-            for (size_t i = 0, e = std::min(cnt, chunk); i < e; ++i) d64[i] = s32[i];
-            for (auto& x : th) x.join();
-        }
-        return PN_OK;
-    }
-
-    // Device -> PAGEABLE host memory: the driver's own staged copy runs at about 4 GB/s into freshly allocated pages (it
-    // faults them in one by one).  Same pipeline as copy_out_widen: D2H in 16 MB pieces through two pinned buffers; while
-    // piece p+1 is in flight, piece p is copied to its destination by a few host threads (page faults in parallel).
-    int copy_out_bytes(void* dstv, const void* src_devv, size_t bytes, cudaStream_t st) {
+    // Device -> host through two pinned buffers, in pieces of PIN_BYTES: while piece p+1 is in flight, piece p is handed
+    // to land(off, piece, lo, hi), which moves bytes [lo, hi) of the piece that starts at byte `off` of the copy to their
+    // destination.  Up to `max_threads` host threads share a piece, in slices that are multiples of `align` bytes.  Into
+    // freshly allocated memory, page faults and the host-side step, not the DMA, are the slow part.
+    template <typename Land>
+    int copy_out_staged(const void* src_dev, size_t bytes, cudaStream_t st, unsigned max_threads, size_t align, Land land) {
         if (bytes == 0) return PN_OK;
         for (int i = 0; i < 2; ++i) {
-            if (!pin_stage[i]) CU(cudaHostAlloc(&pin_stage[i], PIN_BYTES, cudaHostAllocDefault));
-            if (!pin_ev[i]) CU(cudaEventCreateWithFlags(&pin_ev[i], cudaEventDisableTiming));
+            if (!pin_stage[i]) TRY(pin_stage[i].create(PIN_BYTES));
+            if (!pin_ev[i]) TRY(pin_ev[i].create(cudaEventDisableTiming));
         }
-        unsigned char* dst = (unsigned char*)dstv;
-        const unsigned char* src = (const unsigned char*)src_devv;
-        const size_t per = PIN_BYTES;
-        const size_t pieces = (bytes + per - 1) / per;
+        const size_t pieces = (bytes + PIN_BYTES - 1) / PIN_BYTES;
         auto issue = [&](size_t p) -> int {
-            const size_t off = p * per, cnt = std::min(per, bytes - off);
-            CU(cudaMemcpyAsync(pin_stage[p & 1], src + off, cnt, cudaMemcpyDeviceToHost, st));
+            const size_t off = p * PIN_BYTES, cnt = std::min(PIN_BYTES, bytes - off);
+            CU(cudaMemcpyAsync(pin_stage[p & 1], (const unsigned char*)src_dev + off, cnt, cudaMemcpyDeviceToHost, st));
             CU(cudaEventRecord(pin_ev[p & 1], st));
             return PN_OK;
         };
         TRY(issue(0));
-        const unsigned nt = std::max(1u, std::min(8u, std::thread::hardware_concurrency() / 2));
+        const unsigned nt = std::max(1u, std::min(max_threads, std::thread::hardware_concurrency() / 2));
         for (size_t p = 0; p < pieces; ++p) {
             CU(cudaEventSynchronize(pin_ev[p & 1]));
             if (p + 1 < pieces) TRY(issue(p + 1));  // the other buffer was consumed in the previous iteration
-            const size_t off = p * per, cnt = std::min(per, bytes - off);
-            const unsigned char* sp = (const unsigned char*)pin_stage[p & 1];
-            unsigned char* dp = dst + off;
-            const size_t chunk = ((cnt + nt - 1) / nt + 4095) & ~(size_t)4095;
+            const size_t off = p * PIN_BYTES, cnt = std::min(PIN_BYTES, bytes - off);
+            const unsigned char* sp = pin_stage[p & 1].template as<unsigned char>();
+            const size_t chunk = ((cnt + nt - 1) / nt + align - 1) / align * align;
             std::vector<std::thread> th;
             for (unsigned t = 1; t < nt; ++t) {
                 const size_t b = t * chunk, e = std::min(cnt, b + chunk);
-                if (b < e) th.emplace_back([=] { memcpy(dp + b, sp + b, e - b); });
+                if (b < e) th.emplace_back([=] { land(off, sp, b, e); });
             }
-            memcpy(dp, sp, std::min(cnt, chunk));
+            land(off, sp, 0, std::min(cnt, chunk));
             for (auto& x : th) x.join();
         }
         return PN_OK;
@@ -1391,6 +1398,23 @@ struct Engine final : pn_tree {
         if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { (void)cudaGetLastError(); return true; }
         return at.type == cudaMemoryTypeUnregistered;
     }
+    // The k-NN results of one call (count = queries x k) from the device to the caller's host buffers.  Pageable
+    // destinations of 4 MiB of indices and more go through the pinned staging, copied in page-aligned slices on up to 8
+    // host threads: the driver's own staged copy runs at about 4 GB/s into freshly allocated pages (it faults them in one
+    // by one).
+    int results_to_host(uint64_t* idx, A* dist, const uint64_t* idx_dev, const A* dist_dev, size_t count, cudaStream_t st) {
+        if (count * 8 >= ((size_t)4 << 20) && (is_pageable(idx) || is_pageable(dist))) {
+            auto bytes_to = [](void* dst) {
+                return [dst](size_t off, const unsigned char* sp, size_t lo, size_t hi) { memcpy((unsigned char*)dst + off + lo, sp + lo, hi - lo); };
+            };
+            TRY(copy_out_staged(idx_dev, count * 8, st, 8, 4096, bytes_to(idx)));
+            TRY(copy_out_staged(dist_dev, count * sizeof(A), st, 8, 4096, bytes_to(dist)));
+        } else {
+            CU(cudaMemcpyAsync(idx, idx_dev, count * 8, cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(dist, dist_dev, count * sizeof(A), cudaMemcpyDeviceToHost, st));
+        }
+        return PN_OK;
+    }
 
     // every stored point is a query (benches/ball_tree.rs:53-59): no H2D at all
     int knn_self(size_t k, uint64_t* idx, void* distv, bool dev, cudaStream_t st, bool sync) override {
@@ -1399,12 +1423,9 @@ struct Engine final : pn_tree {
         TRY(check_k(k));
         if (k == 0) return PN_OK;
         if (!idx || !distv) return fail(PN_BAD_ARG, "output buffer is null");
-        std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(tree->device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
+        Call call(*this);
         if (!st || !dev) st = stream;
-        TRY(use_stream(st));
-        counters = pn_counters{};
+        TRY(call.open(st));
         const uint32_t nq = (uint32_t)tree->ft.n;
         uint64_t* oi = idx; A* od = (A*)distv;
         if (!dev) {
@@ -1412,23 +1433,13 @@ struct Engine final : pn_tree {
             TRY(w_out_d.ensure((size_t)nq * k * sizeof(A)));
             oi = w_out_i.as<uint64_t>(); od = w_out_d.as<A>();
         }
-        TRY(begin_call(st));
-        CU(cudaEventRecord(ev[0], st));
+        TRY(call.start());
         TRY(knn_device(*tree, tree->d_pts.template as<A>(), nq, tree->ft.dpad, (uint32_t)k, oi, od, st, true));
         if (!dev) {
-            if ((is_pageable(idx) || is_pageable(distv)) && (size_t)nq * k * 8 >= ((size_t)4 << 20)) {
-                TRY(copy_out_bytes(idx, oi, (size_t)nq * k * 8, st));
-                TRY(copy_out_bytes(distv, od, (size_t)nq * k * sizeof(A), st));
-            } else {
-                CU(cudaMemcpyAsync(idx, oi, (size_t)nq * k * 8, cudaMemcpyDeviceToHost, st));
-                CU(cudaMemcpyAsync(distv, od, (size_t)nq * k * sizeof(A), cudaMemcpyDeviceToHost, st));
-            }
+            TRY(results_to_host(idx, (A*)distv, oi, od, (size_t)nq * k, st));
             counters.d2h_bytes = (uint64_t)nq * k * (8 + sizeof(A));
         }
-        CU(cudaEventRecord(ev[1], st));
-        if (sync || !dev) return fetch_counters(st, nq);
-        counters.queries = nq;
-        return PN_OK;
+        return call.finish(nq, sync || !dev);
     }
 
     // Result buffers of the radius call are handed to the caller (released with pn_free = free()).  Large ones are
@@ -1452,49 +1463,46 @@ struct Engine final : pn_tree {
     int radius_host(const void* qv, size_t nq, size_t stride, double rr, uint64_t** offs_out, uint64_t** idx_out) override {
         TRY(check_query_args(qv, nq, stride));
         if (!offs_out || !idx_out) return fail(PN_BAD_ARG, "output pointer is null");
-        std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(tree->device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
+        Call call(*this);
+        TRY(call.device());
         // an extension (the reference VP tree has no radius query): answered from the ball partition of the same points
         std::shared_ptr<DeviceTree<A>> comp;
         if (tree->ft.kind != 0) TRY(tree->companion(stream, comp));
         const DeviceTree<A>& t = comp ? *comp : *tree;
-        counters = pn_counters{};
+        const cudaStream_t st = stream;
+        TRY(call.open(st));
         const A r = (A)rr;
         const A* q = (const A*)qv;
-        cudaStream_t st = stream;
-        TRY(use_stream(st));
         TRY(ensure_io());
         cudaStream_t sx[2] = {s_in, s_out};  // the two pipeline streams (alternate chunks)
-        uint64_t* offs = (uint64_t*)malloc((nq + 1) * 8);
+        // the result arrays, owned here until they are handed to the caller
+        struct Free { void operator()(uint64_t* p) const { free(p); } };
+        std::unique_ptr<uint64_t[], Free> offs((uint64_t*)malloc((nq + 1) * 8)), hit_buf;
         if (!offs) return fail(PN_OOM, "malloc offsets");
+        // on an error return, copies already queued may still write into offs / hit_buf: the device finishes before
+        // they are freed (declared after them, so destroyed first)
+        struct SyncOnError { bool armed = true; ~SyncOnError() { if (armed) cudaDeviceSynchronize(); } } sync_on_error;
         offs[0] = 0;
-        uint64_t* hit_buf = nullptr;
         size_t hit_cap = 0, total = 0;
         const size_t chunk = nq <= (1u << 18) ? std::max<size_t>(nq, 1) : (1u << 17);
         const size_t n_chunks = (nq + chunk - 1) / chunk;
         const uint32_t wpb = 8;
-        auto bail = [&](int rc) { cudaDeviceSynchronize(); free(offs); free(hit_buf); return rc; };
-#define CUB(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) return bail(fail(PN_CUDA, std::string(#x) + ": " + cudaGetErrorString(e_))); } while (0)
-#define TRYB(x) do { int r_ = (x); if (r_ != PN_OK) return bail(r_); } while (0)
         last_used_tensor = false; last_pruned = false;
-        if (!pin_tot) CUB(cudaHostAlloc((void**)&pin_tot, 2 * sizeof(unsigned long long), cudaHostAllocDefault));
-        TRYB(w_counters.ensure(256));
+        if (!pin_tot) TRY(pin_tot.create(2 * sizeof(unsigned long long)));
         const size_t spitch = std::max<size_t>(stride, t.ft.d) * sizeof(A);
         for (int b = 0; b < (n_chunks > 1 ? 2 : 1); ++b) {
-            TRYB(r_qraw[b].ensure(chunk * t.ft.d * sizeof(A)));
-            TRYB(r_q[b].ensure(chunk * t.ft.dpad * sizeof(A)));
-            TRYB(r_counts[b].ensure(chunk * 4));
-            TRYB(r_offsets[b].ensure((chunk + 1) * 8));
-            TRYB(r_sums[b].ensure((chunk / SCAN_BLOCK + 1) * 8));
-            TRYB(r_slab[b].ensure(chunk * RADIUS_CAP * 4));
-            TRYB(r_qlist[b].ensure(chunk * 4));
-            TRYB(r_nlist[b].ensure(16));
+            TRY(r_qraw[b].ensure(chunk * t.ft.d * sizeof(A)));
+            TRY(r_q[b].ensure(chunk * t.ft.dpad * sizeof(A)));
+            TRY(r_counts[b].ensure(chunk * 4));
+            TRY(r_offsets[b].ensure((chunk + 1) * 8));
+            TRY(r_sums[b].ensure((chunk / SCAN_BLOCK + 1) * 8));
+            TRY(r_slab[b].ensure(chunk * RADIUS_CAP * 4));
+            TRY(r_qlist[b].ensure(chunk * 4));
+            TRY(r_nlist[b].ensure(16));
         }
-        CUB(cudaMemsetAsync(w_counters.p, 0, 256, st));
-        CUB(cudaEventRecord(ev[0], st));
-        CUB(cudaEventRecord(ev[2], st));
-        for (int b = 0; b < 2; ++b) CUB(cudaStreamWaitEvent(sx[b], ev[0], 0));
+        TRY(call.start());
+        CU(cudaEventRecord(ev[2], st));
+        for (int b = 0; b < 2; ++b) CU(cudaStreamWaitEvent(sx[b], ev[0], 0));
         auto stage_a = [&](size_t c) -> int {
             const int b = (int)(c & 1);
             const size_t q0 = c * chunk;
@@ -1514,63 +1522,67 @@ struct Engine final : pn_tree {
             offsets_scan_kernel<<<sblocks, 1024, 0, s>>>(r_counts[b].as<uint32_t>(), r_sums[b].as<unsigned long long>(), r_offsets[b].as<uint64_t>(), cq);
             CU(cudaGetLastError());
             ++counters.kernel_launches;
-            CU(cudaMemcpyAsync(&pin_tot[b], r_offsets[b].as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, s));
+            CU(cudaMemcpyAsync(&pin_tot.as<unsigned long long>()[b], r_offsets[b].as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, s));
             CU(cudaEventRecord(e_in[b], s));
             counters.kernel_launches += 3;
             counters.h2d_bytes += (uint64_t)cq * t.ft.d * sizeof(A);
             return PN_OK;
         };
-        if (n_chunks) TRYB(stage_a(0));
+        if (n_chunks) TRY(stage_a(0));
         for (size_t c = 0; c < n_chunks; ++c) {
             const int b = (int)(c & 1);
             const size_t q0 = c * chunk;
             const uint32_t cq = (uint32_t)std::min(chunk, nq - q0);
             cudaStream_t s = sx[b];
-            if (c + 1 < n_chunks) TRYB(stage_a(c + 1));
-            CUB(cudaEventSynchronize(e_in[b]));
-            const uint64_t ctotal = pin_tot[b];  // chunk-local total
+            if (c + 1 < n_chunks) TRY(stage_a(c + 1));
+            CU(cudaEventSynchronize(e_in[b]));
+            const uint64_t ctotal = pin_tot.as<unsigned long long>()[b];  // chunk-local total
             if (total + ctotal > hit_cap) {
                 // sized once from the first chunk's density (+12 %); grows only if later chunks are denser
                 size_t ncap = std::max<size_t>(total + ctotal, c == 0 ? (size_t)((double)ctotal * 1.12 * (double)nq / cq) + 1024 : hit_cap + hit_cap / 2);
-                uint64_t* nb = (uint64_t*)result_alloc(ncap * 8);
-                if (!nb) return bail(fail(PN_OOM, "allocating the result indices"));
-                if (hit_buf) { memcpy(nb, hit_buf, total * 8); free(hit_buf); }
-                hit_buf = nb; hit_cap = ncap;
+                std::unique_ptr<uint64_t[], Free> nb((uint64_t*)result_alloc(ncap * 8));
+                if (!nb) return fail(PN_OOM, "allocating the result indices");
+                if (hit_buf) memcpy(nb.get(), hit_buf.get(), total * 8);
+                hit_buf = std::move(nb); hit_cap = ncap;
             }
-            TRYB(r_hits[b].ensure((ctotal ? ctotal : 1) * 4));
+            TRY(r_hits[b].ensure((ctotal ? ctotal : 1) * 4));
             const unsigned blocks = (cq + wpb - 1) / wpb;
             compact_hits_kernel<<<blocks, wpb * 32, 0, s>>>(r_slab[b].as<uint32_t>(), r_counts[b].as<uint32_t>(), r_offsets[b].as<uint64_t>(), cq,
                                                             r_hits[b].as<uint32_t>(), r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
-            CUB(cudaGetLastError());
+            CU(cudaGetLastError());
             // second traversal for the queries that overflowed their slab only (warps past the list length exit at once)
             radius_kernel<A, 1><<<blocks, wpb * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, nullptr, r_offsets[b].as<uint64_t>(), r_hits[b].as<uint32_t>(),
                                                            nullptr, r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
-            CUB(cudaGetLastError());
+            CU(cudaGetLastError());
             ++counters.kernel_launches;
             segment_sort_kernel<<<blocks, wpb * 32, 0, s>>>(r_offsets[b].as<uint64_t>(), r_hits[b].as<uint32_t>(), cq);
-            CUB(cudaGetLastError());
+            CU(cudaGetLastError());
             if (ctotal > SORT_WARP_MAX) {  // some hit list may be longer than a warp should sort: one block per such query
                 segment_sort_large_kernel<<<std::min<uint32_t>(cq, 8u * (uint32_t)n_sms), 256, 0, s>>>(r_offsets[b].as<uint64_t>(), r_hits[b].as<uint32_t>(), cq);
-                CUB(cudaGetLastError());
+                CU(cudaGetLastError());
                 ++counters.kernel_launches;
             }
             counters.kernel_launches += 2;
-            CUB(cudaMemcpyAsync(offs + q0 + 1, r_offsets[b].as<uint64_t>() + 1, (size_t)cq * 8, cudaMemcpyDeviceToHost, s));
-            TRYB(copy_out_widen(hit_buf + total, r_hits[b].as<uint32_t>(), ctotal, s));
-            CUB(cudaStreamSynchronize(s));
+            CU(cudaMemcpyAsync(offs.get() + q0 + 1, r_offsets[b].as<uint64_t>() + 1, (size_t)cq * 8, cudaMemcpyDeviceToHost, s));
+            // the hits, u32 on the device, widened to u64 on up to 12 host threads
+            uint64_t* dst = hit_buf.get() + total;
+            TRY(copy_out_staged(r_hits[b].p, ctotal * 4, s, 12, 4, [dst](size_t off, const unsigned char* sp, size_t lo, size_t hi) {
+                const uint32_t* s32 = (const uint32_t*)sp;
+                uint64_t* d64 = dst + off / 4;
+                for (size_t i = lo / 4; i < hi / 4; ++i) d64[i] = s32[i];
+            }));
+            CU(cudaStreamSynchronize(s));
             if (total) for (uint32_t i = 1; i <= cq; ++i) offs[q0 + i] += total;  // chunk-local -> global offsets
             total += ctotal;
             counters.d2h_bytes += (uint64_t)cq * 8 + ctotal * 4;
         }
-        for (int b = 0; b < 2; ++b) { CUB(cudaEventRecord(e_cmp[b], sx[b])); CUB(cudaStreamWaitEvent(st, e_cmp[b], 0)); }
-        CUB(cudaEventRecord(ev[3], st));
-        CUB(cudaEventRecord(ev[1], st));
-        if (!hit_buf) hit_buf = (uint64_t*)malloc(8);
-        TRYB(fetch_counters(st, nq));
-#undef CUB
-#undef TRYB
-        *offs_out = offs;
-        *idx_out = hit_buf;
+        for (int b = 0; b < 2; ++b) { CU(cudaEventRecord(e_cmp[b], sx[b])); CU(cudaStreamWaitEvent(st, e_cmp[b], 0)); }
+        CU(cudaEventRecord(ev[3], st));
+        if (!hit_buf) hit_buf.reset((uint64_t*)malloc(8));
+        TRY(call.finish(nq));
+        sync_on_error.armed = false;
+        *offs_out = offs.release();
+        *idx_out = hit_buf.release();
         return PN_OK;
     }
 
@@ -1586,13 +1598,10 @@ struct Engine final : pn_tree {
         if (stats) *stats = pn_shard_stats{};
         if (k == 0 || nq == 0) return PN_OK;
         if (!idx_out || !dist_outv) return fail(PN_BAD_ARG, "output buffer is null");
-        std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(tree->device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
+        Call call(*this);
         if (!st) st = stream;
-        TRY(use_stream(st));
+        TRY(call.open(st));
         TRY(ensure_io());
-        counters = pn_counters{};
         const A* q = (const A*)qv;
         A* dist_out = (A*)dist_outv;
         const int W = cm->world, R = cm->rank;
@@ -1609,12 +1618,10 @@ struct Engine final : pn_tree {
             TRY(sh_gat[b].ensure((size_t)W * chunk * k * 8));
             if (PACKED) TRY(sh_pack[b].ensure(chunk * k * 8)); else TRY(sh_gat_d[b].ensure((size_t)W * chunk * k * sizeof(A)));
         }
-        TRY(w_counters.ensure(256));
-        while (sh_ev.size() < 6 * n_chunks) { cudaEvent_t e; CU(cudaEventCreate(&e)); sh_ev.push_back(e); }
-        auto EV = [&](size_t c, int i) { return sh_ev[6 * c + i]; };  // 0,1 scan; 2,3 exchange; 4,5 merge
+        TRY(grow_events(sh_ev, 6 * n_chunks, cudaEventDefault));
+        auto EV = [&](size_t c, int i) -> cudaEvent_t { return sh_ev[6 * c + i]; };  // 0,1 scan; 2,3 exchange; 4,5 merge
         cudaStream_t cs = cm->stream;
-        CU(cudaMemsetAsync(w_counters.p, 0, 256, st));
-        CU(cudaEventRecord(ev[0], st));
+        TRY(call.start());
         unsigned long long bytes = 0, calls = 0, rows_out = 0;
         // rows of chunk [c0, c1) owned by rank r (SLICE) / all of them (ALLGATHER)
         auto owned = [&](int r, size_t c0, size_t c1, size_t& lo, size_t& cnt) {
@@ -1713,8 +1720,7 @@ struct Engine final : pn_tree {
             if (c >= 1) TRY(merge_chunk(c - 1));   // after the scan of chunk c is queued, so the exchange of c-1 had time to run
         }
         TRY(merge_chunk(n_chunks - 1));
-        CU(cudaEventRecord(ev[1], st));
-        CU(cudaStreamSynchronize(st));
+        TRY(call.finish(nq));
         cm->bytes_sent += bytes; cm->collectives += calls;
         if (stats) {
             float ms = 0.f;
@@ -1727,7 +1733,7 @@ struct Engine final : pn_tree {
             (void)cudaGetLastError();
             stats->nccl_bytes_sent = bytes; stats->nccl_calls = calls; stats->rows_out = rows_out; stats->n_chunks = (uint32_t)n_chunks;
         }
-        return fetch_counters(st, nq);
+        return PN_OK;
     }
 
     // whole waves per chunk, about eight chunks (see knn_sharded)
@@ -1750,14 +1756,11 @@ struct Engine final : pn_tree {
             struct Guard { PeerShared& p; bool ok = false; ~Guard() { if (!ok) p.fail(); } } guard{ps};
             TRY(check_query_args(qv, nq, stride));
             if (k == 0 || k > 255 || W > 64) return fail(PN_BAD_ARG, "peer exchange: 1 <= k <= 255, at most 64 ranks");
-            std::lock_guard<std::mutex> lk(mu);
-            DeviceGuard g(tree->device);
-            if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
-            cudaStream_t st = stream;
-            TRY(use_stream(st));
+            Call call(*this);
+            const cudaStream_t st = stream;
+            TRY(call.open(st));
             TRY(ensure_io());
             cudaStream_t ms = s_out;   // the merge stream
-            counters = pn_counters{};
             if (stats) *stats = pn_shard_stats{};
             const A* q = (const A*)qv;
             const size_t chunk = ps.chunk, n_chunks = ps.n_chunks;
@@ -1772,10 +1775,9 @@ struct Engine final : pn_tree {
                 TRY(sh_ld[b].ensure(chunk * k * 4));
             }
             ps.pack[R] = packall.as<unsigned long long>();
-            while (sh_ev.size() < 2 * n_chunks + 2) { cudaEvent_t e; CU(cudaEventCreate(&e)); sh_ev.push_back(e); }
-            auto EV = [&](size_t c, int i) { return sh_ev[2 * c + i]; };  // scan start / end of chunk c; the last two: merge start / end
-            TRY(begin_call(st));
-            CU(cudaEventRecord(ev[0], st));
+            TRY(grow_events(sh_ev, 2 * n_chunks + 2, cudaEventDefault));
+            auto EV = [&](size_t c, int i) -> cudaEvent_t { return sh_ev[2 * c + i]; };  // scan start / end of chunk c; the last two: merge start / end
+            TRY(call.start());
             for (size_t c = 0; c < n_chunks; ++c) {
                 const int b = (int)(c & 1);
                 const size_t c0 = c * chunk, c1 = std::min(nq, c0 + chunk);
@@ -1834,9 +1836,8 @@ struct Engine final : pn_tree {
     int replicate_send(pn_comm* cm, int root) override {
         if (host_only) return fail(PN_BAD_ARG, "a host-only tree has nothing to replicate");
         if (cm->device != tree->device) return fail(PN_BAD_ARG, "the communicator rank and the tree live on different devices");
-        std::lock_guard<std::mutex> lk(mu);
-        DeviceGuard g(tree->device);
-        if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
+        Call call(*this);
+        TRY(call.device());
         return tree->replicate_send(cm, root);
     }
 
@@ -1845,8 +1846,8 @@ struct Engine final : pn_tree {
     // overlap on the device.
     int session(pn_tree** out) override {
         if (host_only) return fail(PN_BAD_ARG, "a host-only tree has no device arrays to share");
-        std::unique_ptr<Engine<A>> e(new Engine<A>(tree));
-        TRY(e->open_device());
+        std::unique_ptr<Engine> e;
+        TRY(open(tree, false, e));
         e->info = info;
         e->owns_tree = false;
         *out = e.release();
@@ -1882,6 +1883,38 @@ struct Engine final : pn_tree {
 template <typename A>
 static int finish_create(int kind, std::unique_ptr<Engine<A>>& e, const pn_build_opts& o, std::chrono::steady_clock::time_point t0, pn_tree** out);
 
+// The caller's build options, as far as its struct_size reaches (none: the defaults on the current device), with the
+// bucket size normalised.
+static pn_build_opts read_build_opts(const pn_build_opts* in) {
+    pn_build_opts o{};
+    if (in) memcpy(&o, in, std::min<size_t>(sizeof(o), in->struct_size ? in->struct_size : sizeof(o)));
+    else o.device = -1;
+    o.bucket_size = o.bucket_size ? std::max(o.bucket_size, 8u) : 256;
+    return o;
+}
+// the checks every tree build makes, after those of its entry point
+static int check_build_opts(const pn_build_opts& o, int kind) {
+    if (o.prune > PN_PRUNE_OFF) return fail(PN_BAD_ARG, "bad prune option");
+    if (o.partition > PN_PARTITION_TWO_MEANS) return fail(PN_BAD_ARG, "bad partition option");
+    if (o.shard_depth && (kind != PN_KIND_BALL || o.shard_depth > 16 || o.shard_index >= (1u << o.shard_depth)))
+        return fail(PN_BAD_ARG, kind != PN_KIND_BALL ? "subtree sharding is a ball-tree option" : "bad shard_depth / shard_index");
+    return PN_OK;
+}
+// A new handle with an empty tree on the device of `o` (-1: the current one) for the build to fill
+template <typename A>
+static int new_tree_handle(const pn_build_opts& o, bool host_only, std::unique_ptr<Engine<A>>& e) {
+    int dev = o.device;
+    if (!host_only && dev < 0 && cudaGetDevice(&dev) != cudaSuccess) {
+        (void)cudaGetLastError();
+        return fail(PN_CUDA, "no CUDA device available (there is no CPU fallback)");
+    }
+    auto t = std::make_shared<DeviceTree<A>>();
+    t->device = dev;
+    t->algo = o.algo;
+    t->prune_opt = o.prune;
+    return Engine<A>::open(std::move(t), host_only, e);
+}
+
 template <typename A>
 static int create_tree(int kind, const A* points, size_t n, size_t d, size_t row_stride, size_t col_stride,
                        const pn_build_opts* opts_in, pn_tree** out) {
@@ -1893,43 +1926,23 @@ static int create_tree(int kind, const A* points, size_t n, size_t d, size_t row
     if (d == 0) return fail(PN_BAD_ARG, "points have zero columns");
     if (n >= 0xFFFFFFFFull) return fail(PN_BAD_ARG, "n must be < 2^32 - 1 (u32 indices inside the engine)");
     if (n > 1 && row_stride < d) return fail(PN_BAD_ARG, "row_stride < dimension");
-    pn_build_opts o{};
-    if (opts_in) memcpy(&o, opts_in, std::min<size_t>(sizeof(o), opts_in->struct_size ? opts_in->struct_size : sizeof(o)));
-    else o.device = -1;
-    const size_t dpad = (d + VT<A>::N - 1) / VT<A>::N * VT<A>::N;
-    (void)dpad;
-    uint32_t bucket = o.bucket_size ? o.bucket_size : 256;
-    if (bucket < 8) bucket = 8;
+    const pn_build_opts o = read_build_opts(opts_in);
+    const uint32_t bucket = o.bucket_size;
     uint32_t threads = o.host_threads ? o.host_threads : std::max(1u, std::thread::hardware_concurrency());
     auto t0 = std::chrono::steady_clock::now();
     std::unique_ptr<Engine<A>> e;
     const bool host_only = (o.flags & PN_FLAG_HOST_ONLY) != 0;
     if (o.builder > PN_BUILDER_DEVICE) return fail(PN_BAD_ARG, "bad builder");
-    if (o.prune > PN_PRUNE_OFF) return fail(PN_BAD_ARG, "bad prune option");
-    if (o.partition > PN_PARTITION_TWO_MEANS) return fail(PN_BAD_ARG, "bad partition option");
-    if (o.shard_depth && (kind != PN_KIND_BALL || o.shard_depth > 16 || o.shard_index >= (1u << o.shard_depth)))
-        return fail(PN_BAD_ARG, kind != PN_KIND_BALL ? "subtree sharding is a ball-tree option" : "bad shard_depth / shard_index");
+    TRY(check_build_opts(o, kind));
     // ball trees with a device are built there from 32768 points up (bit-identical layout, tests/test_gpu_build.py)
     const bool on_device = !host_only && (o.builder == PN_BUILDER_DEVICE || (o.builder == PN_BUILDER_AUTO && n >= 32768));
     if (o.builder == PN_BUILDER_DEVICE && !on_device) return fail(PN_BAD_ARG, "the device builder needs a device");
-    int dev = o.device;
-    if (!host_only && dev < 0) {
-        if (cudaGetDevice(&dev) != cudaSuccess) {
-            (void)cudaGetLastError();
-            return fail(PN_CUDA, "no CUDA device available (there is no CPU fallback)");
-        }
-    }
     try {
-        e.reset(new Engine<A>(std::make_shared<DeviceTree<A>>()));
-        e->host_only = host_only;
+        TRY(new_tree_handle(o, host_only, e));
         DeviceTree<A>& t = *e->tree;
-        t.device = dev;
-        t.algo = o.algo;
-        t.prune_opt = o.prune;
-        if (!host_only) TRY(e->open_device());
         if (on_device) {
             // raw rows to the device (dense n x d), partition and flatten there
-            DeviceGuard g(dev);
+            DeviceGuard g(t.device);
             if (!g.ok) return fail(PN_CUDA, "no usable CUDA device (there is no CPU fallback)");
             DevBuf raw;
             TRY(raw.ensure(n * d * sizeof(A)));
@@ -1958,7 +1971,7 @@ static int create_tree(int kind, const A* points, size_t n, size_t d, size_t row
     if (!host_only && !on_device) TRY(t.upload(e->stream));
     if (kind == PN_KIND_VP && !host_only && t.tensor_ready && n >= 1024) {
         // the ball partition of the same points for the tensor path (see DeviceTree::part); a failure here only loses the speed-up
-        DeviceGuard g(dev);
+        DeviceGuard g(t.device);
         DevBuf raw;
         std::shared_ptr<DeviceTree<A>> ball;
         if (g.ok && raw.ensure(n * d * sizeof(A)) == PN_OK &&
@@ -2009,29 +2022,17 @@ static int create_tree_dev(const A* points_dev, size_t n, size_t d, size_t row_s
     if (d == 0) return fail(PN_BAD_ARG, "points have zero columns");
     if (n >= 0xFFFFFFFFull) return fail(PN_BAD_ARG, "n must be < 2^32 - 1 (u32 indices inside the engine)");
     if (n > 1 && row_stride < d) return fail(PN_BAD_ARG, "row_stride < dimension");
-    pn_build_opts o{};
-    if (opts_in) memcpy(&o, opts_in, std::min<size_t>(sizeof(o), opts_in->struct_size ? opts_in->struct_size : sizeof(o)));
-    else o.device = -1;
+    const pn_build_opts o = read_build_opts(opts_in);
     if (o.flags & PN_FLAG_HOST_ONLY) return fail(PN_BAD_ARG, "device-resident points cannot build a host-only tree");
     if (o.builder == PN_BUILDER_HOST) return fail(PN_BAD_ARG, "device-resident points are built on the device");
-    if (o.prune > PN_PRUNE_OFF) return fail(PN_BAD_ARG, "bad prune option");
-    if (o.partition > PN_PARTITION_TWO_MEANS) return fail(PN_BAD_ARG, "bad partition option");
-    if (o.shard_depth && (o.shard_depth > 16 || o.shard_index >= (1u << o.shard_depth))) return fail(PN_BAD_ARG, "bad shard_depth / shard_index");
-    uint32_t bucket = o.bucket_size ? o.bucket_size : 256;
-    if (bucket < 8) bucket = 8;
-    int dev = o.device;
-    if (dev < 0 && cudaGetDevice(&dev) != cudaSuccess) { (void)cudaGetLastError(); return fail(PN_CUDA, "no CUDA device available (there is no CPU fallback)"); }
+    TRY(check_build_opts(o, PN_KIND_BALL));
     auto t0 = std::chrono::steady_clock::now();
     std::unique_ptr<Engine<A>> e;
     try {
-        e.reset(new Engine<A>(std::make_shared<DeviceTree<A>>()));
+        TRY(new_tree_handle(o, false, e));
         DeviceTree<A>& t = *e->tree;
-        t.device = dev;
-        t.algo = o.algo;
-        t.prune_opt = o.prune;
-        TRY(e->open_device());
-        TRY(t.build_on_device(points_dev, n, d, row_stride, bucket, o.shard_depth, o.shard_index, 0, e->stream));
-        if (!o.shard_depth) t.two_means_partition(o.partition, bucket, e->stream, t.part);
+        TRY(t.build_on_device(points_dev, n, d, row_stride, o.bucket_size, o.shard_depth, o.shard_index, 0, e->stream));
+        if (!o.shard_depth) t.two_means_partition(o.partition, o.bucket_size, e->stream, t.part);
     } catch (const std::bad_alloc&) {
         return fail(PN_OOM, "host allocation failed while building the tree");
     }
@@ -2042,9 +2043,10 @@ static int create_tree_dev(const A* points_dev, size_t n, size_t d, size_t row_s
 template <typename A>
 static int receive_replica(pn_comm* cm, int root, int kind, pn_tree** out) {
     auto t0 = std::chrono::steady_clock::now();
-    std::unique_ptr<Engine<A>> e(new Engine<A>(std::make_shared<DeviceTree<A>>()));
-    TRY(e->tree->replicate_recv(cm, root));
-    TRY(e->open_device());
+    auto t = std::make_shared<DeviceTree<A>>();
+    TRY(t->replicate_recv(cm, root));
+    std::unique_ptr<Engine<A>> e;
+    TRY(Engine<A>::open(std::move(t), false, e));
     pn_build_opts o{};
     o.algo = e->tree->algo;
     return finish_create<A>(kind, e, o, t0, out);
@@ -2363,8 +2365,6 @@ struct pn_multi {
             for (size_t j = 0; j < i; ++j) dup |= trees[j] == trees[i];
             if (!dup) delete trees[i];
         }
-        for (auto& v : peer.ev_scan)
-            for (cudaEvent_t e : v) if (e) cudaEventDestroy(e);
         for (pn_comm* c : comms) pn_comm_destroy(c);
     }
 };
@@ -2395,8 +2395,7 @@ int32_t pn_multi_balltree_create_f32(const int32_t* devices, int32_t n_dev, uint
     uint32_t depth = 0;
     while ((1 << depth) < n_dev) ++depth;
     if (mode == PN_SHARD_BY_SUBTREE && (1 << depth) != n_dev) return fail(PN_BAD_ARG, "sharding by subtree needs a power-of-two number of devices");
-    pn_build_opts o{};
-    if (opts_in) memcpy(&o, opts_in, std::min<size_t>(sizeof(o), opts_in->struct_size ? opts_in->struct_size : sizeof(o)));
+    pn_build_opts o = read_build_opts(opts_in);
     o.struct_size = sizeof(o);
     if (o.flags & PN_FLAG_HOST_ONLY) return fail(PN_BAD_ARG, "a multi-GPU tree cannot be host-only");
     std::unique_ptr<pn_multi> m(new pn_multi());
@@ -2432,7 +2431,7 @@ int32_t pn_multi_balltree_create_f32(const int32_t* devices, int32_t n_dev, uint
             }
         m->peer.n = n_dev;
         m->peer.pack.assign(n_dev, nullptr);
-        m->peer.ev_scan.assign(n_dev, {});
+        m->peer.ev_scan.resize(n_dev);
         if (m->peer_ok) m->exchange = PN_EXCHANGE_PEER;
     }
     *out = m.release();
@@ -2453,11 +2452,7 @@ int32_t pn_multi_balltree_query_f32(pn_multi* m, const float* q, size_t nq, size
         m->peer.n_chunks = (nq + m->peer.chunk - 1) / m->peer.chunk;
         for (int r = 0; r < W; ++r) {
             DeviceGuard g(m->devices[r]);
-            while (m->peer.ev_scan[r].size() < m->peer.n_chunks) {
-                cudaEvent_t e;
-                CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                m->peer.ev_scan[r].push_back(e);
-            }
+            TRY(grow_events(m->peer.ev_scan[r], m->peer.n_chunks, cudaEventDisableTiming));
         }
     }
     return on_every_rank(W, [&](int r) -> int {

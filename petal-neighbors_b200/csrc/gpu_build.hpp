@@ -96,7 +96,7 @@ int build_vp_tree(const A* raw, uint64_t n, uint32_t d, uint64_t stride, uint32_
                   VpOut<A> (*alloc_out)(void* ctx, uint64_t n, const VpShape& shape), void* ctx, cudaStream_t st, std::string& err);
 
 // mean of the stored rows (double accumulation over fixed chunks of 4096 rows combined in chunk order: the same value
-// as the host pass of Engine::prepare_tensor) and the largest centred coordinate max |p_j - c_j|
+// as the host pass of DeviceTree::prepare_tensor) and the largest centred coordinate max |p_j - c_j|
 int centre_and_range_f32(const float* pts, uint64_t n, uint32_t d, uint32_t dpad, float* center_dev, float* center_host,
                          float* maxabs, cudaStream_t st, std::string& err);
 

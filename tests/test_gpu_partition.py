@@ -1,4 +1,4 @@
-"""The two-means partition behind the pruned tensor scan (csrc/gpu_build.cu rule 1, Engine::two_means_partition).
+"""The two-means partition behind the pruned tensor scan (csrc/gpu_build.cu rule 1, DeviceTree::two_means_partition).
 
 A handle on clustered data keeps a second ball tree over the same rows whose splits follow 2-means directions and whose
 nodes start on tile boundaries; k-NN batches are answered from it.  The reference's pruning rule is the same
