@@ -255,6 +255,15 @@ int32_t pn_merge_topk_dev(uint32_t dtype, int32_t device, const uint64_t *idx_li
                           const void *dist_lists_dev, size_t n_lists, size_t nq, size_t k,
                           uint64_t *idx_out_dev, void *dist_out_dev, void *stream, int32_t sync);
 
+/* Merge of n_lists per-shard CSR radius results over the same nq queries (the step after the exchange when points are
+ * sharded by subtree; no reference equivalent).  offsets_lists_dev[n_lists][nq + 1] are absolute positions into
+ * indices_lists_dev; each list's segment of a query is ascending.  out_offsets_dev[nq + 1]; out_indices_dev holds
+ * sum over lists of (offsets[l][nq] - offsets[l][0]) entries.  Equal indices from different lists are kept, in list
+ * order.  All pointers are device pointers on `device`. */
+int32_t pn_merge_radius_dev(int32_t device, const uint64_t *offsets_lists_dev, const uint64_t *indices_lists_dev,
+                            size_t n_lists, size_t nq, uint64_t *out_offsets_dev, uint64_t *out_indices_dev,
+                            void *stream, int32_t sync);
+
 /* --- multi-GPU inside the library (SURVEY.md 8e; no reference equivalent: the crate is single-threaded).
  * A pn_comm is ONE RANK of an NCCL communicator bound to one device.  One process per GPU: rank 0 calls
  * pn_comm_unique_id, the host language ships the 128 bytes to the other ranks (MPI, torch.distributed, a file ...), every
@@ -318,12 +327,21 @@ int32_t pn_multi_balltree_create_f32(const int32_t *devices, int32_t n_dev, uint
                                      size_t n, size_t d, size_t row_stride, const pn_build_opts *opts, pn_multi **out);
 int32_t pn_multi_balltree_query_f32(pn_multi *m, const float *queries, size_t nq, size_t q_row_stride, size_t k,
                                     uint64_t *idx_out, float *dist_out);
+/* Radius search on a multi-GPU handle: the CSR result pn_balltree_query_radius_f32 returns on a tree of all the points
+ * (strict distance < r, each query's indices ascending), engine-allocated, released with pn_free.
+ * REPLICATE: every device answers its slice of the batch.  BY_SUBTREE: every device answers all queries on its shard, the
+ * owner of each slice pulls the shards' hit lists of its slice with peer copies (no NCCL; pn_multi_set_exchange applies to
+ * k-NN only) and merges them on its device.  Each slice is written straight into its region of the single result. */
+int32_t pn_multi_balltree_query_radius_f32(pn_multi *m, const float *queries, size_t nq, size_t q_row_stride,
+                                           float radius, uint64_t **offsets_out, uint64_t **indices_out);
 /* How the per-shard lists of a BY_SUBTREE handle meet: PN_EXCHANGE_PEER (the default when every pair of devices has peer
  * access) runs NO collective -- the k-way merge kernel of each device reads the other devices' packed lists directly from
  * their memory over NVLink (the exchange fused into the consumer); PN_EXCHANGE_SLICE uses grouped ncclSend/ncclRecv. */
 #define PN_EXCHANGE_PEER 2u
 int32_t pn_multi_set_exchange(pn_multi *m, uint32_t exchange);
-/* per-device statistics of the last query: stats[n_dev] (BY_SUBTREE: the exchange; REPLICATE: zeros but rows_out) */
+/* per-device statistics of the last query: stats[n_dev] (BY_SUBTREE: the exchange; REPLICATE: zeros but rows_out).  After a
+ * radius search: scan_ms = traversal, exchange_ms = peer pulls, merge_ms = counts + offsets scan + merge, total_ms, rows_out,
+ * n_chunks (traversal chunks), peer_mib = MiB pulled from other devices; no NCCL calls. */
 int32_t pn_multi_get_stats(const pn_multi *m, pn_shard_stats *stats, int32_t n_stats);
 int32_t pn_multi_destroy(pn_multi *m);
 

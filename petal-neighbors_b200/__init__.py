@@ -29,7 +29,7 @@ from ._ffi import (PN_ALGO_AUTO, PN_ALGO_SIMT, PN_ALGO_TENSOR, PN_BUILDER_AUTO, 
                    PN_PRUNE_AUTO, PN_PRUNE_ON, PN_PRUNE_OFF,
                    PN_PARTITION_AUTO, PN_PARTITION_REFERENCE, PN_PARTITION_TWO_MEANS)
 
-__all__ = ["BallTree", "VantagePointTree", "ArrayError", "EngineError", "distance", "merge_topk_dev",
+__all__ = ["BallTree", "VantagePointTree", "ArrayError", "EngineError", "distance", "merge_topk_dev", "merge_radius_dev",
            "PN_ALGO_AUTO", "PN_ALGO_SIMT", "PN_ALGO_TENSOR", "PN_BUILDER_AUTO", "PN_BUILDER_HOST", "PN_BUILDER_DEVICE", "PN_PRUNE_AUTO", "PN_PRUNE_ON", "PN_PRUNE_OFF",
            "PN_PARTITION_AUTO", "PN_PARTITION_REFERENCE", "PN_PARTITION_TWO_MEANS"]
 
@@ -75,6 +75,23 @@ def _strides(a):
     rs = a.strides[0] // it if a.shape[0] > 1 else max(a.shape[1], 1)
     cs = a.strides[1] // it if a.shape[1] > 1 else 1
     return rs, cs
+
+
+def _csr_arrays(offs_p, idx_p, nq):
+    """The engine-allocated CSR result of a radius call as numpy arrays (offsets[nq + 1], indices), zero-copy: the buffers
+    back the arrays and are released with pn_free when the arrays are garbage-collected (the Rust shim's
+    Vec::from_raw_parts equivalent)."""
+    L = _ffi.lib()
+    offsets = np.ctypeslib.as_array(offs_p, shape=(nq + 1,))
+    weakref.finalize(offsets, L.pn_free, C.cast(offs_p, C.c_void_p))
+    total = int(offsets[-1])
+    if total:
+        indices = np.ctypeslib.as_array(idx_p, shape=(total,))
+        weakref.finalize(indices, L.pn_free, C.cast(idx_p, C.c_void_p))
+    else:
+        indices = np.empty(0, np.uint64)
+        L.pn_free(idx_p)
+    return offsets, indices
 
 
 class _Tree:
@@ -218,18 +235,7 @@ class _Tree:
         idx_p = C.POINTER(C.c_uint64)()
         fn = getattr(L, f"pn_{self._kind}_query_radius_{self._sfx}")
         _check(fn(self._h, Q.ctypes.data if nq else None, nq, qs, self.dtype.type(radius), C.byref(offs_p), C.byref(idx_p)))
-        # zero-copy: the engine-allocated buffers back the arrays and are released with pn_free when
-        # the arrays are garbage-collected (the Rust shim's Vec::from_raw_parts equivalent)
-        offsets = np.ctypeslib.as_array(offs_p, shape=(nq + 1,))
-        weakref.finalize(offsets, L.pn_free, C.cast(offs_p, C.c_void_p))
-        total = int(offsets[-1])
-        if total:
-            indices = np.ctypeslib.as_array(idx_p, shape=(total,))
-            weakref.finalize(indices, L.pn_free, C.cast(idx_p, C.c_void_p))
-        else:
-            indices = np.empty(0, np.uint64)
-            L.pn_free(idx_p)
-        return offsets, indices
+        return _csr_arrays(offs_p, idx_p, nq)
 
     def query_knn_dev(self, q_ptr: int, nq: int, q_row_stride: int, k: int, idx_ptr: int, dist_ptr: int,
                       stream: int = 0, sync: bool = True):
@@ -321,3 +327,12 @@ def merge_topk_dev(dtype, device: int, idx_lists_ptr: int, dist_lists_ptr: int, 
     code = _ffi.PN_F32 if np.dtype(dtype) == np.float32 else _ffi.PN_F64
     _check(_ffi.lib().pn_merge_topk_dev(code, device, idx_lists_ptr, dist_lists_ptr, n_lists, nq, k, idx_out_ptr,
                                         dist_out_ptr, stream, 1 if sync else 0))
+
+
+def merge_radius_dev(device: int, offsets_ptr: int, indices_ptr: int, n_lists: int, nq: int, out_offsets_ptr: int,
+                     out_indices_ptr: int, stream: int = 0, sync: bool = True):
+    """pn_merge_radius_dev: merge of n_lists CSR radius results over the same nq queries (device pointers, u64).
+    offsets[n_lists][nq + 1] are absolute positions into the indices; each list's segment of a query is ascending.  The
+    merged CSR has each query's indices ascending; equal indices from different lists are all kept, in list order."""
+    _check(_ffi.lib().pn_merge_radius_dev(device, offsets_ptr, indices_ptr, n_lists, nq, out_offsets_ptr, out_indices_ptr,
+                                          stream, 1 if sync else 0))

@@ -29,11 +29,11 @@ EXPORTS = [
     "pn_vptree_query_f32", "pn_vptree_query_f64", "pn_vptree_query_radius_f32", "pn_vptree_query_radius_f64",
     "pn_balltree_query_self_f32", "pn_balltree_query_self_f64", "pn_tree_query_self_dev",
     "pn_pairwise_f32", "pn_pairwise_f64",
-    "pn_free", "pn_tree_query_knn_dev", "pn_merge_topk_dev",
+    "pn_free", "pn_tree_query_knn_dev", "pn_merge_topk_dev", "pn_merge_radius_dev",
     "pn_tree_get_info", "pn_tree_get_counters", "pn_tree_get_layout",
     "pn_comm_unique_id", "pn_comm_create", "pn_comm_create_all", "pn_comm_destroy", "pn_query_slice",
     "pn_sharded_query_knn_dev", "pn_tree_replicate",
-    "pn_multi_balltree_create_f32", "pn_multi_balltree_query_f32", "pn_multi_set_exchange", "pn_multi_get_stats", "pn_multi_destroy",
+    "pn_multi_balltree_create_f32", "pn_multi_balltree_query_f32", "pn_multi_balltree_query_radius_f32", "pn_multi_set_exchange", "pn_multi_get_stats", "pn_multi_destroy",
 ]
 PN_SHARD_REPLICATE, PN_SHARD_BY_SUBTREE = 0, 1
 PN_EXCHANGE_ALLGATHER, PN_EXCHANGE_SLICE, PN_EXCHANGE_PEER = 0, 1, 2
@@ -130,6 +130,8 @@ def lib():
     L.pn_tree_query_self_dev.argtypes = [vp, sz, vp, vp, vp, C.c_int32]
     L.pn_merge_topk_dev.restype = C.c_int32
     L.pn_merge_topk_dev.argtypes = [C.c_uint32, C.c_int32, vp, vp, sz, sz, sz, vp, vp, vp, C.c_int32]
+    L.pn_merge_radius_dev.restype = C.c_int32
+    L.pn_merge_radius_dev.argtypes = [C.c_int32, vp, vp, sz, sz, vp, vp, vp, C.c_int32]
     L.pn_tree_get_info.restype = C.c_int32
     L.pn_tree_get_info.argtypes = [vp, C.POINTER(TreeInfo)]
     L.pn_tree_get_counters.restype = C.c_int32
@@ -154,6 +156,8 @@ def lib():
     L.pn_multi_balltree_create_f32.argtypes = [C.POINTER(C.c_int32), C.c_int32, C.c_uint32, vp, sz, sz, sz, C.POINTER(BuildOpts), C.POINTER(vp)]
     L.pn_multi_balltree_query_f32.restype = C.c_int32
     L.pn_multi_balltree_query_f32.argtypes = [vp, vp, sz, sz, sz, vp, vp]
+    L.pn_multi_balltree_query_radius_f32.restype = C.c_int32
+    L.pn_multi_balltree_query_radius_f32.argtypes = [vp, vp, sz, sz, C.c_float, C.POINTER(u64p), C.POINTER(u64p)]
     L.pn_multi_set_exchange.restype = C.c_int32
     L.pn_multi_set_exchange.argtypes = [vp, C.c_uint32]
     L.pn_multi_get_stats.restype = C.c_int32

@@ -158,11 +158,21 @@ using namespace petal;
 
 // State shared by the rank threads of one pn_multi query in PEER mode: every rank's packed-list buffers and events, and a
 // host barrier the rank threads meet at (an event must have been RECORDED before another rank's stream can wait on it).
+// Radius search uses the barrier and the r_* fields.
 struct PeerShared {
     int n = 0;
     size_t chunk = 0, n_chunks = 0;                           // the chunking of this query (the same on every rank)
     std::vector<const unsigned long long*> pack;              // [rank] packed lists of ALL queries of this call
     std::vector<std::vector<Event>> ev_scan;                  // [rank][chunk]: lists of that chunk are packed
+    // radius search: [rank] CSR of the rank's shard over all queries (BY_SUBTREE), its offsets at the W + 1 slice
+    // boundaries, the hits of the rank's slice; the single result, allocated by rank 0 once every slice total is known
+    std::vector<const uint64_t*> r_offs;
+    std::vector<const uint32_t*> r_hits;
+    std::vector<int> r_dev;
+    std::vector<std::vector<uint64_t>> r_bound;
+    std::vector<uint64_t> r_total;
+    uint64_t* r_out_offs = nullptr;
+    uint64_t* r_out_hits = nullptr;
     std::mutex mu;
     std::condition_variable cv;
     int count = 0, gen = 0;
@@ -177,6 +187,9 @@ struct PeerShared {
         return !failed;
     }
     void fail() { std::lock_guard<std::mutex> lk(mu); failed = true; cv.notify_all(); }
+    // the status of a rank that leaves because another one failed; on_every_rank reports the failure that released it
+    static constexpr const char* RELEASED = "another rank failed";
+    static int released() { return petal::fail(PN_CUDA, RELEASED); }
 };
 
 // The opaque handle.
@@ -200,6 +213,8 @@ struct pn_tree {
     virtual size_t shard_chunk(size_t nq) const = 0;
     virtual int knn_sharded_peer(PeerShared& ps, int rank, int world, const void* q, size_t nq, size_t stride, size_t k, uint64_t* idx, void* dist,
                                  pn_shard_stats* stats) = 0;
+    virtual int radius_multi(PeerShared& ps, int rank, int world, bool by_subtree, const void* q, size_t nq, size_t stride, double r,
+                             pn_shard_stats* stats) = 0;
 };
 
 namespace petal {
@@ -660,6 +675,8 @@ struct Engine final : pn_tree {
     DevBuf w_qraw2[2], w_oi2[2], w_od2[2];
     DevBuf sh_li[2], sh_ld[2], sh_pack[2], sh_gat[2], sh_gat_d[2];   // sharded k-NN: local lists, packed keys, gathered lists
     DevBuf r_qraw[2], r_q[2], r_counts[2], r_offsets[2], r_hits[2], r_slab[2], r_qlist[2], r_nlist[2], r_sums[2];  // radius pipeline workspaces
+    // radius search of a multi-GPU handle: queries, the CSR of radius_device, the lists pulled from every shard, their merge
+    DevBuf rd_q, rd_offs, rd_hits, rp_offs, rp_hits, rm_offs, rm_hits;
     // tensor path (f32 input only): per-call workspaces, see tc_filter.cuh
     DevBuf w_aaug, w_qmargin, w_trace, w_gbound;
     // pruned tensor scan (tc_prune.cuh): per-call workspaces
@@ -1455,6 +1472,110 @@ struct Engine final : pn_tree {
         return p;
     }
 
+    // the host step of copy_out_staged for radius hits: u32 on the device, u64 at dst
+    static auto widen_to(uint64_t* dst) {
+        return [dst](size_t off, const unsigned char* sp, size_t lo, size_t hi) {
+            const uint32_t* s32 = (const uint32_t*)sp;
+            uint64_t* d64 = dst + off / 4;
+            for (size_t i = lo / 4; i < hi / 4; ++i) d64[i] = s32[i];
+        };
+    }
+
+    // ---- the device stages of radius search over one chunk of at most `chunk` queries, in workspace set b, on stream s.
+    // Split in two because the host must size the hit buffer from the count pass before the fill pass runs.
+    static constexpr uint32_t RADIUS_WPB = 8;   // warps (queries) per block of the traversal, compaction and sort
+    int radius_workspace(const DeviceTree<A>& t, int n_sets, size_t chunk) {
+        for (int b = 0; b < n_sets; ++b) {
+            TRY(r_q[b].ensure(chunk * t.ft.dpad * sizeof(A)));
+            TRY(r_counts[b].ensure(chunk * 4));
+            TRY(r_offsets[b].ensure((chunk + 1) * 8));
+            TRY(r_sums[b].ensure((chunk / SCAN_BLOCK + 1) * 8));
+            TRY(r_slab[b].ensure(chunk * RADIUS_CAP * 4));
+            TRY(r_qlist[b].ensure(chunk * 4));
+            TRY(r_nlist[b].ensure(16));
+        }
+        return PN_OK;
+    }
+    // pad the queries (row stride q_stride elements), count traversal with the first RADIUS_CAP hits of each query in its
+    // slab, chunk-local offsets (r_offsets[b][cq] is the chunk's total)
+    int radius_count(const DeviceTree<A>& t, int b, const A* q, size_t q_stride, uint32_t cq, A r, cudaStream_t s) {
+        const size_t tot = (size_t)cq * t.ft.dpad;
+        pad_queries_kernel<A><<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(q, q_stride, cq, t.ft.d, t.ft.dpad, r_q[b].as<A>());
+        CU(cudaGetLastError());
+        const unsigned blocks = (cq + RADIUS_WPB - 1) / RADIUS_WPB;
+        CU(cudaMemsetAsync(r_nlist[b].p, 0, 4, s));
+        radius_kernel<A, 0><<<blocks, RADIUS_WPB * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, r_counts[b].as<uint32_t>(), nullptr, r_slab[b].as<uint32_t>(),
+                                                              w_counters.as<unsigned long long>());
+        CU(cudaGetLastError());
+        const unsigned sblocks = std::max(1u, (cq + SCAN_BLOCK - 1) / SCAN_BLOCK);
+        scan_sums_kernel<<<sblocks, 1024, 0, s>>>(r_counts[b].as<uint32_t>(), cq, r_sums[b].as<unsigned long long>());
+        offsets_scan_kernel<<<sblocks, 1024, 0, s>>>(r_counts[b].as<uint32_t>(), r_sums[b].as<unsigned long long>(), r_offsets[b].as<uint64_t>(), cq);
+        CU(cudaGetLastError());
+        counters.kernel_launches += 4;
+        return PN_OK;
+    }
+    // slabs -> hits[0 .. ctotal) at the chunk-local offsets, second traversal of the queries that overflowed their slab,
+    // per-query ascending sort
+    int radius_fill(const DeviceTree<A>& t, int b, uint32_t cq, A r, uint64_t ctotal, uint32_t* hits, cudaStream_t s) {
+        const unsigned blocks = (cq + RADIUS_WPB - 1) / RADIUS_WPB;
+        compact_hits_kernel<<<blocks, RADIUS_WPB * 32, 0, s>>>(r_slab[b].as<uint32_t>(), r_counts[b].as<uint32_t>(), r_offsets[b].as<uint64_t>(), cq,
+                                                               hits, r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
+        CU(cudaGetLastError());
+        // second traversal for the queries that overflowed their slab only (warps past the list length exit at once)
+        radius_kernel<A, 1><<<blocks, RADIUS_WPB * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, nullptr, r_offsets[b].as<uint64_t>(), hits,
+                                                              nullptr, r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
+        CU(cudaGetLastError());
+        segment_sort_kernel<<<blocks, RADIUS_WPB * 32, 0, s>>>(r_offsets[b].as<uint64_t>(), hits, cq);
+        CU(cudaGetLastError());
+        if (ctotal > SORT_WARP_MAX) {  // some hit list may be longer than a warp should sort: one block per such query
+            segment_sort_large_kernel<<<std::min<uint32_t>(cq, 8u * (uint32_t)n_sms), 256, 0, s>>>(r_offsets[b].as<uint64_t>(), hits, cq);
+            CU(cudaGetLastError());
+            ++counters.kernel_launches;
+        }
+        counters.kernel_launches += 3;
+        return PN_OK;
+    }
+
+    // Radius search of nq queries already on the tree's device (row stride `stride` elements), called under an open Call
+    // on its stream st: the CSR result is left in rd_offs (u64, nq + 1 entries over the whole batch) and rd_hits (u32, each
+    // query's hits ascending).  The chunks of radius_host run one after the other on one workspace set, so the workspace
+    // stays bounded per chunk; only the hits grow with the result.  *total_out = rd_offs[nq].
+    int radius_device(const DeviceTree<A>& t, const A* q, size_t nq, size_t stride, A r, cudaStream_t st, uint64_t* total_out,
+                      uint32_t* n_chunks_out) {
+        const size_t chunk = nq <= (1u << 18) ? std::max<size_t>(nq, 1) : (1u << 17);
+        const size_t n_chunks = (nq + chunk - 1) / chunk;
+        TRY(rd_offs.ensure((nq + 1) * 8));
+        TRY(rd_hits.ensure(4));
+        TRY(radius_workspace(t, 1, chunk));
+        if (!pin_tot) TRY(pin_tot.create(2 * sizeof(unsigned long long)));
+        CU(cudaMemsetAsync(rd_offs.p, 0, 8, st));
+        uint64_t total = 0;
+        for (size_t c = 0; c < n_chunks; ++c) {
+            const size_t q0 = c * chunk;
+            const uint32_t cq = (uint32_t)std::min(chunk, nq - q0);
+            TRY(radius_count(t, 0, q + q0 * stride, stride, cq, r, st));
+            CU(cudaMemcpyAsync(pin_tot.as<unsigned long long>(), r_offsets[0].as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, st));
+            CU(cudaStreamSynchronize(st));
+            const uint64_t ctotal = pin_tot.as<unsigned long long>()[0];
+            if ((total + ctotal) * 4 > rd_hits.cap) {
+                // sized as radius_host sizes its result; a later, denser chunk grows it, keeping the hits of the earlier ones
+                const size_t want = c == 0 ? (size_t)((double)ctotal * 1.12 * (double)nq / cq) + 1024 : rd_hits.cap / 4 + rd_hits.cap / 8;
+                DevBuf nb;
+                TRY(nb.ensure(std::max<size_t>(total + ctotal, want) * 4));
+                if (total) CU(cudaMemcpyAsync(nb.p, rd_hits.p, total * 4, cudaMemcpyDeviceToDevice, st));
+                rd_hits = std::move(nb);
+            }
+            TRY(radius_fill(t, 0, cq, r, ctotal, rd_hits.as<uint32_t>() + total, st));
+            rebase_offsets_kernel<<<(cq + 255) / 256, 256, 0, st>>>(r_offsets[0].as<uint64_t>() + 1, cq, 0, total, rd_offs.as<uint64_t>() + q0 + 1);
+            CU(cudaGetLastError());
+            ++counters.kernel_launches;
+            total += ctotal;
+        }
+        *total_out = total;
+        *n_chunks_out = (uint32_t)n_chunks;
+        return PN_OK;
+    }
+
     // Two-stage software pipeline over chunks of queries, two workspace sets on two streams:
     //   A(c): H2D queries, pad, count traversal, offsets scan, chunk total -> pinned word
     //   B(c): fill traversal at the offsets, per-query sort, D2H of offsets and hits (widened u32 -> u64 on the host)
@@ -1486,20 +1607,11 @@ struct Engine final : pn_tree {
         size_t hit_cap = 0, total = 0;
         const size_t chunk = nq <= (1u << 18) ? std::max<size_t>(nq, 1) : (1u << 17);
         const size_t n_chunks = (nq + chunk - 1) / chunk;
-        const uint32_t wpb = 8;
         last_used_tensor = false; last_pruned = false;
         if (!pin_tot) TRY(pin_tot.create(2 * sizeof(unsigned long long)));
         const size_t spitch = std::max<size_t>(stride, t.ft.d) * sizeof(A);
-        for (int b = 0; b < (n_chunks > 1 ? 2 : 1); ++b) {
-            TRY(r_qraw[b].ensure(chunk * t.ft.d * sizeof(A)));
-            TRY(r_q[b].ensure(chunk * t.ft.dpad * sizeof(A)));
-            TRY(r_counts[b].ensure(chunk * 4));
-            TRY(r_offsets[b].ensure((chunk + 1) * 8));
-            TRY(r_sums[b].ensure((chunk / SCAN_BLOCK + 1) * 8));
-            TRY(r_slab[b].ensure(chunk * RADIUS_CAP * 4));
-            TRY(r_qlist[b].ensure(chunk * 4));
-            TRY(r_nlist[b].ensure(16));
-        }
+        for (int b = 0; b < (n_chunks > 1 ? 2 : 1); ++b) TRY(r_qraw[b].ensure(chunk * t.ft.d * sizeof(A)));
+        TRY(radius_workspace(t, n_chunks > 1 ? 2 : 1, chunk));
         TRY(call.start());
         CU(cudaEventRecord(ev[2], st));
         for (int b = 0; b < 2; ++b) CU(cudaStreamWaitEvent(sx[b], ev[0], 0));
@@ -1509,22 +1621,9 @@ struct Engine final : pn_tree {
             const uint32_t cq = (uint32_t)std::min(chunk, nq - q0);
             cudaStream_t s = sx[b];
             CU(cudaMemcpy2DAsync(r_qraw[b].p, t.ft.d * sizeof(A), q + q0 * stride, spitch, t.ft.d * sizeof(A), cq, cudaMemcpyHostToDevice, s));
-            const size_t tot = (size_t)cq * t.ft.dpad;
-            pad_queries_kernel<A><<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(r_qraw[b].as<A>(), t.ft.d, cq, t.ft.d, t.ft.dpad, r_q[b].as<A>());
-            CU(cudaGetLastError());
-            const unsigned blocks = (cq + wpb - 1) / wpb;
-            CU(cudaMemsetAsync(r_nlist[b].p, 0, 4, s));
-            radius_kernel<A, 0><<<blocks, wpb * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, r_counts[b].as<uint32_t>(), nullptr, r_slab[b].as<uint32_t>(),
-                                                           w_counters.as<unsigned long long>());
-            CU(cudaGetLastError());
-            const unsigned sblocks = std::max(1u, (cq + SCAN_BLOCK - 1) / SCAN_BLOCK);
-            scan_sums_kernel<<<sblocks, 1024, 0, s>>>(r_counts[b].as<uint32_t>(), cq, r_sums[b].as<unsigned long long>());
-            offsets_scan_kernel<<<sblocks, 1024, 0, s>>>(r_counts[b].as<uint32_t>(), r_sums[b].as<unsigned long long>(), r_offsets[b].as<uint64_t>(), cq);
-            CU(cudaGetLastError());
-            ++counters.kernel_launches;
+            TRY(radius_count(t, b, r_qraw[b].as<A>(), t.ft.d, cq, r, s));
             CU(cudaMemcpyAsync(&pin_tot.as<unsigned long long>()[b], r_offsets[b].as<uint64_t>() + cq, 8, cudaMemcpyDeviceToHost, s));
             CU(cudaEventRecord(e_in[b], s));
-            counters.kernel_launches += 3;
             counters.h2d_bytes += (uint64_t)cq * t.ft.d * sizeof(A);
             return PN_OK;
         };
@@ -1546,31 +1645,10 @@ struct Engine final : pn_tree {
                 hit_buf = std::move(nb); hit_cap = ncap;
             }
             TRY(r_hits[b].ensure((ctotal ? ctotal : 1) * 4));
-            const unsigned blocks = (cq + wpb - 1) / wpb;
-            compact_hits_kernel<<<blocks, wpb * 32, 0, s>>>(r_slab[b].as<uint32_t>(), r_counts[b].as<uint32_t>(), r_offsets[b].as<uint64_t>(), cq,
-                                                            r_hits[b].as<uint32_t>(), r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
-            CU(cudaGetLastError());
-            // second traversal for the queries that overflowed their slab only (warps past the list length exit at once)
-            radius_kernel<A, 1><<<blocks, wpb * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, nullptr, r_offsets[b].as<uint64_t>(), r_hits[b].as<uint32_t>(),
-                                                           nullptr, r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
-            CU(cudaGetLastError());
-            ++counters.kernel_launches;
-            segment_sort_kernel<<<blocks, wpb * 32, 0, s>>>(r_offsets[b].as<uint64_t>(), r_hits[b].as<uint32_t>(), cq);
-            CU(cudaGetLastError());
-            if (ctotal > SORT_WARP_MAX) {  // some hit list may be longer than a warp should sort: one block per such query
-                segment_sort_large_kernel<<<std::min<uint32_t>(cq, 8u * (uint32_t)n_sms), 256, 0, s>>>(r_offsets[b].as<uint64_t>(), r_hits[b].as<uint32_t>(), cq);
-                CU(cudaGetLastError());
-                ++counters.kernel_launches;
-            }
-            counters.kernel_launches += 2;
+            TRY(radius_fill(t, b, cq, r, ctotal, r_hits[b].as<uint32_t>(), s));
             CU(cudaMemcpyAsync(offs.get() + q0 + 1, r_offsets[b].as<uint64_t>() + 1, (size_t)cq * 8, cudaMemcpyDeviceToHost, s));
             // the hits, u32 on the device, widened to u64 on up to 12 host threads
-            uint64_t* dst = hit_buf.get() + total;
-            TRY(copy_out_staged(r_hits[b].p, ctotal * 4, s, 12, 4, [dst](size_t off, const unsigned char* sp, size_t lo, size_t hi) {
-                const uint32_t* s32 = (const uint32_t*)sp;
-                uint64_t* d64 = dst + off / 4;
-                for (size_t i = lo / 4; i < hi / 4; ++i) d64[i] = s32[i];
-            }));
+            TRY(copy_out_staged(r_hits[b].p, ctotal * 4, s, 12, 4, widen_to(hit_buf.get() + total)));
             CU(cudaStreamSynchronize(s));
             if (total) for (uint32_t i = 1; i <= cq; ++i) offs[q0 + i] += total;  // chunk-local -> global offsets
             total += ctotal;
@@ -1792,7 +1870,7 @@ struct Engine final : pn_tree {
                 CU(cudaEventRecord(EV(c, 1), st));
                 CU(cudaEventRecord(ps.ev_scan[R][c], st));
             }
-            if (!ps.barrier()) return fail(PN_CUDA, "another rank failed");   // every rank's buffers exist and all scan events are recorded
+            if (!ps.barrier()) return ps.released();   // every rank's buffers exist and all scan events are recorded
             std::vector<const unsigned long long*> hp(ps.pack.begin(), ps.pack.end());
             CU(cudaMemcpyAsync(ptrs.p, hp.data(), hp.size() * sizeof(void*), cudaMemcpyHostToDevice, ms));
             unsigned long long rows_out = 0, peer_bytes = 0;
@@ -1816,7 +1894,7 @@ struct Engine final : pn_tree {
             CU(cudaEventRecord(ev[1], st));
             CU(cudaStreamSynchronize(st));
             // nobody may free or reuse a packed buffer while a peer still reads it
-            if (!ps.barrier()) return fail(PN_CUDA, "another rank failed");
+            if (!ps.barrier()) return ps.released();
             guard.ok = true;
             if (stats) {
                 float ms_ = 0.f;
@@ -1830,6 +1908,137 @@ struct Engine final : pn_tree {
                 stats->peer_mib = (uint32_t)std::min<unsigned long long>((peer_bytes + (1u << 20) - 1) >> 20, 0xffffffffull);
             }
             return fetch_counters(st, nq);
+        }
+    }
+
+    // ---- radius search of a multi-GPU handle (pn_multi_balltree_query_radius_f32), called on every rank's thread.  `q` holds
+    // the caller's nq host queries; rank R owns result rows [lo, hi) = pn_query_slice(nq, R, W).
+    //   REPLICATE: radius_device over the slice on this rank's replica.
+    //   BY_SUBTREE: radius_device over ALL queries on this rank's shard; once the ranks have met, the owner of a slice pulls
+    //   every shard's offsets and hits of that slice into local staging (cudaMemcpyPeerAsync: over NVLink with peer access,
+    //   staged by the driver without it; no collective, so pn_multi_set_exchange does not apply) and merges the lists by
+    //   rank (merge_radius_lists, u32).  Shard trees hold global ids, so the hits need no translation.
+    // Then every rank publishes its slice total; rank 0 allocates the single result once all totals are known, and every
+    // rank writes its offsets (plus the totals of the slices before it) and its hits, widened to u64, into its region.
+    int radius_multi(PeerShared& ps, int R, int W, bool by_subtree, const void* qv, size_t nq, size_t stride, double rr,
+                     pn_shard_stats* stats) override {
+        if constexpr (sizeof(A) != 4) {
+            (void)ps; (void)R; (void)W; (void)by_subtree; (void)qv; (void)nq; (void)stride; (void)rr; (void)stats;
+            return fail(PN_BAD_ARG, "multi-GPU radius search serves f32 trees");
+        } else {
+            struct Guard { PeerShared& p; bool ok = false; ~Guard() { if (!ok) p.fail(); } } guard{ps};
+            TRY(check_query_args(qv, nq, stride));
+            if (stats) *stats = pn_shard_stats{};
+            size_t lo, hi;
+            pn_query_slice(nq, R, W, &lo, &hi);
+            const size_t rows = hi - lo, nql = by_subtree ? nq : rows;   // rows owned, queries traversed
+            const size_t d = tree->ft.d;
+            Call call(*this);
+            const cudaStream_t st = stream;
+            TRY(call.open(st));
+            // on an error return, a copy into the caller's result may still be queued: the device finishes before the
+            // result is freed (declared after `guard` and `call`, so destroyed first)
+            struct SyncOnError { bool armed = true; ~SyncOnError() { if (armed) cudaDeviceSynchronize(); } } sync_on_error;
+            last_used_tensor = false; last_pruned = false;
+            TRY(rd_q.ensure(std::max<size_t>(nql, 1) * d * 4));
+            TRY(grow_events(sh_ev, 5, cudaEventDefault));   // traversal start / end, pulls end, merge end, pulls start
+            TRY(call.start());
+            if (nql) {
+                const float* q = (const float*)qv + (by_subtree ? 0 : lo * stride);
+                CU(cudaMemcpy2DAsync(rd_q.p, d * 4, q, std::max(stride, d) * 4, d * 4, nql, cudaMemcpyHostToDevice, st));
+            }
+            counters.h2d_bytes = (uint64_t)nql * d * 4;
+            CU(cudaEventRecord(sh_ev[0], st));
+            uint64_t slice_total = 0;
+            uint32_t n_chunks = 0;
+            TRY(radius_device(*tree, rd_q.as<float>(), nql, d, (float)rr, st, &slice_total, &n_chunks));
+            CU(cudaEventRecord(sh_ev[1], st));
+            const uint64_t* offs_dev = rd_offs.as<uint64_t>();   // this rank's slice as CSR on the device
+            const uint32_t* hits_dev = rd_hits.as<uint32_t>();
+            unsigned long long peer_bytes = 0;
+            const bool pulled = by_subtree && rows;
+            if (by_subtree) {
+                std::vector<uint64_t>& bnd = ps.r_bound[R];   // this shard's offsets at every rank's slice start, and at nq
+                bnd.assign(W + 1, 0);
+                for (int j = 0; j <= W; ++j) {
+                    size_t b = nq;
+                    if (j < W) pn_query_slice(nq, j, W, &b, nullptr);
+                    CU(cudaMemcpyAsync(&bnd[j], rd_offs.as<uint64_t>() + b, 8, cudaMemcpyDeviceToHost, st));
+                }
+                CU(cudaStreamSynchronize(st));
+                ps.r_offs[R] = rd_offs.as<uint64_t>();
+                ps.r_hits[R] = rd_hits.as<uint32_t>();
+                ps.r_dev[R] = tree->device;
+                if (!ps.barrier()) return ps.released();   // every shard's CSR is complete
+                std::vector<uint64_t> base(W + 1, 0);   // where shard s's hits of this slice start in the pulled staging
+                for (int s = 0; s < W; ++s) base[s + 1] = base[s] + (ps.r_bound[s][R + 1] - ps.r_bound[s][R]);
+                slice_total = base[W];
+                if (pulled) {
+                    TRY(rp_offs.ensure((size_t)W * (rows + 1) * 8));
+                    TRY(rp_hits.ensure(std::max<uint64_t>(slice_total, 1) * 4));
+                    TRY(rm_offs.ensure((rows + 1) * 8));
+                    TRY(rm_hits.ensure(std::max<uint64_t>(slice_total, 1) * 4));
+                    TRY(r_counts[0].ensure(rows * 4));
+                    TRY(r_sums[0].ensure((rows / SCAN_BLOCK + 1) * 8));
+                    uint64_t* po = rp_offs.as<uint64_t>();
+                    CU(cudaEventRecord(sh_ev[4], st));
+                    for (int s = 0; s < W; ++s) {
+                        const uint64_t nh = base[s + 1] - base[s];
+                        CU(cudaMemcpyPeerAsync(po + (size_t)s * (rows + 1), tree->device, ps.r_offs[s] + lo, ps.r_dev[s], (rows + 1) * 8, st));
+                        if (nh) CU(cudaMemcpyPeerAsync(rp_hits.as<uint32_t>() + base[s], tree->device, ps.r_hits[s] + ps.r_bound[s][R], ps.r_dev[s], nh * 4, st));
+                        if (s != R) peer_bytes += (rows + 1) * 8 + nh * 4;
+                    }
+                    CU(cudaEventRecord(sh_ev[2], st));
+                    // shard s's offsets into its own hit array -> positions in the concatenation of the pulled hits
+                    for (int s = 0; s < W; ++s)
+                        rebase_offsets_kernel<<<(unsigned)((rows + 1 + 255) / 256), 256, 0, st>>>(po + (size_t)s * (rows + 1), rows + 1, ps.r_bound[s][R],
+                                                                                                 base[s], po + (size_t)s * (rows + 1));
+                    const unsigned blocks = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((slice_total + 255) / 256, 8ull * n_sms));
+                    CU(merge_radius_lists<uint32_t>(st, po, rp_hits.as<uint32_t>(), (uint32_t)W, (uint32_t)rows, rm_offs.as<uint64_t>(),
+                                                    rm_hits.as<uint32_t>(), r_counts[0].as<uint32_t>(), r_sums[0].as<unsigned long long>(), blocks));
+                    CU(cudaEventRecord(sh_ev[3], st));
+                    counters.kernel_launches += (uint64_t)W + 4;
+                    offs_dev = rm_offs.as<uint64_t>();
+                    hits_dev = rm_hits.as<uint32_t>();
+                }
+                // the pulls are done before this rank passes the next barrier, so no rank reads another's buffers after it
+                CU(cudaStreamSynchronize(st));
+            }
+            ps.r_total[R] = slice_total;
+            if (!ps.barrier()) return ps.released();   // every slice total is known
+            if (R == 0) {
+                uint64_t all = 0;
+                for (uint64_t t : ps.r_total) all += t;
+                ps.r_out_offs = (uint64_t*)result_alloc((nq + 1) * 8);
+                ps.r_out_hits = (uint64_t*)result_alloc(all * 8);
+                if (!ps.r_out_offs || !ps.r_out_hits) return fail(PN_OOM, "allocating the result");
+                ps.r_out_offs[0] = 0;
+            }
+            if (!ps.barrier()) return ps.released();   // the result is allocated
+            if (rows) {
+                uint64_t base = 0;
+                for (int j = 0; j < R; ++j) base += ps.r_total[j];
+                uint64_t* offs_out = ps.r_out_offs + lo;
+                CU(cudaMemcpyAsync(offs_out + 1, offs_dev + 1, rows * 8, cudaMemcpyDeviceToHost, st));
+                TRY(copy_out_staged(hits_dev, slice_total * 4, st, 12, 4, widen_to(ps.r_out_hits + base)));
+                CU(cudaStreamSynchronize(st));
+                if (base) for (size_t i = 1; i <= rows; ++i) offs_out[i] += base;
+            }
+            counters.d2h_bytes = (uint64_t)rows * 8 + slice_total * 4;
+            TRY(call.finish(nql));
+            sync_on_error.armed = false;
+            guard.ok = true;
+            if (stats) {
+                float ms = 0.f;
+                if (cudaEventElapsedTime(&ms, sh_ev[0], sh_ev[1]) == cudaSuccess) stats->scan_ms = ms;
+                if (pulled && cudaEventElapsedTime(&ms, sh_ev[4], sh_ev[2]) == cudaSuccess) stats->exchange_ms = ms;
+                if (pulled && cudaEventElapsedTime(&ms, sh_ev[2], sh_ev[3]) == cudaSuccess) stats->merge_ms = ms;
+                (void)cudaGetLastError();
+                stats->total_ms = counters.device_ms;
+                stats->rows_out = rows; stats->n_chunks = n_chunks;
+                stats->peer_mib = (uint32_t)std::min<unsigned long long>((peer_bytes + (1u << 20) - 1) >> 20, 0xffffffffull);
+            }
+            return PN_OK;
         }
     }
 
@@ -2068,6 +2277,32 @@ static int merge_topk_dev(int device, const uint64_t* idx_lists, const A* dist_l
     return PN_OK;
 }
 
+static int merge_radius_dev(int device, const uint64_t* offsets, const uint64_t* indices, size_t n_lists, size_t nq, uint64_t* out_offsets,
+                            uint64_t* out_indices, cudaStream_t st, bool sync) {
+    if (!offsets || !indices || !out_offsets || !out_indices) return fail(PN_BAD_ARG, "null pointer");
+    if (n_lists == 0 || n_lists > (size_t)MAX_LISTS) return fail(PN_BAD_ARG, "n_lists must be in 1..256");
+    if (nq >= (1ull << 32)) return fail(PN_BAD_ARG, "nq must be < 2^32");
+    DeviceGuard g(device);
+    if (!g.ok) return fail(PN_CUDA, "cudaSetDevice failed");
+    if (nq == 0) {
+        CU(cudaMemsetAsync(out_offsets, 0, 8, st));
+    } else {
+        int n_sms = 0;
+        CU(cudaDeviceGetAttribute(&n_sms, cudaDevAttrMultiProcessorCount, device));
+        // stream-ordered workspace (sums, then the u32 counts), so the call does not synchronise the device
+        const size_t sums_bytes = ((nq / SCAN_BLOCK + 1) * 8 + 255) / 256 * 256;
+        void* ws = nullptr;
+        CU(cudaMallocAsync(&ws, sums_bytes + nq * 4, st));
+        const cudaError_t e = merge_radius_lists<uint64_t>(st, offsets, indices, (uint32_t)n_lists, (uint32_t)nq, out_offsets, out_indices,
+                                                           (uint32_t*)((char*)ws + sums_bytes), (unsigned long long*)ws, 8u * (unsigned)n_sms);
+        const cudaError_t ef = cudaFreeAsync(ws, st);
+        CU(e);
+        CU(ef);
+    }
+    if (sync) CU(cudaStreamSynchronize(st));
+    return PN_OK;
+}
+
 template <typename A>
 static int pairwise_host(int device, const A* x, size_t n, size_t d, size_t row_stride, A* out) {
     if (n == 0) return PN_OK;
@@ -2228,6 +2463,11 @@ int32_t pn_merge_topk_dev(uint32_t dtype, int32_t device, const uint64_t* il, co
     GUARD_END
 }
 
+int32_t pn_merge_radius_dev(int32_t device, const uint64_t* ol, const uint64_t* il, size_t n_lists, size_t nq, uint64_t* oo, uint64_t* io,
+                            void* stream, int32_t sync) {
+    GUARD_BEGIN return merge_radius_dev(device, ol, il, n_lists, nq, oo, io, (cudaStream_t)stream, sync != 0); GUARD_END
+}
+
 // ---- multi-GPU: communicator ranks, sharded k-NN, replication ---------------------------------------------------------
 void pn_query_slice(size_t nq, int32_t rank, int32_t world, size_t* lo, size_t* hi) {
     if (world < 1) world = 1;
@@ -2380,8 +2620,10 @@ static int on_every_rank(int n, F fn) {
             if (rc[r] != PN_OK) msg[r] = g_err;
         });
     for (auto& t : th) t.join();
-    for (int r = 0; r < n; ++r)
-        if (rc[r] != PN_OK) return fail(rc[r], "device rank " + std::to_string(r) + ": " + msg[r]);
+    int first = -1;   // the first rank that failed on its own, else the first that was released by another's failure
+    for (int r = n - 1; r >= 0; --r)
+        if (rc[r] != PN_OK && (first < 0 || msg[r] != PeerShared::RELEASED || msg[first] == PeerShared::RELEASED)) first = r;
+    if (first >= 0) return fail(rc[first], "device rank " + std::to_string(first) + ": " + msg[first]);
     return PN_OK;
 }
 extern "C" {
@@ -2405,6 +2647,7 @@ int32_t pn_multi_balltree_create_f32(const int32_t* devices, int32_t n_dev, uint
     m->trees.assign(n_dev, nullptr);
     m->stats.assign(n_dev, pn_shard_stats{});
     m->q_dev.resize(n_dev); m->idx_dev.resize(n_dev); m->dist_dev.resize(n_dev);
+    m->peer.n = n_dev;
     TRY(pn_comm_create_all(devices, n_dev, m->comms.data()));
     if (mode == PN_SHARD_REPLICATE) {
         pn_build_opts o0 = o;
@@ -2429,7 +2672,6 @@ int32_t pn_multi_balltree_create_f32(const int32_t* devices, int32_t n_dev, uint
                 if (e != cudaSuccess && e != cudaErrorPeerAccessAlreadyEnabled) m->peer_ok = false;
                 (void)cudaGetLastError();
             }
-        m->peer.n = n_dev;
         m->peer.pack.assign(n_dev, nullptr);
         m->peer.ev_scan.resize(n_dev);
         if (m->peer_ok) m->exchange = PN_EXCHANGE_PEER;
@@ -2484,6 +2726,42 @@ int32_t pn_multi_balltree_query_f32(pn_multi* m, const float* q, size_t nq, size
         }
         return PN_OK;
     });
+    GUARD_END
+}
+int32_t pn_multi_balltree_query_radius_f32(pn_multi* m, const float* q, size_t nq, size_t qs, float radius, uint64_t** offsets_out,
+                                           uint64_t** indices_out) {
+    GUARD_BEGIN
+    if (!offsets_out || !indices_out) return fail(PN_BAD_ARG, "output pointer is null");
+    if (nq && !q) return fail(PN_BAD_ARG, "queries is null");
+    if (nq >= (1ull << 32)) return fail(PN_BAD_ARG, "nq must be < 2^32 per call");
+    if (!m) return fail(PN_BAD_ARG, "handle is null");
+    if (nq > 1 && qs < m->d) return fail(PN_BAD_ARG, "q_row_stride < dimension");
+    const int W = m->n_dev;
+    for (int r = 0; r < W; ++r) m->stats[r] = pn_shard_stats{};
+    PeerShared& ps = m->peer;
+    { std::lock_guard<std::mutex> lk(ps.mu); ps.failed = false; ps.count = 0; }
+    ps.r_offs.assign(W, nullptr); ps.r_hits.assign(W, nullptr); ps.r_dev.assign(W, -1);
+    ps.r_bound.assign(W, {}); ps.r_total.assign(W, 0);
+    ps.r_out_offs = nullptr; ps.r_out_hits = nullptr;
+    int rc = PN_OK;
+    if (nq == 0) {   // as pn_balltree_query_radius_f32: offsets {0} and an empty index array, both for pn_free
+        ps.r_out_offs = (uint64_t*)malloc(8);
+        ps.r_out_hits = (uint64_t*)malloc(8);
+        if (ps.r_out_offs) ps.r_out_offs[0] = 0;
+        if (!ps.r_out_offs || !ps.r_out_hits) rc = fail(PN_OOM, "malloc offsets");
+    } else {
+        rc = on_every_rank(W, [&](int r) -> int {
+            return m->trees[r]->radius_multi(ps, r, W, m->mode == PN_SHARD_BY_SUBTREE, q, nq, qs, (double)radius, &m->stats[r]);
+        });
+    }
+    if (rc != PN_OK) {
+        free(ps.r_out_offs); free(ps.r_out_hits);
+        ps.r_out_offs = nullptr; ps.r_out_hits = nullptr;
+        return rc;
+    }
+    *offsets_out = ps.r_out_offs; *indices_out = ps.r_out_hits;
+    ps.r_out_offs = nullptr; ps.r_out_hits = nullptr;
+    return PN_OK;
     GUARD_END
 }
 int32_t pn_multi_set_exchange(pn_multi* m, uint32_t exchange) {

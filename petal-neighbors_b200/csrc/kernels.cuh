@@ -1042,6 +1042,108 @@ __global__ void offsets_scan_kernel(const uint32_t* __restrict__ counts, const u
     if (n == 0 && blockIdx.x == 0 && threadIdx.x == 0) offsets[0] = 0;
 }
 
+// add to every entry of a u64 offset array: out[i] = in[i] - sub + add (chunk-local CSR offsets -> batch offsets, pulled
+// offsets -> positions in the concatenation of the pulled hit lists).  in == out is allowed.
+__global__ void rebase_offsets_kernel(const uint64_t* in, size_t n, uint64_t sub, uint64_t add, uint64_t* out) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = in[i] - sub + add;
+}
+
+// ---- merge of n_lists CSR radius results over the same nq queries (per-shard hit lists of a point set sharded by
+// subtree).  offsets[l * (nq + 1) + q] are absolute positions into one indices array; list l holds the entries
+// [offsets[l][0], offsets[l][nq]) and its segment of query q, [offsets[l][q], offsets[l][q + 1]), is non-decreasing.
+// Segment lengths per query, u32, for scan_sums_kernel + offsets_scan_kernel (a decreasing pair counts as empty; a sum
+// beyond u32 saturates, and merge_radius_lists_kernel then drops what no longer fits its row).
+__global__ void merge_radius_counts_kernel(const uint64_t* __restrict__ offsets, uint32_t n_lists, uint32_t nq,
+                                           uint32_t* __restrict__ counts) {
+    const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    unsigned long long c = 0;
+    for (uint32_t l = 0; l < n_lists; ++l) {
+        const uint64_t a = offsets[(size_t)l * ((size_t)nq + 1) + q], b = offsets[(size_t)l * ((size_t)nq + 1) + q + 1];
+        c += b > a ? b - a : 0;
+    }
+    counts[q] = (uint32_t)min(c, 0xffffffffull);
+}
+
+// first position in [lo, hi) whose value is > v (UPPER) or >= v (!UPPER)
+template <bool UPPER, typename I>
+__device__ __forceinline__ uint64_t csr_bound(const I* __restrict__ v, uint64_t lo, uint64_t hi, I x) {
+    while (lo < hi) {
+        const uint64_t mid = lo + (hi - lo) / 2;
+        const I y = v[mid];
+        if (UPPER ? y <= x : y < x) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+// Merge by rank, one thread per input element, no sort and no per-query work split: element j of list s's segment of
+// query q (value v) goes to out_offsets[q] + j + (entries <= v in the segments of q of lists before s) + (entries < v in
+// those of lists after s).  That is a stable merge: equal values from different lists are all kept, in list order, so a
+// query with millions of hits costs no more than as many queries with few.  The grid strides over the n_lists entries
+// counted in the list lengths (offsets[l][nq] - offsets[l][0]); every block rebuilds their prefix in shared memory, so the
+// host needs to know neither the total nor any offset.  Bounds: an element is read only from its list's range
+// [offsets[s][0], offsets[s][nq]), written only when its query was found (offsets[s][q] <= p < offsets[s][q + 1]), and
+// only to a position inside [out_offsets[q], out_offsets[q + 1]) that is also below the sum of the list lengths (the
+// capacity of out_indices: with offsets that decrease, the counts above can add up to more) -- indices that are not sorted
+// or offsets that are not monotone give a wrong result, never an out-of-bounds write.
+template <typename I>
+__global__ void __launch_bounds__(256) merge_radius_lists_kernel(const uint64_t* __restrict__ offsets, const I* __restrict__ indices,
+                                                                 uint32_t n_lists, uint32_t nq, const uint64_t* __restrict__ out_offsets,
+                                                                 I* __restrict__ out_indices) {
+    __shared__ unsigned long long start[MAX_LISTS + 1];   // start[l]: first element of list l in the grid's numbering
+    if (threadIdx.x == 0) {
+        unsigned long long s = 0;
+        for (uint32_t l = 0; l < n_lists; ++l) {
+            start[l] = s;
+            const uint64_t a = offsets[(size_t)l * ((size_t)nq + 1)], b = offsets[(size_t)l * ((size_t)nq + 1) + nq];
+            s += b > a ? b - a : 0;
+        }
+        start[n_lists] = s;
+    }
+    __syncthreads();
+    const unsigned long long total = start[n_lists];
+    for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (unsigned long long)gridDim.x * blockDim.x) {
+        uint32_t lo = 0, hi = n_lists;   // the list: last l with start[l] <= i (empty lists share their start with the next)
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) / 2;
+            if (start[mid] <= i) lo = mid; else hi = mid;
+        }
+        const uint32_t s = lo;
+        const uint64_t* os = offsets + (size_t)s * ((size_t)nq + 1);
+        const uint64_t p = os[0] + (i - start[s]);
+        // the query: last q with os[q] <= p
+        uint32_t qa = 0, qb = nq;
+        while (qb - qa > 1) {
+            const uint32_t mid = qa + (qb - qa) / 2;
+            if (os[mid] <= p) qa = mid; else qb = mid;
+        }
+        const uint32_t q = qa;
+        if (!(os[q] <= p && p < os[q + 1])) continue;
+        const I v = indices[p];
+        uint64_t pos = out_offsets[q] + (p - os[q]);
+        for (uint32_t l = 0; l < n_lists; ++l) {
+            if (l == s) continue;
+            const uint64_t a = offsets[(size_t)l * ((size_t)nq + 1) + q], b = offsets[(size_t)l * ((size_t)nq + 1) + q + 1];
+            if (b <= a) continue;
+            pos += (l < s ? csr_bound<true>(indices, a, b, v) : csr_bound<false>(indices, a, b, v)) - a;
+        }
+        if (pos < out_offsets[q + 1] && pos < total) out_indices[pos] = v;
+    }
+}
+// The whole merge on `st` (nq >= 1): counts, the offsets scan, the merge on `blocks` blocks.  Workspaces: counts[nq],
+// sums[nq / SCAN_BLOCK + 1].
+template <typename I>
+inline cudaError_t merge_radius_lists(cudaStream_t st, const uint64_t* offsets, const I* indices, uint32_t n_lists, uint32_t nq,
+                                      uint64_t* out_offsets, I* out_indices, uint32_t* counts, unsigned long long* sums, unsigned blocks) {
+    merge_radius_counts_kernel<<<(unsigned)(((size_t)nq + 255) / 256), 256, 0, st>>>(offsets, n_lists, nq, counts);
+    const unsigned sblocks = (unsigned)(((size_t)nq + SCAN_BLOCK - 1) / SCAN_BLOCK);
+    scan_sums_kernel<<<sblocks, 1024, 0, st>>>(counts, nq, sums);
+    offsets_scan_kernel<<<sblocks, 1024, 0, st>>>(counts, sums, out_offsets, nq);
+    merge_radius_lists_kernel<I><<<blocks, 256, 0, st>>>(offsets, indices, n_lists, nq, out_offsets, out_indices);
+    return cudaGetLastError();
+}
+
 // ascending sort of each query's hit list (the reference's order is unspecified DFS order and its tests sort before
 // comparing, src/ball_tree.rs:667, 777): bitonic network over the segment padded to a power of two with virtual +inf
 // keys.  Segments of up to SORT_WARP_MAX entries are sorted by one warp each; longer ones (large radii: whole subtrees

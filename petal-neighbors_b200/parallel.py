@@ -21,7 +21,7 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from . import BallTree, _Tree, _check, _ffi, merge_topk_dev  # noqa: F401
+from . import BallTree, _Tree, _check, _csr_arrays, _ffi, merge_radius_dev, merge_topk_dev  # noqa: F401
 from ._ffi import PN_EXCHANGE_ALLGATHER, PN_EXCHANGE_PEER, PN_EXCHANGE_SLICE, PN_SHARD_BY_SUBTREE, PN_SHARD_REPLICATE
 
 
@@ -184,6 +184,20 @@ class MultiGpuBallTree:
         dist = np.empty((nq, k), np.float32)
         _check(_ffi.lib().pn_multi_balltree_query_f32(self._h, Q.ctypes.data, nq, self.dim, k, idx.ctypes.data, dist.ctypes.data))
         return idx, dist
+
+    def query_radius_batch(self, Q, radius):
+        """pn_multi_balltree_query_radius_f32: CSR (offsets[nq+1], indices), as BallTree.query_radius_batch returns it
+        for a tree of all the points (strict `distance < radius`, each query's indices ascending).  BY_SUBTREE handles pull
+        the per-shard hit lists with peer copies and merge them on the device; no NCCL, whatever set_exchange chose."""
+        Q = np.ascontiguousarray(Q, dtype=np.float32)
+        if Q.ndim != 2 or Q.shape[1] != self.dim:
+            raise ValueError("queries must be nq x d")
+        nq = Q.shape[0]
+        offs_p = C.POINTER(C.c_uint64)()
+        idx_p = C.POINTER(C.c_uint64)()
+        _check(_ffi.lib().pn_multi_balltree_query_radius_f32(self._h, Q.ctypes.data if nq else None, nq, self.dim, np.float32(radius),
+                                                            C.byref(offs_p), C.byref(idx_p)))
+        return _csr_arrays(offs_p, idx_p, nq)
 
     def set_exchange(self, exchange: int):
         """BY_SUBTREE handles: PN_EXCHANGE_PEER (merge kernels read the other devices' lists over NVLink, no collective; the

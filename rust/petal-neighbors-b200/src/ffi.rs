@@ -72,7 +72,12 @@ extern "C" {
                                         row_stride: usize, opts: *const pn_build_opts, out: *mut *mut pn_multi) -> i32;
     pub fn pn_multi_balltree_query_f32(m: *mut pn_multi, q: *const f32, nq: usize, q_row_stride: usize, k: usize,
                                        idx: *mut u64, dist: *mut f32) -> i32;
+    pub fn pn_multi_balltree_query_radius_f32(m: *mut pn_multi, q: *const f32, nq: usize, q_row_stride: usize, radius: f32,
+                                              offsets: *mut *mut u64, indices: *mut *mut u64) -> i32;
     pub fn pn_multi_destroy(m: *mut pn_multi) -> i32;
+    // merge of per-shard CSR radius results on one device (all pointers are device pointers)
+    pub fn pn_merge_radius_dev(device: i32, offsets_lists_dev: *const u64, indices_lists_dev: *const u64, n_lists: usize, nq: usize,
+                               out_offsets_dev: *mut u64, out_indices_dev: *mut u64, stream: *mut std::ffi::c_void, sync: i32) -> i32;
 }
 
 #[repr(C)]

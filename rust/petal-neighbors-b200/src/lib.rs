@@ -332,6 +332,24 @@ impl MultiGpuBallTree {
             Array2::from_shape_vec((nq, k), dist).unwrap(),
         )
     }
+
+    /// Batched radius search over all devices: CSR `(offsets[nq + 1], indices)`, as [`BallTree::query_radius_batch`]
+    /// returns it for a tree of all the points.
+    pub fn query_radius_batch(&mut self, queries: &ArrayView2<f32>, distance: f32) -> (Vec<usize>, Vec<usize>) {
+        check_dim(queries.ncols(), self.d, "query batch");
+        let q = queries.as_standard_layout();
+        let nq = q.nrows();
+        let (mut po, mut pi) = (std::ptr::null_mut::<u64>(), std::ptr::null_mut::<u64>());
+        check(unsafe { ffi::pn_multi_balltree_query_radius_f32(self.handle, q.as_ptr(), nq, self.d, distance, &mut po, &mut pi) });
+        unsafe {
+            let offsets: Vec<usize> = std::slice::from_raw_parts(po, nq + 1).iter().map(|&v| v as usize).collect();
+            let total = *offsets.last().unwrap();
+            let indices: Vec<usize> = std::slice::from_raw_parts(pi, total).iter().map(|&v| v as usize).collect();
+            ffi::pn_free(po.cast());
+            ffi::pn_free(pi.cast());
+            (offsets, indices)
+        }
+    }
 }
 
 impl Drop for MultiGpuBallTree {
