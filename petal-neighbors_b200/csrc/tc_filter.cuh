@@ -186,6 +186,36 @@ __device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[32]) {
                  : "memory");
 }
 
+// three-input min (FMNMX3); NaN inputs drop out as in fminf.  Written in PTX: from nested fminf the compiler forms
+// two-input mins of the columns first and spends 38 instructions on 64 columns instead of 32.
+__device__ __forceinline__ float min3f(float a, float b, float c) {
+    float d;
+    asm("min.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
+    return d;
+}
+// Minimum of a 64-column accumulator unit with 31 three-input mins and one two-input min, as one chain: it keeps a
+// single partial minimum live next to the 64 columns, which the hit search still needs (the epilogue runs at 80
+// registers).  The result is <= theta iff some column is (a NaN column never is).
+__device__ __forceinline__ float unit_min64(const uint32_t (&r)[2][32]) {
+    float acc = min3f(__uint_as_float(r[0][0]), __uint_as_float(r[0][1]), __uint_as_float(r[0][2]));
+#pragma unroll
+    for (int c = 3; c < 63; c += 2) acc = min3f(acc, __uint_as_float(r[c / 32][c % 32]), __uint_as_float(r[(c + 1) / 32][(c + 1) % 32]));
+    return fminf(acc, __uint_as_float(r[1][31]));
+}
+// the same wait for the two 32-column groups of a 64-column unit: one tcgen05.wait::ld covers every load issued before it
+__device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[2][32]) {
+    asm volatile("tcgen05.wait::ld.sync.aligned;"
+                 : "+r"(r[0][0]), "+r"(r[0][1]), "+r"(r[0][2]), "+r"(r[0][3]), "+r"(r[0][4]), "+r"(r[0][5]), "+r"(r[0][6]), "+r"(r[0][7]),
+                   "+r"(r[0][8]), "+r"(r[0][9]), "+r"(r[0][10]), "+r"(r[0][11]), "+r"(r[0][12]), "+r"(r[0][13]), "+r"(r[0][14]), "+r"(r[0][15]),
+                   "+r"(r[0][16]), "+r"(r[0][17]), "+r"(r[0][18]), "+r"(r[0][19]), "+r"(r[0][20]), "+r"(r[0][21]), "+r"(r[0][22]), "+r"(r[0][23]),
+                   "+r"(r[0][24]), "+r"(r[0][25]), "+r"(r[0][26]), "+r"(r[0][27]), "+r"(r[0][28]), "+r"(r[0][29]), "+r"(r[0][30]), "+r"(r[0][31]),
+                   "+r"(r[1][0]), "+r"(r[1][1]), "+r"(r[1][2]), "+r"(r[1][3]), "+r"(r[1][4]), "+r"(r[1][5]), "+r"(r[1][6]), "+r"(r[1][7]),
+                   "+r"(r[1][8]), "+r"(r[1][9]), "+r"(r[1][10]), "+r"(r[1][11]), "+r"(r[1][12]), "+r"(r[1][13]), "+r"(r[1][14]), "+r"(r[1][15]),
+                   "+r"(r[1][16]), "+r"(r[1][17]), "+r"(r[1][18]), "+r"(r[1][19]), "+r"(r[1][20]), "+r"(r[1][21]), "+r"(r[1][22]), "+r"(r[1][23]),
+                   "+r"(r[1][24]), "+r"(r[1][25]), "+r"(r[1][26]), "+r"(r[1][27]), "+r"(r[1][28]), "+r"(r[1][29]), "+r"(r[1][30]), "+r"(r[1][31])
+                 :
+                 : "memory");
+}
 // Per-thread running top-k kept in SHARED memory ([slot][lane], conflict-free): it is only touched
 // when the hit queue is drained, and keeping it out of the register file lets the epilogue hold a
 // whole accumulator stage in registers instead.  Only the k-th key / thresh2 live in registers.
@@ -760,42 +790,67 @@ knn_filter_kernel(const __grid_constant__ CUtensorMap map_a, const unsigned char
             // while this one is read out and tested, and the four warps sharing a stage get half a tile of slack against
             // each other (with one whole-tile stage the slowest sibling's hit path gated every tile of its subtile).
             // A stage is released as soon as its columns are in registers, before they are tested.
+            // The no-hit path of a unit is its read-out, one min tree over its 64 columns and one vote: a warp meets a hit
+            // in about one unit in twelve on the seeded d = 16 scan, so everything the search for the hit columns needs
+            // (block minima, column bits, the tail-tile mask) is computed only on the units that have one.
             constexpr int G = SW / 32;          // 32-column groups per unit
+            static_assert(NUM_ACC == U, "unit h of every tile uses accumulator stage h");
             uint32_t r[G][32];
-            const uint32_t lane_off = (uint32_t)(quad * 32) << 16;
-            uint32_t u = 0;
-            PROF_DECL;
-            for (uint32_t jr = 0; jr < n_my; ++jr) {
-                const uint32_t j = PRUNE ? titer.next() : j_begin + jr;  // absolute tile (point rows); stage and phase follow the CTA's own count
+            // per-warp constants: unit h reads stage h at taddr0 + h MT SW and waits on / releases barrier h MT + mt
+            // (a shuffled value: ptxas keeps it instead of rebuilding it from the warp index on every unit)
+            const uint32_t taddr0 = __shfl_sync(full, tmem_base + ((uint32_t)(quad * 32) << 16) + mt * SW, 0);
+            uint64_t* const tfull_w = tfull_bar + mt;
+            uint64_t* const tempty_w = tempty_bar + mt;
+            // hit columns of one 32-column group [col0, col0 + 32) of tile j, searched in blocks of 8: a column is a
+            // candidate iff its value is <= theta (never a NaN)
+            auto hit_bits = [&](const uint32_t (&rg)[32], uint32_t j, int col0) -> uint32_t {
+                uint32_t bits = 0;
 #pragma unroll
-                for (int h = 0; h < U; ++h, ++u) {
-                    const uint32_t as = u % NUM_ACC, aph = (u / NUM_ACC) & 1u;
+                for (int b = 0; b < 4; ++b) {
+                    const float x0 = fminf(__uint_as_float(rg[8 * b]), fminf(__uint_as_float(rg[8 * b + 1]), __uint_as_float(rg[8 * b + 2])));
+                    const float x1 = fminf(__uint_as_float(rg[8 * b + 3]), fminf(__uint_as_float(rg[8 * b + 4]), __uint_as_float(rg[8 * b + 5])));
+                    const float mb = fminf(fminf(x0, x1), fminf(__uint_as_float(rg[8 * b + 6]), __uint_as_float(rg[8 * b + 7])));
+                    if (mb <= theta) {
+#pragma unroll
+                        for (int i = 0; i < 8; ++i) bits |= (__uint_as_float(rg[8 * b + i]) <= theta ? 1u : 0u) << (8 * b + i);
+                    }
+                }
+                if (j + 1 == a.n_tiles) {  // rows past the last point are zero-filled
+                    const int valid = (int)t.n - (int)(j * BN + col0);
+                    if (valid < 32) bits &= valid > 0 ? ((1u << valid) - 1u) : 0u;
+                }
+                return bits;
+            };
+            PROF_DECL;
+            uint32_t jn = j_begin;  // counted along: computing j_begin + jr makes ptxas rebuild j_begin from blockIdx.y every tile
+            for (uint32_t jr = 0; jr < n_my; ++jr, ++jn) {
+                const uint32_t j = PRUNE ? titer.next() : jn;  // absolute tile (point rows); stage and phase follow the CTA's own count
+                const uint32_t aph = jr & 1u;                  // both stages complete once per tile
+#pragma unroll
+                for (int h = 0; h < U; ++h) {
                     PROF_ADD(3);
-                    mbar_wait(&tfull_bar[as * MT + mt], aph);
+                    mbar_wait(tfull_w + h * MT, aph);
                     tc_fence_after();
                     PROF_ADD(0);
                     if (lane == 0 && h == 0) TRACE(warp, j, 0);
-                    const uint32_t taddr = tmem_base + lane_off + (as * MT + mt) * SW;
     #pragma unroll
-                    for (int g = 0; g < G; ++g) tmem_ld32_issue(taddr + g * 32, r[g]);
-    #pragma unroll
-                    for (int g = 0; g < G; ++g) tmem_ld_wait(r[g]);
+                    for (int g = 0; g < G; ++g) tmem_ld32_issue(taddr0 + h * MT * SW + g * 32, r[g]);
+                    tmem_ld_wait(r);
                     tc_fence_before();
                     __syncwarp();
-                    if (lane == 0) mbar_arrive(&tempty_bar[as * MT + mt]);
+                    if (elect_one()) mbar_arrive(tempty_w + h * MT);  // one lane: unlike lane == 0 it needs no thread index
                     PROF_ADD(1);
                     if (lane == 0 && h == 0) TRACE(warp, j, 1);
     #ifdef PN_TC_PROFILE
                     if (a.dbg & 1u) continue;
     #endif
-                    uint32_t bits[G];
-                    uint32_t any = 0;  // groups with a hit in some lane (warp-uniform)
+                    if (__any_sync(full, unit_min64(r) <= theta)) {
+                        // both groups are searched against the same theta before either is pushed
+                        uint32_t bits[G];
     #pragma unroll
-                    for (int g = 0; g < G; ++g) any |= test32(r[g], j, (h * G + g) * 32, bits[g]) ? 1u << g : 0u;
-                    if (any) {
+                        for (int g = 0; g < G; ++g) bits[g] = hit_bits(r[g], j, (h * G + g) * 32);
     #pragma unroll
-                        for (int g = 0; g < G; ++g)
-                            if (any & (1u << g)) push32(bits[g], j, (h * G + g) * 32);
+                        for (int g = 0; g < G; ++g) push32(bits[g], j, (h * G + g) * 32);
                     }
                     PROF_ADD(2);
                 }
