@@ -226,7 +226,10 @@ int32_t pn_vptree_query_radius_f64(pn_tree *tree, const double *queries, size_t 
  * benches/ball_tree.rs:53-59, and the k-NN-graph shape of downstream clustering).  Row i of the
  * n x k outputs is the answer for points[i]; the point itself is its own first neighbour
  * (distance 0, lowest index among exact duplicates).  No query upload: the stored, bucket-ordered
- * points are the query tiles. */
+ * points are the query tiles.  pn_tree_query_self_dev is the same call into device buffers (n x k on the tree's
+ * device; `stream` and `sync` as for pn_tree_query_knn_dev below).  It takes any handle of a whole tree -- ball or
+ * vantage-point tree, or a session of either -- and gives the same rows on each; a handle that holds one shard of a
+ * tree (shard_depth > 0) returns PN_BAD_ARG. */
 int32_t pn_balltree_query_self_f32(pn_tree *tree, size_t k, uint64_t *idx_out, float *dist_out);
 int32_t pn_balltree_query_self_f64(pn_tree *tree, size_t k, uint64_t *idx_out, double *dist_out);
 int32_t pn_tree_query_self_dev(pn_tree *tree, size_t k, uint64_t *idx_dev, void *dist_dev, void *stream,

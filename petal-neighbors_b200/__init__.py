@@ -243,6 +243,11 @@ class _Tree:
         _check(_ffi.lib().pn_tree_query_knn_dev(self._h, q_ptr, nq, q_row_stride, k, idx_ptr, dist_ptr, stream,
                                                 1 if sync else 0))
 
+    def query_self_dev(self, k: int, idx_ptr: int, dist_ptr: int, stream: int = 0, sync: bool = True):
+        """Device-pointer self-query (pn_tree_query_self_dev): every stored point is a query, row i of the n x k
+        outputs (already in HBM) is the answer for points[i]."""
+        _check(_ffi.lib().pn_tree_query_self_dev(self._h, k, idx_ptr, dist_ptr, stream, 1 if sync else 0))
+
 
 class BallTree(_Tree):
     """petal_neighbors::BallTree<A, Euclidean> on the GPU (src/ball_tree.rs:15-24)."""

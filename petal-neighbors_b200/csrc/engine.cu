@@ -722,7 +722,7 @@ struct Engine final : pn_tree {
     int launch_knn_t(const DeviceTree<A>& t, const KnnArgs<A>& a, dim3 grid, cudaStream_t st) {
         size_t smem = DVR < 0 ? 0 : 2 * TILE_BYTES + (DVR == 0 ? (size_t)TQ * t.ft.dpad * sizeof(A) : 0);
         auto kern = knn_tile_kernel<A, DVR, K, KIND>;
-        if (smem > 32 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        if (smem > 32 * 1024) CU(allow_max_dynamic_smem(kern));
         kern<<<grid, TQ, smem, st>>>(a);
         CU(cudaGetLastError());
         return PN_OK;
@@ -784,7 +784,7 @@ struct Engine final : pn_tree {
     int launch_filter_s(const DeviceTree<A>& t, const CUtensorMap& map_a, const tc::FilterArgs& fa, cudaStream_t st) {
         const size_t smem = filter_fixed_smem(MT, fa.k) + (size_t)MT * fa.nkc * tc::A_CHUNK_BYTES + (size_t)fa.stages * fa.gs * tc::CHUNK_BYTES;
         auto kern = tc::knn_filter_kernel<DVR, K, MT, NACC, SHARED, SW, PRUNE>;
-        CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        CU(allow_max_dynamic_smem(kern));
         const unsigned gx = (fa.nq - fa.row0 + MT * tc::BM - 1) / (MT * tc::BM);
         const unsigned gy = PRUNE ? 1u : (fa.n_tiles + fa.tiles_per_split - 1) / fa.tiles_per_split;
         kern<<<dim3(gx, gy), (5 * MT + 2) * 32, smem, st>>>(map_a, t.d_baug.template as<unsigned char>(), fa);
@@ -939,8 +939,8 @@ struct Engine final : pn_tree {
             TRY(w_wslot.ensure((size_t)n_warps * 4)); TRY(w_wlist.ensure((size_t)wide_cap * 4)); TRY(w_wbits.ensure((size_t)wide_cap * words * 4));
             TRY(w_nwide.ensure(4));
             if (smem > 48u * 1024u) {
-                CU(cudaFuncSetAttribute(tc::ball_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                CU(cudaFuncSetAttribute(tc::ball_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                CU(allow_max_dynamic_smem(tc::ball_tile_kernel<false>));
+                CU(allow_max_dynamic_smem(tc::ball_tile_kernel<true>));
             }
             CU(cudaMemsetAsync(w_nwide.p, 0, 4, st));
             tc::warp_balls_kernel<<<(n_warps + 7) / 8, 256, 0, st>>>(qsorted, w_seed.as<float>(), nq, n_warps, t.dt.dv, w_bcen.as<float4>(), w_brad.as<float>(),

@@ -575,7 +575,7 @@ static int partition_levels(const A* raw, uint64_t stride, uint32_t d, const Tre
     if (rule == 1) {
         GB_CU(sc.get(&wdir, (size_t)max_seg * d));
         if (dir_smem > 200u * 1024u) { err = "rows too wide for the two-means split rule"; return (int)cudaErrorInvalidValue; }
-        GB_CU(cudaFuncSetAttribute(two_means_dir_kernel<A>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dir_smem));
+        GB_CU(allow_max_dynamic_smem(two_means_dir_kernel<A>));
     } else {
         GB_CU(sc.get(&mn, (size_t)max_seg * d));
         GB_CU(sc.get(&mx, (size_t)max_seg * d));

@@ -11,10 +11,38 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <mutex>
+#include <set>
 #include <string>
+#include <utility>
 #include <vector>
 
 namespace petal {
+
+// Lets `kern` launch with as much dynamic shared memory as the current device offers a block.  The limit a launch is
+// checked against is state of the kernel shared by every thread of the process: if each caller set the size it needs,
+// a caller on another thread (another session, another tree) could lower it between this caller's setting and its
+// launch, which then fails with cudaErrorInvalidValue.  Every caller sets the same value instead, once per kernel and
+// device: later calls cost a cudaGetDevice and a lookup.
+template <typename F>
+inline cudaError_t allow_max_dynamic_smem(F* kern) {
+    static std::mutex mu;
+    static std::set<std::pair<const void*, int>> done;   // (kernel, device) pairs whose limit is raised
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    const std::pair<const void*, int> key((const void*)kern, dev);
+    std::lock_guard<std::mutex> lk(mu);
+    if (done.count(key)) return cudaSuccess;
+    int optin = 0;
+    cudaFuncAttributes fa{};
+    e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, kern);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, optin - (int)fa.sharedSizeBytes);
+    if (e == cudaSuccess) done.insert(key);
+    return e;
+}
+
 namespace gb {
 
 // Shape of the implicit complete tree over n points cut at level L (host arithmetic only, shared by both builders):
