@@ -251,6 +251,31 @@ int32_t pn_tree_query_knn_dev(pn_tree *tree, const void *queries_dev, size_t nq,
                               size_t q_row_stride, size_t k, uint64_t *idx_dev, void *dist_dev,
                               void *stream, int32_t sync);
 
+/* Radius search from and into device memory: the result of pn_balltree_query_radius_* / pn_vptree_query_radius_* (strict
+ * `distance < r` on the bit-exact distance, each query's indices ascending) as CSR in caller buffers on the tree's device.
+ * - The element type of queries_dev is the tree's dtype; `radius` is converted to it (exact for any value of that type).
+ * - Any handle: a ball or vantage-point tree (a VP tree answers from its ball partition, as its radius call does), a
+ *   session of either, or a handle of one shard (shard_depth > 0), whose indices are global.
+ * - offsets_dev[nq + 1] is always written in full and equals the offsets the host call returns; offsets_dev[nq] is the
+ *   total.  offsets_dev == NULL is PN_BAD_ARG.  nq == 0 writes offsets_dev[0] = 0.
+ * - Query q's segment is written to indices_dev[offsets[q] .. offsets[q + 1]) if and only if offsets[q + 1] <= capacity;
+ *   nothing is ever written at or past `capacity`.  The offsets do not decrease, so the written queries are a prefix of
+ *   the batch: a caller whose buffer was too small reads the total, then reallocates or re-issues only the queries after
+ *   that prefix.  indices_dev may be NULL only with capacity == 0 (offsets only).
+ * - Argument checks as pn_tree_query_knn_dev: a PN_FLAG_HOST_ONLY handle returns PN_CUDA; nq < 2^32; q_row_stride >= d
+ *   when nq > 1.
+ * - `stream` NULL is the handle's own stream.  With sync == 0 the call returns after enqueueing: no stream, event or device
+ *   synchronisation and no device-to-host copy happens inside, except that (1) the first radius call on a VP handle
+ *   may build its ball partition (f64, d < 16 or fewer than 1024 points); (2) a call on another stream than the
+ *   handle's previous call first waits for that stream, as for k-NN; (3) the workspaces are sized per chunk of
+ *   queries (the whole batch up to 2^18 queries, otherwise chunks of 2^17), and a call whose chunk is larger than that
+ *   of every earlier radius call on the handle allocates larger ones -- freeing and allocating device memory can
+ *   synchronise the device, as for k-NN.  Once the workspaces are warm, the guarantee holds without exception.  With
+ *   sync != 0 the call waits, and the counters (pairs, device_ms, ...) describe it. */
+int32_t pn_tree_query_radius_dev(pn_tree *tree, const void *queries_dev, size_t nq, size_t q_row_stride,
+                                 double radius, uint64_t *offsets_dev, uint64_t *indices_dev, size_t capacity,
+                                 void *stream, int32_t sync);
+
 /* K-way merge of `n_lists` per-shard sorted top-k lists (layout [list][nq][k]) by
  * (distance, index): the step after the all-gather when points are sharded by subtree
  * (no reference equivalent; SURVEY.md 8e).  All pointers are device pointers on `device`. */

@@ -12,7 +12,9 @@ mirrors the reference's public surface name for name:
     petal_neighbors::distance::{Metric, Euclidean}                src/distance.rs:9-55
 
 plus the batched additions (`query_batch`, `query_nearest_batch`, `query_radius_batch`) that a
-GPU engine needs; the single-point methods are batches of one.  All compute happens in the CUDA
+GPU engine needs; the single-point methods are batches of one.  The batched calls also take a torch CUDA tensor of
+queries on the tree's device: they then run on torch's current stream and return CUDA tensors (int64 indices, -1 where
+the host path pads with 2^64 - 1; distances in the tree's dtype; radius search: int64 offsets and indices).  All compute happens in the CUDA
 library; nothing here falls back to the CPU.  (The Rust crate that binds the same ABI is under
 rust/petal-neighbors-b200/, see INTEGRATION.md.)
 """
@@ -75,6 +77,16 @@ def _strides(a):
     rs = a.strides[0] // it if a.shape[0] > 1 else max(a.shape[1], 1)
     cs = a.strides[1] // it if a.shape[1] > 1 else 1
     return rs, cs
+
+
+_CUDA_STREAM_LEGACY = 1   # cudaStreamLegacy
+# the largest first index buffer of a CUDA-tensor radius search (1 GiB of int64): a larger result is completed by
+# re-issuing the queries that did not fit, so the cap bounds memory, not the result
+_RADIUS_GUESS_MAX = 1 << 27
+
+
+def _is_cuda_tensor(x):
+    return hasattr(x, "data_ptr") and getattr(x, "is_cuda", False)
 
 
 def _csr_arrays(offs_p, idx_p, nq):
@@ -214,7 +226,69 @@ class _Tree:
             Q = np.ascontiguousarray(Q)
         return Q, (Q.strides[0] // Q.dtype.itemsize if Q.shape[0] > 1 else max(Q.shape[1], 1))
 
+    def _tensor_queries(self, Q):
+        """A CUDA tensor of queries on the tree's device, in the tree's dtype and with unit column stride (copied only if
+        needed), its row stride, and the handle of the current torch stream of that device.  Torch's default stream is the
+        legacy NULL stream, handle 0, which the C API reads as the tree handle's own stream: it is passed as
+        cudaStreamLegacy."""
+        import torch
+        dev = self.info()["device"]
+        if Q.device.index != dev:
+            raise ValueError(f"queries are on {Q.device}, the tree on cuda:{dev}")
+        if Q.dim() != 2:
+            raise ValueError("queries must be 2-D (nq x d)")
+        if Q.shape[1] != self.dim:
+            raise ValueError(f"query dimension {Q.shape[1]} != tree dimension {self.dim}")
+        Q = Q.to(torch.float32 if self.dtype == np.float32 else torch.float64)
+        nq, d = Q.shape
+        if (d > 1 and Q.stride(1) != 1) or (nq > 1 and Q.stride(0) < d):
+            Q = Q.contiguous()
+        return Q, (Q.stride(0) if nq > 1 else max(d, 1)), torch.cuda.current_stream(Q.device).cuda_stream or _CUDA_STREAM_LEGACY
+
+    def _knn_tensor(self, Q, k):
+        """k-NN of CUDA-tensor queries on the current stream, without synchronising: (indices[nq, k] int64, -1 where
+        k > n; distances[nq, k] in the tree's dtype)."""
+        import torch
+        Q, qs, st = self._tensor_queries(Q)
+        nq = Q.shape[0]
+        idx = torch.empty((nq, k), dtype=torch.int64, device=Q.device)
+        dist = torch.empty((nq, k), dtype=Q.dtype, device=Q.device)
+        if nq and k:
+            self.query_knn_dev(Q.data_ptr(), nq, qs, k, idx.data_ptr(), dist.data_ptr(), stream=st, sync=False)
+        return idx, dist
+
+    def _radius_tensor(self, Q, radius):
+        """Radius search of CUDA-tensor queries on the current stream: (offsets[nq + 1], indices) int64 CUDA tensors.  The
+        indices first go to a buffer sized from the density of this handle's previous tensor call, but never larger than
+        nq x (points of the handle) or _RADIUS_GUESS_MAX entries; the one synchronisation reads the total.  If the buffer
+        was too small, only the queries that did not fit are issued again, into the exact-size remainder; if it was much
+        too large, the indices are returned in a copy of their own size."""
+        import torch
+        Q, qs, st = self._tensor_queries(Q)
+        nq = Q.shape[0]
+        offs = torch.empty(nq + 1, dtype=torch.int64, device=Q.device)
+        guess = int(nq * getattr(self, "_radius_density", 8.0) * 1.12) + 1024
+        cap = min(guess, nq * int(self.info()["n_points"]), _RADIUS_GUESS_MAX)
+        idx = torch.empty(cap, dtype=torch.int64, device=Q.device)
+        self.query_radius_dev(Q.data_ptr(), nq, qs, radius, offs.data_ptr(), idx.data_ptr(), cap, stream=st,
+                              sync=False)
+        # the queries written: those whose segment ends at or below cap (a prefix); their end is where the rest goes
+        done = torch.searchsorted(offs[1:], cap, right=True).view(1)
+        total, done, base = torch.cat([offs[-1:], done, offs.index_select(0, done)]).tolist()
+        self._radius_density = total / max(nq, 1)
+        if total <= cap:   # a view would keep the whole guess alive as long as the result
+            return offs, (idx[:total] if cap - total <= total // 4 else idx[:total].clone())
+        out = torch.empty(total, dtype=torch.int64, device=Q.device)
+        out[:base] = idx[:base]
+        rest = Q[done:]
+        self.query_radius_dev(rest.data_ptr(), nq - done, qs, radius, offs[done:].data_ptr(), out[base:].data_ptr(),
+                              total - base, stream=st, sync=False)
+        offs[done:] += base
+        return offs, out
+
     def _knn(self, fname, Q, k):
+        if _is_cuda_tensor(Q):
+            return self._knn_tensor(Q, k)
         Q, qs = self._queries(Q)
         nq = Q.shape[0]
         idx = np.empty((nq, k), np.uint64)
@@ -228,6 +302,8 @@ class _Tree:
         return idx, dist
 
     def _radius(self, Q, radius):
+        if _is_cuda_tensor(Q):
+            return self._radius_tensor(Q, radius)
         Q, qs = self._queries(Q)
         nq = Q.shape[0]
         L = _ffi.lib()
@@ -243,6 +319,13 @@ class _Tree:
         _check(_ffi.lib().pn_tree_query_knn_dev(self._h, q_ptr, nq, q_row_stride, k, idx_ptr, dist_ptr, stream,
                                                 1 if sync else 0))
 
+    def query_radius_dev(self, q_ptr: int, nq: int, q_row_stride: int, radius, offsets_ptr: int, indices_ptr: int,
+                         capacity: int, stream: int = 0, sync: bool = True):
+        """Device-pointer radius search (pn_tree_query_radius_dev): queries and the CSR outputs in HBM.  offsets[nq + 1]
+        is always written; query q's indices are written only if offsets[q + 1] <= capacity (a prefix of the batch)."""
+        _check(_ffi.lib().pn_tree_query_radius_dev(self._h, q_ptr, nq, q_row_stride, float(self.dtype.type(radius)),
+                                                   offsets_ptr, indices_ptr, capacity, stream, 1 if sync else 0))
+
     def query_self_dev(self, k: int, idx_ptr: int, dist_ptr: int, stream: int = 0, sync: bool = True):
         """Device-pointer self-query (pn_tree_query_self_dev): every stored point is a query, row i of the n x k
         outputs (already in HBM) is the answer for points[i]."""
@@ -255,7 +338,9 @@ class BallTree(_Tree):
 
     def query_batch(self, Q, k: int):
         """Batched BallTree::query: (indices[nq, k] u64, distances[nq, k]); rows padded with
-        (2^64-1, +inf) when k > n."""
+        (2^64-1, +inf) when k > n.
+        CUDA-tensor queries (on the tree's device, any float dtype and strides): CUDA tensors on torch's current stream,
+        without synchronising; indices int64, -1 where k > n pads; distances in the tree's dtype."""
         return self._knn("pn_balltree_query", Q, int(k))
 
     def query(self, point, k: int):
@@ -275,6 +360,8 @@ class BallTree(_Tree):
         return idx, dist
 
     def query_nearest_batch(self, Q):
+        """Batched BallTree::query_nearest: (indices[nq] u64, distances[nq]).  CUDA-tensor queries (on the tree's device): CUDA tensors on torch's current stream, without synchronising;
+        indices int64, distances in the tree's dtype."""
         idx, dist = self._knn("pn_balltree_query_nearest", Q, 1)
         return idx[:, 0], dist[:, 0]
 
@@ -285,7 +372,9 @@ class BallTree(_Tree):
 
     def query_radius_batch(self, Q, radius):
         """Batched BallTree::query_radius: CSR (offsets[nq+1], indices), each query's indices
-        ascending; strict `distance < radius` (src/ball_tree.rs:277)."""
+        ascending; strict `distance < radius` (src/ball_tree.rs:277).  Numpy queries: u64 numpy arrays.
+        CUDA-tensor queries (on the tree's device): int64 CUDA tensors on torch's current stream; the call
+        synchronises once, to read the total."""
         return self._radius(Q, radius)
 
     def query_radius(self, point, radius):
@@ -299,6 +388,8 @@ class VantagePointTree(_Tree):
     _kind = "vptree"
 
     def query_nearest_batch(self, Q):
+        """Batched VantagePointTree::query_nearest: (indices[nq] u64, distances[nq]).  CUDA-tensor queries (on the tree's device): CUDA tensors on torch's current stream, without synchronising;
+        indices int64, distances in the tree's dtype."""
         idx, dist = self._knn("pn_vptree_query_nearest", Q, 1)
         return idx[:, 0], dist[:, 0]
 
@@ -309,7 +400,10 @@ class VantagePointTree(_Tree):
 
     # Extensions (the reference VP tree has query_nearest only): the answers BallTree gives for the same points.
     def query_batch(self, Q, k: int):
-        """k-NN on the vantage-point handle: (indices[nq, k] u64, distances[nq, k]), (distance, index) ascending."""
+        """k-NN on the vantage-point handle: (indices[nq, k] u64, distances[nq, k]), (distance, index) ascending; rows
+        padded with (2^64-1, +inf) when k > n.
+        CUDA-tensor queries (on the tree's device, any float dtype and strides): CUDA tensors on torch's current stream,
+        without synchronising; indices int64, -1 where k > n pads; distances in the tree's dtype."""
         return self._knn("pn_vptree_query", Q, int(k))
 
     def query(self, point, k: int):
@@ -318,7 +412,10 @@ class VantagePointTree(_Tree):
         return idx[0, :m].astype(np.uintp), dist[0, :m]
 
     def query_radius_batch(self, Q, radius):
-        """Radius search on the vantage-point handle: CSR (offsets[nq+1], indices), strict `distance < radius`."""
+        """Radius search on the vantage-point handle: CSR (offsets[nq+1], indices), strict `distance < radius`.  Numpy
+        queries: u64 numpy arrays.
+        CUDA-tensor queries (on the tree's device): int64 CUDA tensors on torch's current stream; the call
+        synchronises once, to read the total."""
         return self._radius(Q, radius)
 
     def query_radius(self, point, radius):

@@ -29,7 +29,7 @@ EXPORTS = [
     "pn_vptree_query_f32", "pn_vptree_query_f64", "pn_vptree_query_radius_f32", "pn_vptree_query_radius_f64",
     "pn_balltree_query_self_f32", "pn_balltree_query_self_f64", "pn_tree_query_self_dev",
     "pn_pairwise_f32", "pn_pairwise_f64",
-    "pn_free", "pn_tree_query_knn_dev", "pn_merge_topk_dev", "pn_merge_radius_dev",
+    "pn_free", "pn_tree_query_knn_dev", "pn_tree_query_radius_dev", "pn_merge_topk_dev", "pn_merge_radius_dev",
     "pn_tree_get_info", "pn_tree_get_counters", "pn_tree_get_layout",
     "pn_comm_unique_id", "pn_comm_create", "pn_comm_create_all", "pn_comm_destroy", "pn_query_slice",
     "pn_sharded_query_knn_dev", "pn_tree_replicate",
@@ -126,6 +126,8 @@ def lib():
     L.pn_free.restype = None
     L.pn_tree_query_knn_dev.restype = C.c_int32
     L.pn_tree_query_knn_dev.argtypes = [vp, vp, sz, sz, sz, vp, vp, vp, C.c_int32]
+    L.pn_tree_query_radius_dev.restype = C.c_int32
+    L.pn_tree_query_radius_dev.argtypes = [vp, vp, sz, sz, C.c_double, vp, vp, sz, vp, C.c_int32]
     L.pn_tree_query_self_dev.restype = C.c_int32
     L.pn_tree_query_self_dev.argtypes = [vp, sz, vp, vp, vp, C.c_int32]
     L.pn_merge_topk_dev.restype = C.c_int32

@@ -205,6 +205,8 @@ struct pn_tree {
     virtual int knn_dev(const void* q, size_t nq, size_t stride, size_t k, uint64_t* idx, void* dist,
                         cudaStream_t st, bool sync) = 0;
     virtual int radius_host(const void* q, size_t nq, size_t stride, double r, uint64_t** offs, uint64_t** idx) = 0;
+    virtual int radius_dev(const void* q, size_t nq, size_t stride, double r, uint64_t* offs, uint64_t* idx, size_t capacity,
+                           cudaStream_t st, bool sync) = 0;
     virtual int knn_self(size_t k, uint64_t* idx, void* dist, bool dev, cudaStream_t st, bool sync) = 0;
     virtual int layout(uint32_t* ids, uint32_t* blo, uint32_t* bhi, void* rad, void* cen, void* pts) = 0;
     virtual int knn_sharded(pn_comm* cm, const void* q, size_t nq, size_t stride, size_t k, uint32_t exchange, uint64_t* idx, void* dist,
@@ -675,6 +677,7 @@ struct Engine final : pn_tree {
     DevBuf w_qraw2[2], w_oi2[2], w_od2[2];
     DevBuf sh_li[2], sh_ld[2], sh_pack[2], sh_gat[2], sh_gat_d[2];   // sharded k-NN: local lists, packed keys, gathered lists
     DevBuf r_qraw[2], r_q[2], r_counts[2], r_offsets[2], r_hits[2], r_slab[2], r_qlist[2], r_nlist[2], r_sums[2];  // radius pipeline workspaces
+    DevBuf r_llist;               // radius_dev: the queries of a chunk whose hits the block sort orders
     // radius search of a multi-GPU handle: queries, the CSR of radius_device, the lists pulled from every shard, their merge
     DevBuf rd_q, rd_offs, rd_hits, rp_offs, rp_hits, rm_offs, rm_hits;
     // tensor path (f32 input only): per-call workspaces, see tc_filter.cuh
@@ -1497,38 +1500,49 @@ struct Engine final : pn_tree {
         return PN_OK;
     }
     // pad the queries (row stride q_stride elements), count traversal with the first RADIUS_CAP hits of each query in its
-    // slab, chunk-local offsets (r_offsets[b][cq] is the chunk's total)
-    int radius_count(const DeviceTree<A>& t, int b, const A* q, size_t q_stride, uint32_t cq, A r, cudaStream_t s) {
+    // slab, chunk-local offsets (r_offsets[b][cq] is the chunk's total).  radius_dev passes `offs`, the caller's array at
+    // the chunk's first query, and from the second chunk on `base` == offs: the offsets are then absolute.
+    int radius_count(const DeviceTree<A>& t, int b, const A* q, size_t q_stride, uint32_t cq, A r, cudaStream_t s,
+                     uint64_t* offs = nullptr, const uint64_t* base = nullptr) {
         const size_t tot = (size_t)cq * t.ft.dpad;
         pad_queries_kernel<A><<<(unsigned)((tot + 255) / 256), 256, 0, s>>>(q, q_stride, cq, t.ft.d, t.ft.dpad, r_q[b].as<A>());
         CU(cudaGetLastError());
         const unsigned blocks = (cq + RADIUS_WPB - 1) / RADIUS_WPB;
-        CU(cudaMemsetAsync(r_nlist[b].p, 0, 4, s));
+        CU(cudaMemsetAsync(r_nlist[b].p, 0, 8, s));   // the lengths of the two lists of radius_fill
         radius_kernel<A, 0><<<blocks, RADIUS_WPB * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, r_counts[b].as<uint32_t>(), nullptr, r_slab[b].as<uint32_t>(),
                                                               w_counters.as<unsigned long long>());
         CU(cudaGetLastError());
         const unsigned sblocks = std::max(1u, (cq + SCAN_BLOCK - 1) / SCAN_BLOCK);
         scan_sums_kernel<<<sblocks, 1024, 0, s>>>(r_counts[b].as<uint32_t>(), cq, r_sums[b].as<unsigned long long>());
-        offsets_scan_kernel<<<sblocks, 1024, 0, s>>>(r_counts[b].as<uint32_t>(), r_sums[b].as<unsigned long long>(), r_offsets[b].as<uint64_t>(), cq);
+        offsets_scan_kernel<<<sblocks, 1024, 0, s>>>(r_counts[b].as<uint32_t>(), r_sums[b].as<unsigned long long>(),
+                                                     offs ? offs : r_offsets[b].as<uint64_t>(), cq, base);
         CU(cudaGetLastError());
         counters.kernel_launches += 4;
         return PN_OK;
     }
-    // slabs -> hits[0 .. ctotal) at the chunk-local offsets, second traversal of the queries that overflowed their slab,
-    // per-query ascending sort
-    int radius_fill(const DeviceTree<A>& t, int b, uint32_t cq, A r, uint64_t ctotal, uint32_t* hits, cudaStream_t s) {
+    // slabs -> hits at the offsets, second traversal of the queries that overflowed their slab, per-query ascending sort.
+    // Host pipelines: chunk-local offsets (r_offsets[b]), hits[0 .. ctotal) u32, and the block sort is launched when the
+    // chunk's total says some list may need it.  radius_dev: `offs` as in radius_count, hits the caller's u64 array, only
+    // the queries whose segment ends at or below `capacity` are written, and the block sort always runs, over the list of
+    // long segments the compaction builds (ctotal is not known on the host).
+    template <typename I>
+    int radius_fill(const DeviceTree<A>& t, int b, uint32_t cq, A r, uint64_t ctotal, I* hits, cudaStream_t s,
+                    const uint64_t* offs = nullptr, uint64_t capacity = ~0ull) {
         const unsigned blocks = (cq + RADIUS_WPB - 1) / RADIUS_WPB;
-        compact_hits_kernel<<<blocks, RADIUS_WPB * 32, 0, s>>>(r_slab[b].as<uint32_t>(), r_counts[b].as<uint32_t>(), r_offsets[b].as<uint64_t>(), cq,
-                                                               hits, r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
+        const uint64_t* o = offs ? offs : r_offsets[b].as<uint64_t>();
+        uint32_t* n_lists = r_nlist[b].as<uint32_t>();   // [0]: slab overflows, [1]: long segments (radius_dev)
+        uint32_t* llist = offs ? r_llist.as<uint32_t>() : nullptr;
+        compact_hits_kernel<I><<<blocks, RADIUS_WPB * 32, 0, s>>>(r_slab[b].as<uint32_t>(), r_counts[b].as<uint32_t>(), o, cq, hits,
+                                                                  r_qlist[b].as<uint32_t>(), n_lists, capacity, llist, n_lists + 1);
         CU(cudaGetLastError());
         // second traversal for the queries that overflowed their slab only (warps past the list length exit at once)
-        radius_kernel<A, 1><<<blocks, RADIUS_WPB * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, nullptr, r_offsets[b].as<uint64_t>(), hits,
-                                                              nullptr, r_qlist[b].as<uint32_t>(), r_nlist[b].as<uint32_t>());
+        radius_kernel<A, 1, I><<<blocks, RADIUS_WPB * 32, 0, s>>>(t.dt, r_q[b].as<V>(), cq, r, nullptr, o, hits,
+                                                                 nullptr, r_qlist[b].as<uint32_t>(), n_lists);
         CU(cudaGetLastError());
-        segment_sort_kernel<<<blocks, RADIUS_WPB * 32, 0, s>>>(r_offsets[b].as<uint64_t>(), hits, cq);
+        segment_sort_kernel<I><<<blocks, RADIUS_WPB * 32, 0, s>>>(o, hits, cq, capacity);
         CU(cudaGetLastError());
-        if (ctotal > SORT_WARP_MAX) {  // some hit list may be longer than a warp should sort: one block per such query
-            segment_sort_large_kernel<<<std::min<uint32_t>(cq, 8u * (uint32_t)n_sms), 256, 0, s>>>(r_offsets[b].as<uint64_t>(), hits, cq);
+        if (llist || ctotal > SORT_WARP_MAX) {  // some hit list may be longer than a warp should sort: one block per such query
+            segment_sort_large_kernel<I><<<std::min<uint32_t>(cq, 8u * (uint32_t)n_sms), 256, 0, s>>>(o, hits, cq, llist, n_lists + 1);
             CU(cudaGetLastError());
             ++counters.kernel_launches;
         }
@@ -1662,6 +1676,40 @@ struct Engine final : pn_tree {
         *offs_out = offs.release();
         *idx_out = hit_buf.release();
         return PN_OK;
+    }
+
+    // Radius search from and into device memory (pn_tree_query_radius_dev), enqueued on one stream over the chunks of
+    // radius_device: per chunk the count pass scans its offsets onto the total the previous chunk left in offs[q0], and the
+    // fill pass writes the hits of the queries that fit below `capacity` straight into the caller's u64 array.  Nothing
+    // waits for a result on the host; the workspaces are bounded per chunk.
+    int radius_dev(const void* qv, size_t nq, size_t stride, double rr, uint64_t* offs, uint64_t* idx, size_t capacity,
+                   cudaStream_t st, bool sync) override {
+        TRY(check_query_args(qv, nq, stride));
+        if (!offs) return fail(PN_BAD_ARG, "offsets_dev is null");
+        if (!idx && capacity) return fail(PN_BAD_ARG, "indices_dev is null with capacity > 0");
+        Call call(*this);
+        TRY(call.device());
+        std::shared_ptr<DeviceTree<A>> comp;   // a VP handle answers from its ball companion, as radius_host does
+        if (nq && tree->ft.kind != 0) TRY(tree->companion(stream, comp));
+        const DeviceTree<A>& t = comp ? *comp : *tree;
+        TRY(call.open(st ? st : (cudaStream_t)stream));
+        const A r = (A)rr;
+        const A* q = (const A*)qv;
+        const size_t chunk = nq <= (1u << 18) ? std::max<size_t>(nq, 1) : (1u << 17);
+        last_used_tensor = false; last_pruned = false;
+        // every allocation before the first enqueue (a cudaMalloc can synchronise)
+        TRY(radius_workspace(t, 1, chunk));
+        TRY(r_llist.ensure(chunk * 4));
+        TRY(call.start());
+        if (nq == 0) CU(cudaMemsetAsync(offs, 0, 8, call.st));
+        CU(cudaEventRecord(ev[2], call.st));
+        for (size_t q0 = 0; q0 < nq; q0 += chunk) {
+            const uint32_t cq = (uint32_t)std::min(chunk, nq - q0);
+            TRY(radius_count(t, 0, q + q0 * stride, stride, cq, r, call.st, offs + q0, q0 ? offs + q0 : nullptr));
+            TRY(radius_fill<uint64_t>(t, 0, cq, r, 0, idx, call.st, offs + q0, capacity));
+        }
+        CU(cudaEventRecord(ev[3], call.st));
+        return call.finish(nq, sync);
     }
 
     // ---- point sharding by subtree: local scan -> NCCL exchange -> k-way merge, pipelined over chunks of queries ----------
@@ -2452,6 +2500,13 @@ int32_t pn_tree_query_knn_dev(pn_tree* t, const void* q, size_t nq, size_t qs, s
     GUARD_BEGIN
     if (!t) return fail(PN_BAD_ARG, "tree is null");
     return t->knn_dev(q, nq, qs, k, io, dd, (cudaStream_t)stream, sync != 0);
+    GUARD_END
+}
+int32_t pn_tree_query_radius_dev(pn_tree* t, const void* q, size_t nq, size_t qs, double radius, uint64_t* oo, uint64_t* io, size_t capacity,
+                                 void* stream, int32_t sync) {
+    GUARD_BEGIN
+    if (!t) return fail(PN_BAD_ARG, "tree is null");
+    return t->radius_dev(q, nq, qs, radius, oo, io, capacity, (cudaStream_t)stream, sync != 0);
     GUARD_END
 }
 int32_t pn_merge_topk_dev(uint32_t dtype, int32_t device, const uint64_t* il, const void* dl, size_t n_lists, size_t nq, size_t k,

@@ -889,12 +889,13 @@ __global__ void scatter_order_kernel(const uint32_t* __restrict__ home, uint32_t
 // Single traversal for the common case: MODE 0 writes the first RADIUS_CAP hits of every query into its slab
 // (slab[qi * RADIUS_CAP + ..]) and the full count into counts[]; compact_hits_kernel then moves the slabs to their CSR
 // positions and lists the queries whose count exceeds the slab, and only those are traversed again (MODE 1: fill at
-// offsets[qi], queries taken from qlist[0 .. *n_list)).
+// offsets[qi], queries taken from qlist[0 .. *n_list)).  I is the type of the output indices: u32 into the slab and the
+// engine's own hit buffers, u64 into the caller's array of the device-resident call.
 constexpr uint32_t RADIUS_CAP = 64;
-template <typename A, int MODE>
+template <typename A, int MODE, typename I = uint32_t>
 __global__ void radius_kernel(const DevTree<A> t, const typename VT<A>::V* __restrict__ q, uint32_t nq, A r,
                               uint32_t* __restrict__ counts, const uint64_t* __restrict__ offsets,
-                              uint32_t* __restrict__ out, unsigned long long* counters,
+                              I* __restrict__ out, unsigned long long* counters,
                               const uint32_t* __restrict__ qlist = nullptr, const uint32_t* __restrict__ n_list = nullptr) {
     using V = typename VT<A>::V;
     const unsigned full = 0xffffffffu;
@@ -955,24 +956,36 @@ __global__ void radius_kernel(const DevTree<A> t, const typename VT<A>::V* __res
     if (counters && lane == 0) atomicAdd(&counters[0], pairs);
 }
 
+// Segments of up to SORT_WARP_MAX hits are sorted by one warp each, longer ones by one block each (see segment_sort_kernel).
+constexpr uint32_t SORT_WARP_MAX = 1024;
+
 // slabs -> CSR: one warp per query copies its (at most RADIUS_CAP) hits to offsets[qi]; queries that overflowed their
-// slab are appended to qlist for the second traversal
+// slab are appended to qlist for the second traversal.  Only a query whose segment ends at or below `capacity`
+// (offsets[qi] + counts[qi] <= capacity) is written or listed; with `llist`, such a query with more than SORT_WARP_MAX hits
+// is also appended to llist for the block sort.
+template <typename I>
 __global__ void compact_hits_kernel(const uint32_t* __restrict__ slab, const uint32_t* __restrict__ counts, const uint64_t* __restrict__ offsets,
-                                    uint32_t nq, uint32_t* __restrict__ hits, uint32_t* __restrict__ qlist, uint32_t* __restrict__ n_list) {
+                                    uint32_t nq, I* __restrict__ hits, uint32_t* __restrict__ qlist, uint32_t* __restrict__ n_list,
+                                    uint64_t capacity = ~0ull, uint32_t* __restrict__ llist = nullptr, uint32_t* __restrict__ n_llist = nullptr) {
     const int lane = threadIdx.x & 31;
     const uint32_t qi = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (qi >= nq) return;
     const uint32_t c = counts[qi];
+    const uint64_t o = offsets[qi];
+    if (o + c > capacity) return;
+    if (llist && c > SORT_WARP_MAX && lane == 0) llist[atomicAdd(n_llist, 1u)] = qi;
     if (c > RADIUS_CAP) {
         if (lane == 0) qlist[atomicAdd(n_list, 1u)] = qi;
         return;
     }
-    const uint64_t o = offsets[qi];
     for (uint32_t i = lane; i < c; i += 32) hits[o + i] = slab[(uint64_t)qi * RADIUS_CAP + i];
 }
 
 // u32 counts -> u64 exclusive offsets, offsets[n] = total.  Two launches over blocks of SCAN_BLOCK counts: the sums of the
 // blocks, then every block adds the sums of the blocks before it (at most a few hundred values) to its own scan.
+// With `base_in`, the offsets start at *base_in instead of 0: the device-resident radius call scans chunk c onto the total
+// that chunk c - 1 left at the same position (base_in == offsets, read before any thread writes it, and rewritten with
+// the value read), so the host never needs a chunk's total.
 constexpr uint32_t SCAN_BLOCK = 4096;   // 1024 threads x 4 counts
 __global__ void scan_sums_kernel(const uint32_t* __restrict__ counts, uint32_t n, unsigned long long* __restrict__ sums) {
     __shared__ unsigned long long ws[32];
@@ -994,11 +1007,11 @@ __global__ void scan_sums_kernel(const uint32_t* __restrict__ counts, uint32_t n
     }
 }
 __global__ void offsets_scan_kernel(const uint32_t* __restrict__ counts, const unsigned long long* __restrict__ sums,
-                                    uint64_t* __restrict__ offsets, uint32_t n) {
+                                    uint64_t* offsets, uint32_t n, const uint64_t* base_in = nullptr) {
     __shared__ unsigned long long ws[33];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     // sum of the blocks before this one
-    unsigned long long base = 0;
+    unsigned long long base = (base_in && threadIdx.x == 0) ? *base_in : 0;
     for (uint32_t b = threadIdx.x; b < blockIdx.x; b += blockDim.x) base += sums[b];
     for (int o = 16; o; o >>= 1) base += __shfl_down_sync(0xffffffffu, base, o);
     if (lane == 0) ws[w] = base;
@@ -1148,23 +1161,27 @@ inline cudaError_t merge_radius_lists(cudaStream_t st, const uint64_t* offsets, 
 // comparing, src/ball_tree.rs:667, 777): bitonic network over the segment padded to a power of two with virtual +inf
 // keys.  Segments of up to SORT_WARP_MAX entries are sorted by one warp each; longer ones (large radii: whole subtrees
 // included) by one 256-thread block each in a second launch, so that a few huge hit lists do not serialise on 32 lanes.
-constexpr uint32_t SORT_WARP_MAX = 1024;
+// I is the type of the indices (u32 in the engine's hit buffers, u64 in the caller's array of the device-resident call).
 // all-ascending form of the network (first step of each phase mirrors, i ^ (size-1)): every compare-exchange moves the
 // smaller key down, so the virtual +inf keys at >= n never move
-__device__ __forceinline__ void sort_cmpx(uint32_t* v, uint32_t n, uint32_t i, uint32_t j) {
+template <typename I>
+__device__ __forceinline__ void sort_cmpx(I* v, uint32_t n, uint32_t i, uint32_t j) {
     if (j > i && j < n) {
-        const uint32_t x = v[i], y = v[j];
+        const I x = v[i], y = v[j];
         if (x > y) { v[i] = y; v[j] = x; }
     }
 }
-__global__ void segment_sort_kernel(const uint64_t* __restrict__ offsets, uint32_t* __restrict__ vals, uint32_t nq) {
+// segments that end past `capacity` were not written (compact_hits_kernel) and are left alone
+template <typename I>
+__global__ void segment_sort_kernel(const uint64_t* __restrict__ offsets, I* __restrict__ vals, uint32_t nq, uint64_t capacity = ~0ull) {
     const int lane = threadIdx.x & 31;
     const uint32_t qi = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (qi >= nq) return;
     const uint64_t lo = offsets[qi];
+    if (offsets[qi + 1] > capacity) return;
     const uint32_t n = (uint32_t)(offsets[qi + 1] - lo);
     if (n < 2 || n > SORT_WARP_MAX) return;
-    uint32_t* v = vals + lo;
+    I* v = vals + lo;
     uint32_t np2 = 1;
     while (np2 < n) np2 <<= 1;
     for (uint32_t size = 2; size <= np2; size <<= 1) {
@@ -1176,13 +1193,20 @@ __global__ void segment_sort_kernel(const uint64_t* __restrict__ offsets, uint32
         }
     }
 }
-__global__ void __launch_bounds__(256) segment_sort_large_kernel(const uint64_t* __restrict__ offsets, uint32_t* __restrict__ vals, uint32_t nq) {
-  for (uint32_t qi = blockIdx.x; qi < nq; qi += gridDim.x) {   // a fixed grid walks the queries; long lists are rare
+// Without `list`, the grid walks all nq queries; with it, only the queries list[0 .. *n_list) (built on the device by
+// compact_hits_kernel), so the launch needs no host-side knowledge of the hit counts and exits at once on an empty list.
+template <typename I>
+__global__ void __launch_bounds__(256) segment_sort_large_kernel(const uint64_t* __restrict__ offsets, I* __restrict__ vals, uint32_t nq,
+                                                                 const uint32_t* __restrict__ list = nullptr,
+                                                                 const uint32_t* __restrict__ n_list = nullptr) {
+  const uint32_t n_walk = list ? *n_list : nq;
+  for (uint32_t j = blockIdx.x; j < n_walk; j += gridDim.x) {   // a fixed grid walks the queries; long lists are rare
+    const uint32_t qi = list ? list[j] : j;
     const uint64_t lo = offsets[qi];
     const uint64_t n64 = offsets[qi + 1] - lo;
     if (n64 <= SORT_WARP_MAX) continue;        // block-uniform
     const uint32_t n = (uint32_t)n64;
-    uint32_t* v = vals + lo;
+    I* v = vals + lo;
     uint64_t np2 = 1;
     while (np2 < n) np2 <<= 1;
     for (uint64_t size = 2; size <= np2; size <<= 1) {

@@ -78,6 +78,10 @@ extern "C" {
     // merge of per-shard CSR radius results on one device (all pointers are device pointers)
     pub fn pn_merge_radius_dev(device: i32, offsets_lists_dev: *const u64, indices_lists_dev: *const u64, n_lists: usize, nq: usize,
                                out_offsets_dev: *mut u64, out_indices_dev: *mut u64, stream: *mut std::ffi::c_void, sync: i32) -> i32;
+    // radius search from and into device memory on the tree's device (include/petal_b200.h: pn_tree_query_radius_dev)
+    pub fn pn_tree_query_radius_dev(t: *mut pn_tree, queries_dev: *const std::ffi::c_void, nq: usize, q_row_stride: usize,
+                                    radius: f64, offsets_dev: *mut u64, indices_dev: *mut u64, capacity: usize,
+                                    stream: *mut std::ffi::c_void, sync: i32) -> i32;
 }
 
 #[repr(C)]
